@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: converged ascent-NLP solves per second.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -42,6 +42,37 @@ METRIC = "converged ascent-NLP solves/sec at batch 64K"
 # by (dcost on, problems in the launch, nt) and reported only when the run matches that workload, otherwise null.
 NCU_TRAFFIC = {(True, 65536, 200): (217.761e9 + 123.660e9, "profiles/r02_ncu_ascent_ipm_kernel_metrics.csv"),
                (True, 4096, 2001): (596.359e9 + 265.691e9, "profiles/r02_ncu_ascent_coop_kernel_cfg5_metrics.csv")}
+DUMP_BYTES = 48 * 2**20        # --dump-outputs: all files together stay below this (a full config-4 step is ~1 GB)
+
+
+def dump_outputs(dirname, raw, traj_offset=0):
+    """Write the arrays one step returned (``solve_rows``' dict) as ``dirname/<name>.npy``, all float64 (status and
+    iterations convert exactly).  The per-problem results cover the whole batch when they fit a quarter of
+    DUMP_BYTES, the [10, nt, n] trajectory block as many problems as the rest allows; where not every problem
+    fits, the problems are a fixed seeded sample.  ``index.npy`` / ``traj_index.npy`` name the problems (index
+    in the batch) row for row, so the files of two builds run with the same arguments compare element-wise."""
+    import numpy as np
+    import torch
+
+    def pick(B, bytes_per_problem, budget):
+        n = min(B, budget // bytes_per_problem)
+        if n == B:
+            return torch.arange(B)
+        return torch.randperm(B, generator=torch.Generator().manual_seed(0))[:n].sort().values
+
+    keys = [k for k in ("tf", "final_mass", "status", "iterations", "kkt") if raw.get(k) is not None]
+    idx = pick(int(raw["tf"].shape[0]), 8 * (len(keys) + 1), DUMP_BYTES // 4)
+    out = {k: raw[k][idx.to(raw[k].device)] for k in keys}
+    out["index"] = idx
+    traj = raw.get("traj")
+    if traj is not None:
+        used = sum(8 * v.numel() for v in out.values())
+        j = pick(int(traj.shape[2]), 8 * (traj.shape[0] * traj.shape[1] + 1), DUMP_BYTES - used)
+        out["traj"] = traj[:, :, j.to(traj.device)]
+        out["traj_index"] = j + traj_offset
+    os.makedirs(dirname, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(dirname, f"{k}.npy"), v.cpu().numpy().astype(np.float64))
 
 
 def bind_to_gpu_numa_node(index):
@@ -223,6 +254,9 @@ def run_reference(args, rank, world):
         nconv += int((st == 0).sum()); iters += it.tolist()
     wall = time.perf_counter() - t0
     pool.close()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"tf": torch.from_numpy(tf), "status": torch.from_numpy(st),
+                                         "iterations": torch.from_numpy(it)})
     val = nconv / wall
     kind = "reference" if gekko_ok else "port"
     sample = f"{per_step} problems per step (one per host core) of the seed-11 cfg{args.config} dispersions, nt={nt}, tol={opts.tol:g}"
@@ -262,7 +296,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-traj", action="store_true", help="do not materialise the [10,nt,B] trajectory block")
     ap.add_argument("--no-weak", action="store_true", help="skip the additional weak-scaling measurement at N>1")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.batch is None:
         args.batch = 65536 if args.config == 4 else 4096
     if args.nt is None:
@@ -356,6 +394,9 @@ def main():
         launches_all = int(launches)
     conv_all, iters_all = float(conv), float(iters_total)
     value = conv_all / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # `raw` is the last timed step's result: every problem's scalars, this rank's trajectory shard [lo, hi)
+        dump_outputs(args.dump_outputs, raw, lo)
 
     # ---- end-to-end through the host API (pinned host tensors in, pinned host tensors out), this rank's shard ----
     shard_hosts = [r[:, lo:hi].contiguous().pin_memory() for r in rows_hosts]

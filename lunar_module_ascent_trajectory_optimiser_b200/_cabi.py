@@ -8,6 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import shutil
 import subprocess
 import sys
 from typing import Optional
@@ -50,6 +51,18 @@ class LmatoError(RuntimeError):
 LAST_BUILD = {"action": None, "seconds": 0.0}     # what the last build_library() call did: "compiled" | "reused"
 
 
+def cuda_tool(name: str) -> str:
+    """Path of a CUDA toolkit program (``nvcc``, ``cuobjdump``): from PATH, else from ``$CUDA_HOME/bin``,
+    ``$CUDA_PATH/bin`` or ``/usr/local/cuda/bin``, so that a shell whose PATH lacks the toolkit still builds."""
+    found = shutil.which(name)
+    if found:
+        return found
+    for root in (os.environ.get("CUDA_HOME"), os.environ.get("CUDA_PATH"), "/usr/local/cuda"):
+        if root and os.access(os.path.join(root, "bin", name), os.X_OK):
+            return os.path.join(root, "bin", name)
+    raise LmatoError(f"{name} not found on PATH, in $CUDA_HOME/bin, $CUDA_PATH/bin or /usr/local/cuda/bin")
+
+
 def build_library(force: bool = False, verbose: bool = False) -> str:
     """Compile csrc/ascent_cabi.cu for sm_100a into the in-tree shared library (or reuse it if it is newer than
     every source; ``LAST_BUILD`` says which)."""
@@ -61,7 +74,7 @@ def build_library(force: bool = False, verbose: bool = False) -> str:
         if all(os.path.getmtime(LIB_PATH) >= os.path.getmtime(s) for s in srcs):
             LAST_BUILD.update(action="reused", seconds=0.0)
             return LIB_PATH
-    cmd = ["nvcc"] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + \
+    cmd = [cuda_tool("nvcc")] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + \
           ["-o", LIB_PATH, os.path.join(CSRC, "ascent_cabi.cu")]
     t0 = _time.time()
     r = subprocess.run(cmd, capture_output=True, text=True)

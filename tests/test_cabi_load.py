@@ -29,7 +29,8 @@ def test_header_functions_are_exported(built_lib):
 
 
 def test_library_is_sm100a_and_has_no_torch_types(built_lib):
-    out = subprocess.run(["cuobjdump", "-lelf", built_lib], capture_output=True, text=True).stdout
+    from lunar_module_ascent_trajectory_optimiser_b200 import _cabi
+    out = subprocess.run([_cabi.cuda_tool("cuobjdump"), "-lelf", built_lib], capture_output=True, text=True).stdout
     assert "sm_100a" in out, out
     nm = subprocess.run(["nm", "-D", "--defined-only", built_lib], capture_output=True, text=True).stdout
     exported = [l.split()[-1] for l in nm.splitlines() if " T " in l]
