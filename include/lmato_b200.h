@@ -124,7 +124,9 @@ typedef struct {
  *           problem, needs ~37 888 problems in flight to fill a B200;
  *   COOP    eight lanes of a warp per problem, stage-parallel model evaluation, cost-to-go distributed by rows:
  *           short critical path per problem, fills the GPU with ~4 700 problems;
- *   AUTO    COOP up to 24 576 problems per call, THREAD above. */
+ *   AUTO    COOP up to 6 144 problems per call, THREAD above; the circular model with its move term (dcost > 0) always
+ *           runs on COOP.  COOP takes 32 lanes per problem up to 8 problems per SM and 8 lanes above that, and
+ *           two CTAs per SM once one CTA per SM cannot hold the whole batch. */
 typedef enum { LMATO_KERNEL_AUTO = 0, LMATO_KERNEL_THREAD = 1, LMATO_KERNEL_COOP = 2 } lmato_kernel_t;
 
 /* Fill `o` with the defaults above. */
@@ -199,7 +201,10 @@ lmato_status_t lmato_set_initial_guess(lmato_handle* h, const double* guess_traj
  * (tf in the reference's scaled units, parameter in the units of the params block) for the parameters of
  * lmato_sens_t, from the multipliers at the solution (envelope theorem; costs one pass over the converged
  * iterate).  A DEVICE pointer for lmato_solve_batch, a HOST pointer for lmato_solve_batch_host; NULL (the
- * default) switches the output off.  Entries of problems that did not converge are meaningless. */
+ * default) switches the output off.  Entries of problems that did not converge are meaningless.  For
+ * LMATO_MODEL_CIRCULAR the LMATO_S_ANGLE_DOUBLEDOT_MAX entry is NaN: that model has no pitch-acceleration limit
+ * (its MV is the pitch angle itself, PDF p.27), so tf does not depend on that row of the params block; the other
+ * three entries are computed as for the elliptical model. */
 #define LMATO_NSENS 4
 typedef enum lmato_sens {
   LMATO_S_FT = 0,                   /* thrust Ft (LO:61) */

@@ -155,7 +155,8 @@ class AscentBatchSolution:
     kkt_error: torch.Tensor          # [B]
     time: torch.Tensor               # [nt] normalised mesh (m.time)
     # optional: d tf / d parameter, name -> [B] (scaled tf per unit of the raw parameter), for
-    # Ft, M0, M_dot, angle_doubledot_max; only with ``sensitivities=True``
+    # Ft, M0, M_dot, angle_doubledot_max (NaN for the circular model, which has no such limit); only with
+    # ``sensitivities=True``
     dtf_dparam: Optional[Dict[str, torch.Tensor]] = None
     # which reference variable `control` is: the MV `angledoubledot` (LO:96) or, for the circular model, the MV
     # `angle` (PDF p.27 src 69-73)

@@ -216,7 +216,8 @@ __device__ __noinline__ void write_results(const KArgs& a, const Params& P, cons
     a.sens[(long)LMATO_S_FT * B + b] = s_ft * inv;
     a.sens[(long)LMATO_S_M0 * B + b] = s_m0 * inv;
     a.sens[(long)LMATO_S_M_DOT * B + b] = s_mf * inv / P.fuel;
-    a.sens[(long)LMATO_S_ANGLE_DOUBLEDOT_MAX * B + b] = s_asc * inv / 3.0;
+    // the circular model has no pitch-acceleration limit (its MV is the angle): no such derivative exists there
+    a.sens[(long)LMATO_S_ANGLE_DOUBLEDOT_MAX * B + b] = a.model == LMATO_MODEL_CIRCULAR ? NAN : s_asc * inv / 3.0;
   }
 }
 
@@ -394,7 +395,7 @@ __device__ __noinline__ void coop_write_results(const KArgs& a, const Params& P,
       a.sens[(long)LMATO_S_FT * B + b] = s_ft * inv;
       a.sens[(long)LMATO_S_M0 * B + b] = s_m0 * inv;
       a.sens[(long)LMATO_S_M_DOT * B + b] = s_mf * inv / P.fuel;
-      a.sens[(long)LMATO_S_ANGLE_DOUBLEDOT_MAX * B + b] = s_asc * inv / 3.0;
+      a.sens[(long)LMATO_S_ANGLE_DOUBLEDOT_MAX * B + b] = a.model == LMATO_MODEL_CIRCULAR ? NAN : s_asc * inv / 3.0;
     }
   }
 }

@@ -69,7 +69,7 @@ def main():
              final_mass=np.array(fms), traj=np.stack(trajs), names=np.array(VAR_ROWS))
 
 
-if __name__ == "__main__" and not any(a in sys.argv for a in ("--dense", "--dcost", "--sens", "--nodes", "--config3", "--circular-dcost", "--config4")):
+if __name__ == "__main__" and not any(a in sys.argv for a in ("--dense", "--dcost", "--sens", "--nodes", "--config3", "--circular-dcost", "--config4", "--coarse", "--sens-batch")):
     main()
 
 
@@ -267,3 +267,110 @@ def config4_slice(B=512, stride=20):
 
 if __name__ == "__main__" and "--config4" in sys.argv:
     config4_slice()
+
+
+def _oracle_one(args):
+    """One oracle solve for the pooled modes below: (key, AscentParams, nt) -> key, tf, final mass, trajectory,
+    iterations, KKT error.  Other start times are tried when the first stops short (no restoration phase)."""
+    key, p, nt = args
+    nlp = AscentNLP(p, nt=nt, obj_scale=10.0)
+    r = None
+    for tf0 in (0.9, 0.95, 0.85, 0.92):
+        r = solve_ipm(nlp, nlp.initial_guess(tf0), IPMOptions(tol=1e-12, max_iter=500))
+        if r.status == 0:
+            break
+    nv = nlp.node_values(r.x)
+    traj = np.stack([nv[n] for n in VAR_ROWS if n in nv])
+    return key, nv["tf"], p.M0 - p.fuel_mass * nv["mass"][-1], traj, r.iterations, r.kkt_error, r.status
+
+
+def _pool_map(jobs):
+    import multiprocessing as mp
+    with mp.Pool(int(os.environ.get("GOLDEN_PROCS", os.cpu_count()))) as pool:
+        return {r[0]: r[1:] for r in pool.imap_unordered(_oracle_one, jobs, chunksize=1)}
+
+
+COARSE_CASES = [(nt, dc) for nt in (4, 5, 9, 17, 33) for dc in (0.0, 1e-5)] + [(3, 1e-5)]
+
+
+def coarse():
+    """Coarse meshes: the nominal problem at nt = 4, 5, 9, 17, 33, each without and with DCOST = 1e-5, and nt = 3
+    with DCOST only (without it the oracle's line search fails there, status 2).  Meshes this small leave lanes of
+    the cooperative kernel without a stage and let its record ring prefetch past the last stage.  Kept per case: tf,
+    final mass, all ten variables at every node, iterations and KKT error (converged to 1e-12).
+
+        python tests/golden/make_golden.py --coarse        (11 oracle solves; 7 s on 8 CPU cores)
+    """
+    import dataclasses
+    jobs = [(i, dataclasses.replace(AscentParams(), dcost=dc), nt) for i, (nt, dc) in enumerate(COARSE_CASES)]
+    res = _pool_map(jobs)
+    out = dict(nt=np.array([c[0] for c in COARSE_CASES]), dcost=np.array([c[1] for c in COARSE_CASES]),
+               names=np.array(VAR_ROWS))
+    for k in ("tf", "final_mass", "iters", "kkt"):
+        out[k] = np.array([res[i][("tf", "final_mass", "traj", "iters", "kkt").index(k)] for i in range(len(jobs))])
+    for i in range(len(jobs)):
+        tf, fm, traj, it, kkt, st = res[i]
+        assert st == 0, (COARSE_CASES[i], st, kkt)
+        out[f"traj_{i}"] = traj
+        print("coarse nt", COARSE_CASES[i][0], "dcost", COARSE_CASES[i][1], "tf", tf, "iters", it, "kkt", kkt)
+    np.savez(os.path.join(HERE, "elliptical_coarse_nt3to33.npz"), **out)
+
+
+if __name__ == "__main__" and "--coarse" in sys.argv:
+    coarse()
+
+
+SENS_NAMES = ["Ft", "M0", "M_dot", "angle_doubledot_max"]
+SENS_STEPS = {"Ft": 1e-4, "M0": 1e-4, "M_dot": 1e-4, "angle_doubledot_max": 1e-3}   # relative, as --sens
+
+
+def sens_batch(B=6):
+    """d tf / d (Ft, M0, M_dot, angle_doubledot_max) for the first 6 problems of the config-4 draws
+    (dispersed_params(., seed=11), problem 0 = the nominal case) at nt = 200, with DCOST = 1e-5 and without it, by
+    central differences of oracle solves (relative steps of --sens); and d tf / d (Ft, M0, M_dot) of the circular
+    model's nominal case, with and without its DCOST.  tf at both ends of every difference is kept, so that a test can
+    bound the truncation error by |forward - backward| difference quotient.
+
+        python tests/golden/make_golden.py --sens-batch    (122 oracle solves; 2 min on 8 CPU cores)
+    """
+    import dataclasses
+    import torch  # noqa: F401
+    from lunar_module_ascent_trajectory_optimiser_b200.dispersions import dispersed_params
+    rows = dispersed_params(B, seed=11).rows(B).numpy()
+    dcosts = [1e-5, 0.0]
+    base = [[AscentParams(Ft=rows[3, b], M0=rows[4, b], M_dot=rows[5, b], angle_doubledot_max=rows[7, b],
+                          r_periapsis=rows[8, b], r_apoapsis=rows[9, b], dcost=dc) for b in range(B)] for dc in dcosts]
+    circ = [dataclasses.replace(AscentParams.circular(), dcost=dc) for dc in dcosts]
+    step = np.array([[SENS_STEPS[n] * getattr(base[0][b], n) for n in SENS_NAMES] for b in range(B)])   # [B, 4]
+    cstep = np.array([SENS_STEPS[n] * getattr(circ[0], n) for n in SENS_NAMES[:3]])
+    jobs = []
+    for d in range(len(dcosts)):
+        for b in range(B):
+            p = base[d][b]
+            jobs.append((("e", d, b, -1, 0), p, 200))
+            for j, n in enumerate(SENS_NAMES):
+                for s in (1, -1):
+                    jobs.append((("e", d, b, j, s), dataclasses.replace(p, **{n: getattr(p, n) + s * step[b, j]}), 200))
+        p = circ[d]
+        jobs.append((("c", d, 0, -1, 0), p, 200))
+        for j, n in enumerate(SENS_NAMES[:3]):
+            for s in (1, -1):
+                jobs.append((("c", d, 0, j, s), dataclasses.replace(p, **{n: getattr(p, n) + s * cstep[j]}), 200))
+    res = _pool_map(jobs)
+    assert max(r[4] for r in res.values()) < 1e-9, max(r[4] for r in res.values())
+    tf = np.array([[res[("e", d, b, -1, 0)][0] for b in range(B)] for d in range(2)])
+    up = np.array([[[res[("e", d, b, j, 1)][0] for j in range(4)] for b in range(B)] for d in range(2)])
+    dn = np.array([[[res[("e", d, b, j, -1)][0] for j in range(4)] for b in range(B)] for d in range(2)])
+    ctf = np.array([res[("c", d, 0, -1, 0)][0] for d in range(2)])
+    cup = np.array([[res[("c", d, 0, j, 1)][0] for j in range(3)] for d in range(2)])
+    cdn = np.array([[res[("c", d, 0, j, -1)][0] for j in range(3)] for d in range(2)])
+    kkt = max(r[4] for r in res.values())
+    np.savez(os.path.join(HERE, "sens_disp6_seed11_nt200.npz"), names=np.array(SENS_NAMES), rows=rows,
+             dcost=np.array(dcosts), step=step, tf=tf, tf_up=up, tf_dn=dn, dtf=(up - dn) / (2 * step),
+             circ_step=cstep, circ_tf=ctf, circ_tf_up=cup, circ_tf_dn=cdn, circ_dtf=(cup - cdn) / (2 * cstep),
+             max_kkt=kkt)
+    print("sens batch: dtf", (up - dn) / (2 * step), "circular", (cup - cdn) / (2 * cstep), "max kkt", kkt)
+
+
+if __name__ == "__main__" and "--sens-batch" in sys.argv:
+    sens_batch()

@@ -95,12 +95,13 @@ def test_cooperative_sweeps_source_matches_goldens_and_thread_sweeps(hostsim, mo
     monkeypatch.delenv("CIRCULAR", raising=False)
     monkeypatch.delenv("NPOL", raising=False)
 
-    def both(raw, gold_tf, gold_traj=None, **kw):
+    def both(raw, gold_tf, gold_traj=None, tf_rtol=1e-8, iter_tol=1, **kw):
         a = _solve(hostsim, raw, fn="hostsim_solve", **kw)
         b = _solve(hostsim, raw, fn="hostsim_solve_coop", **kw)
         assert a[0] == 0 and b[0] == 0
-        assert abs(b[1] - gold_tf) / gold_tf < 1e-8 and abs(a[1] - b[1]) / a[1] < 1e-11
-        assert abs(a[2] - b[2]) <= 1, (a[2], b[2])                    # iterations
+        assert abs(a[1] - gold_tf) / gold_tf < tf_rtol and abs(b[1] - gold_tf) / gold_tf < tf_rtol
+        assert abs(a[1] - b[1]) / a[1] < 1e-11
+        assert abs(a[2] - b[2]) <= iter_tol, (a[2], b[2])             # iterations
         if gold_traj is not None:
             err = _rel(b[3], gold_traj)
             assert err[:9].max() < 1e-4 and err[9] < 2e-4, err
@@ -118,6 +119,18 @@ def test_cooperative_sweeps_source_matches_goldens_and_thread_sweeps(hostsim, mo
     for b in range(4):
         both(g["rows"][:, b], g["tf"][b], g["traj"][b])
     monkeypatch.delenv("WDC"); monkeypatch.delenv("NPOL")
+    # coarse meshes (nt = 3..33): a cooperative group then has lanes without a stage and its record ring prefetches
+    # past the last stage; the move weight is per step of THIS mesh (objective_nodes = nt - 1, as the device sets it)
+    g = np.load(os.path.join(GOLDEN, "elliptical_coarse_nt3to33.npz"))
+    for i, (nt, dc) in enumerate(zip(g["nt"].tolist(), g["dcost"].tolist())):
+        if dc > 0:
+            monkeypatch.setenv("WDC", repr(10.0 * dc / (nt - 1))); monkeypatch.setenv("NPOL", "2")
+        # nt = 5 with DCOST spends ~50 iterations at mu = 0.1 under inertia correction, where rounding differences
+        # grow ~10x per iteration: thrust moved by up to 3 ulp gives either sweep order anywhere from 55 to 73 iterations
+        # (the unperturbed problem: 61 and 56).  Every other case agrees to one iteration.
+        both(NOMINAL, float(g["tf"][i]), g[f"traj_{i}"], tf_rtol=5e-13, iter_tol=8 if (nt, dc > 0) == (5, True) else 1,
+             nt=nt)
+        monkeypatch.delenv("WDC", raising=False); monkeypatch.delenv("NPOL", raising=False)
     g = np.load(os.path.join(GOLDEN, "circular_nominal_nt200.npz"))
     monkeypatch.setenv("CIRCULAR", "1")
     raw = NOMINAL.copy(); raw[8] = raw[9] = 53108.4; raw[11] = 2576.0
