@@ -22,9 +22,8 @@
 #include <vector>
 
 #include "../../include/lmato_b200.h"
-#include "ascent_ipm_dc.cuh"
-#include "ascent_coop.cuh"
 #include "ascent_colloc.cuh"
+#include "ascent_result.cuh"
 
 using namespace lmato;
 
@@ -61,14 +60,7 @@ constexpr long kWarmStartMinBatch = 512;
 
 struct KArgs {
   const double* params;  // [NPARAM][B]
-  long B;
-  double* traj;          // [NVAR][nt][B] or null
-  double* tf;
-  double* fmass;
-  int* status;
-  int* iters;
-  double* kkt;
-  double* sens;          // [LMATO_NSENS][B] d tf / d parameter, or null
+  ResultOut res;         // the outputs; res.B is the batch size B of every [..][B] array here
   const double* guess_traj;  // caller-supplied start point [NVAR][nt][B] and [B], or null
   const double* guess_tf;
   double* ws;            // [N+1][slots/32][N_FIELDS][32]
@@ -100,42 +92,6 @@ __global__ void __launch_bounds__(256) mean_params_kernel(const double* __restri
   if (threadIdx.x == 0) out[row] = red[0] / (double)B;
 }
 
-__device__ __forceinline__ Params derive_params(const double* __restrict__ p, long B, long b, int model, bool move = false) {
-  // LO:50-75, 107-109
-  Params P;
-  const double G = p[LMATO_P_G * B + b], Mm = p[LMATO_P_M * B + b];
-  const double R0 = p[LMATO_P_R0 * B + b];
-  const double fuel = p[LMATO_P_FUEL_MASS * B + b];
-  const double rp = p[LMATO_P_R_PERIAPSIS * B + b], ra = p[LMATO_P_R_APOAPSIS * B + b];
-  P.GM = G * Mm;
-  P.R0 = R0;
-  P.Ft = p[LMATO_P_FT * B + b];
-  P.M0 = p[LMATO_P_M0 * B + b];
-  P.S = rp;
-  P.ms = p[LMATO_P_MASS_SCALAR * B + b];
-  P.mflow = p[LMATO_P_M_DOT * B + b] / fuel;
-  P.asc = p[LMATO_P_ANGLE_DOUBLEDOT_MAX * B + b] / 3.0;
-  P.T = p[LMATO_P_FINAL_TIME * B + b];
-  P.a_ub = p[LMATO_P_ANGLE_UB * B + b];
-  P.u_ub = p[LMATO_P_U_BOUND * B + b];
-  const double vt = sqrt(P.GM / (R0 + 0.5 * (rp + ra)));
-  P.vt2 = (vt / P.S) * (vt / P.S);
-  P.rt = (R0 + P.S) / P.S;
-  P.R0S = R0 / P.S;
-  P.tf_ub = fmin(1.0, 1.0 / (P.mflow * P.T));
-  P.fuel = fuel;
-  P.Sinv = 1.0 / P.S;
-  P.coup5 = 1.0;
-  P.mT = P.mflow * P.T;
-  if (model == LMATO_MODEL_CIRCULAR) {
-    // PDF p.27 src 69-73: the MV is the pitch angle itself; no rate or acceleration limit exists
-    P.coup5 = 0.0;
-    P.asc = move ? 0.0 : 1.0;     // with the move term the MV slot holds the pitch angle itself (mv_is_angle())
-    P.u_ub = 1e20;
-  }
-  return P;
-}
-
 // Params padded to an odd number of doubles per thread so that the per-thread structs in shared memory
 // are bank-conflict free (Params = 19 doubles -> stride 21 doubles = 42 words; 42 mod 32 = 10).
 struct alignas(8) ParamsSlot { Params p; double pad[(sizeof(Params) / 8) % 2 == 0 ? 1 : 2]; };
@@ -144,82 +100,6 @@ static_assert(GuessSrc::V_Y == LMATO_V_Y && GuessSrc::V_YDOT == LMATO_V_YDOT && 
               GuessSrc::V_XDOT == LMATO_V_XDOT && GuessSrc::V_ANGLE == LMATO_V_ANGLE &&
               GuessSrc::V_ANGLEDOT == LMATO_V_ANGLEDOT && GuessSrc::V_U == LMATO_V_ANGLEDOUBLEDOT,
               "the guess uses the output layout of include/lmato_b200.h");
-
-// Results of one finished problem (LO:178-202: tf, the per-node values of all ten variables, final
-// mass, status).  The iterate is read back from the thread's workspace column; ydoubledot,
-// xdoubledot and mass, which the device formulation eliminates, are recomputed (LO:123, 127-136).
-template <class SW>
-__device__ __noinline__ void write_results(const KArgs& a, const Params& P, const Ws& W, const IpmState& S, long b) {
-  SolveOut out;
-  ipm_result(S, out);
-  const int nt = a.N + 1;
-  a.tf[b] = out.tf;
-  a.fmass[b] = P.M0 - P.fuel * (P.mflow * P.T * out.tf);   // mass(nt-1) = mflow*T*tf (LO:123)
-  a.status[b] = out.status;
-  a.iters[b] = out.iters;
-  if (a.kkt) a.kkt[b] = out.kkt;
-  if (!a.traj && !a.sens) return;
-  double* __restrict__ t = a.traj;
-  const long B = a.B;
-  if (t) {
-#pragma unroll
-    for (int v = 0; v < LMATO_NVAR; ++v) t[((long)v * nt) * B + b] = 0.0;   // node 0 pinned
-  }
-  // Parametric sensitivity of the optimum (envelope theorem): d objective* / d theta = d Lagrangian / d theta
-  // = sum_k lambda_k . d c_k / d theta at the solution, with c_k = s_k - s_{k-1} - h_k T tf F(s_k, u_k; theta).
-  // theta enters only the velocity rows (through the thrust acceleration Ft / (M0 - ms*mass), LO:127-136,
-  // and mass = mflow*T*tau*tf, LO:123) and the angledot row (angle_scalar, LO:121).
-  double s_ft = 0.0, s_m0 = 0.0, s_mf = 0.0, s_asc = 0.0;
-  for (int k = 1; k <= a.N; ++k) {
-    const double* sp = W.stage(k);
-    double z[6];
-#pragma unroll
-    for (int i = 0; i < 6; ++i) z[i] = WS_AT(sp, out.cur * SW::NITER + SW::FZ + i);
-    const double u = WS_AT(sp, out.cur * SW::NITER + SW::FU);
-    const double m = P.mflow * P.T * a.tau[k] * out.tf;
-    double ay, ax;
-    if (a.sens) {
-      Accel1 f;
-      accel_first(P, z[0], z[2], z[4], m, f);
-      ay = f.ay; ax = f.ax;
-      const double al = a.h[k] * P.T * out.tf;
-      const double l1 = WS_AT(sp, out.cur * SW::NITER + SW::FLAM + 1);     // multiplier of the ydot row
-      const double l3 = WS_AT(sp, out.cur * SW::NITER + SW::FLAM + 3);     // xdot row
-      const double l5 = WS_AT(sp, out.cur * SW::NITER + SW::FLAM + 5);     // angledot row
-      const double thrust = l1 * (f.AT * f.Ty * P.Sinv) + l3 * (f.AT * f.Tx * P.Sinv);
-      s_ft -= al * thrust / P.Ft;
-      s_m0 += al * thrust * (f.AT / P.Ft);                                  // d AT / d M0 = -AT / (M0 - ms*mass)
-      s_mf -= al * (l1 * f.ay_m + l3 * f.ax_m) * (P.T * a.tau[k] * out.tf);
-      s_asc -= al * u * l5;
-    } else {
-      accel_value(P, z[0], z[2], z[4], m, ay, ax);
-    }
-    if (!t) continue;
-    t[((long)LMATO_V_Y * nt + k) * B + b] = z[0];
-    t[((long)LMATO_V_YDOT * nt + k) * B + b] = z[1];
-    t[((long)LMATO_V_YDOUBLEDOT * nt + k) * B + b] = ay;
-    t[((long)LMATO_V_X * nt + k) * B + b] = z[2];
-    t[((long)LMATO_V_XDOT * nt + k) * B + b] = z[3];
-    t[((long)LMATO_V_XDOUBLEDOT * nt + k) * B + b] = ax;
-    t[((long)LMATO_V_ANGLE * nt + k) * B + b] = z[4];
-    t[((long)LMATO_V_ANGLEDOT * nt + k) * B + b] = z[5];
-    t[((long)LMATO_V_MASS * nt + k) * B + b] = m;
-    t[((long)LMATO_V_ANGLEDOUBLEDOT * nt + k) * B + b] = u;
-  }
-  if (a.sens) {
-    // per unit of the RAW parameters of include/lmato_b200.h: M_dot = mflow * fuel_mass (LO:65),
-    // angle_doubledot_max = 3 * angle_scalar (LO:109); tf in the reference's scaled units (0..1)
-    const double inv = 1.0 / a.O.obj_scale;
-    // the mass bound 0 <= mass <= 1 (LO:83) is carried as tf <= tf_ub = 1 / (mflow T): where that is the binding
-    // upper bound on tf, its multiplier contributes  -zUt * d tf_ub / d mflow = zUt / (mflow^2 T)
-    if (P.tf_ub < 1.0) s_mf += S.cur.zUt / (P.mflow * P.mflow * P.T);
-    a.sens[(long)LMATO_S_FT * B + b] = s_ft * inv;
-    a.sens[(long)LMATO_S_M0 * B + b] = s_m0 * inv;
-    a.sens[(long)LMATO_S_M_DOT * B + b] = s_mf * inv / P.fuel;
-    // the circular model has no pitch-acceleration limit (its MV is the angle): no such derivative exists there
-    a.sens[(long)LMATO_S_ANGLE_DOUBLEDOT_MAX * B + b] = a.model == LMATO_MODEL_CIRCULAR ? NAN : s_asc * inv / 3.0;
-  }
-}
 
 // SW = Sweeps7 (dcost = 0) or Sweeps8 (with the reference's move-suppression term, LO:99)
 template <class SW>
@@ -262,7 +142,7 @@ __global__ void __launch_bounds__(kBlock, kBlocksPerSM) ascent_ipm_kernel(KArgs 
     //      [variable][node][problem] output is then one coalesced 256-byte store per warp (the output
     //      may be pinned host memory written over PCIe while the other warps keep computing) ----
     if (chunk_done && __any_sync(0xffffffffu, pending)) {
-      if (pending) write_results<SW>(a, P, W, S, b);
+      if (pending) write_results<SW, 1>(a.res, P, M, O.obj_scale, a.model, W, 0, 1u << lane, S, b);
       pending = false;
     }
     if (!exhausted && chunk_done) {
@@ -276,19 +156,19 @@ __global__ void __launch_bounds__(kBlock, kBlocksPerSM) ascent_ipm_kernel(KArgs 
         if (lane == 0) chunk = atomicAdd(a.counter, 1) + gridDim.x * warps_per_block;
         chunk = __shfl_sync(0xffffffffu, chunk, 0);
       }
-      if ((long)chunk * 32 >= a.B) {
+      if ((long)chunk * 32 >= a.res.B) {
         exhausted = true;
       } else {
         b = (long)chunk * 32 + lane;
-        if (b < a.B) {
-          P = derive_params(a.params, a.B, b, a.model);
+        if (b < a.res.B) {
+          P = derive_params(a.params, a.res.B, b, a.model);
           ipm_begin(O, S);
           double mu0 = 0.0;
           // ref_mode 2: start from the batch reference.  ref_mode 1 (the reference solve itself):
           // start from the previous call's reference if the handle has one (consecutive batches of a
           // campaign have nearly the same mean, so it re-converges in one or two iterations).
           if (a.guess_traj) {
-            SW::guess_from(P, M, O, W, GuessSrc{a.guess_traj, a.guess_tf, a.B, b}, S.cur);
+            SW::guess_from(P, M, O, W, GuessSrc{a.guess_traj, a.guess_tf, a.res.B, b}, S.cur);
             S.from_guess = true;
           } else if (a.ref_mode != 0 && SW::load_ref(P, M, O, W, a.ref, S.cur, &mu0)) {
             S.warm = true;
@@ -333,73 +213,6 @@ constexpr int kCoopG = 8;
 constexpr int kCoopScrStride = coop::SCR_DOUBLES;       // per group: record ring + transpose tiles (even: 16-byte aligned)
 static size_t coop_smem(int gp) { return sizeof(double) * (size_t)(kCoopBlock / gp) * kCoopScrStride; }
 
-template <int G, class CW>
-__device__ __noinline__ void coop_write_results(const KArgs& a, const Params& P, const CW& W, const IpmState& S, long b) {
-  SolveOut out;
-  ipm_result(S, out);
-  const int nt = a.N + 1;
-  const long B = a.B;
-  if (W.g == 0) {
-    a.tf[b] = out.tf;
-    a.fmass[b] = P.M0 - P.fuel * (P.mflow * P.T * out.tf);   // mass(nt-1) = mflow*T*tf (LO:123)
-    a.status[b] = out.status;
-    a.iters[b] = out.iters;
-    if (a.kkt) a.kkt[b] = out.kkt;
-  }
-  if (!a.traj && !a.sens) return;
-  double* __restrict__ t = a.traj;
-  if (t) {
-    for (int v = W.g; v < LMATO_NVAR; v += G) t[((long)v * nt) * B + b] = 0.0;   // node 0 pinned
-  }
-  // (see write_results above for the sensitivity formulas)
-  double s_ft = 0.0, s_m0 = 0.0, s_mf = 0.0, s_asc = 0.0;
-  for (int k = 1 + W.g; k <= a.N; k += G) {
-    double x[coop::XR];
-    coop::ldv<coop::XR>(W.X(out.cur, k), x);
-    const double* z = x + coop::X_Z;
-    const double u = x[coop::X_U];
-    const double m = P.mflow * P.T * a.tau[k] * out.tf;
-    double ay, ax;
-    if (a.sens) {
-      Accel1 f;
-      accel_first(P, z[0], z[2], z[4], m, f);
-      ay = f.ay; ax = f.ax;
-      const double al = a.h[k] * P.T * out.tf;
-      const double l1 = x[coop::X_LAM + 1], l3 = x[coop::X_LAM + 3], l5 = x[coop::X_LAM + 5];
-      const double thrust = l1 * (f.AT * f.Ty * P.Sinv) + l3 * (f.AT * f.Tx * P.Sinv);
-      s_ft -= al * thrust / P.Ft;
-      s_m0 += al * thrust * (f.AT / P.Ft);
-      s_mf -= al * (l1 * f.ay_m + l3 * f.ax_m) * (P.T * a.tau[k] * out.tf);
-      s_asc -= al * u * l5;
-    } else {
-      accel_value(P, z[0], z[2], z[4], m, ay, ax);
-    }
-    if (!t) continue;
-    t[((long)LMATO_V_Y * nt + k) * B + b] = z[0];
-    t[((long)LMATO_V_YDOT * nt + k) * B + b] = z[1];
-    t[((long)LMATO_V_YDOUBLEDOT * nt + k) * B + b] = ay;
-    t[((long)LMATO_V_X * nt + k) * B + b] = z[2];
-    t[((long)LMATO_V_XDOT * nt + k) * B + b] = z[3];
-    t[((long)LMATO_V_XDOUBLEDOT * nt + k) * B + b] = ax;
-    t[((long)LMATO_V_ANGLE * nt + k) * B + b] = z[4];
-    t[((long)LMATO_V_ANGLEDOT * nt + k) * B + b] = z[5];
-    t[((long)LMATO_V_MASS * nt + k) * B + b] = m;
-    t[((long)LMATO_V_ANGLEDOUBLEDOT * nt + k) * B + b] = u;
-  }
-  if (a.sens) {
-    s_ft = coop::Grp<G>::sum(W.mask, s_ft); s_m0 = coop::Grp<G>::sum(W.mask, s_m0);
-    s_mf = coop::Grp<G>::sum(W.mask, s_mf); s_asc = coop::Grp<G>::sum(W.mask, s_asc);
-    if (P.tf_ub < 1.0) s_mf += S.cur.zUt / (P.mflow * P.mflow * P.T);     // see write_results()
-    if (W.g == 0) {
-      const double inv = 1.0 / a.O.obj_scale;
-      a.sens[(long)LMATO_S_FT * B + b] = s_ft * inv;
-      a.sens[(long)LMATO_S_M0 * B + b] = s_m0 * inv;
-      a.sens[(long)LMATO_S_M_DOT * B + b] = s_mf * inv / P.fuel;
-      a.sens[(long)LMATO_S_ANGLE_DOUBLEDOT_MAX * B + b] = a.model == LMATO_MODEL_CIRCULAR ? NAN : s_asc * inv / 3.0;
-    }
-  }
-}
-
 // A warp holds 32/GP problems; its groups run the IPM driver in lock step (same sweep at the same time, each
 // with its own lane mask), finished groups idle until the warp's chunk is done, then the warp claims the next
 // chunk from the device-wide queue.  IpmState (filter, barrier parameter, ...) is carried redundantly by the
@@ -439,7 +252,7 @@ __global__ void __launch_bounds__(kCoopBlock, BPS) ascent_coop_kernel(KArgs a) {
   while (true) {
     const bool chunk_done = !__any_sync(0xffffffffu, active);
     if (chunk_done && __any_sync(0xffffffffu, pending)) {
-      if (pending) coop_write_results<GP>(a, P, W, S, b);
+      if (pending) write_results<SW, GP>(a.res, P, M, O.obj_scale, a.model, W, W.g, W.mask, S, b);
       pending = false;
     }
     if (!exhausted && chunk_done) {
@@ -451,17 +264,17 @@ __global__ void __launch_bounds__(kCoopBlock, BPS) ascent_coop_kernel(KArgs a) {
         if (lane == 0) chunk = atomicAdd(a.counter, 1) + gridDim.x * warps_per_block;
         chunk = __shfl_sync(0xffffffffu, chunk, 0);
       }
-      if ((long)chunk * PPW >= a.B) {
+      if ((long)chunk * PPW >= a.res.B) {
         exhausted = true;
       } else {
         b = (long)chunk * PPW + lane / GP;
-        if (b < a.B) {
-          if (W.g == 0) P = derive_params(a.params, a.B, b, a.model, MOVE == 2);
+        if (b < a.res.B) {
+          if (W.g == 0) P = derive_params(a.params, a.res.B, b, a.model, MOVE == 2);
           coop::Grp<GP>::sync(gmask);
           ipm_begin(O, S);
           double mu0 = 0.0;
           if (a.guess_traj) {
-            SW::guess_from(P, M, O, W, GuessSrc{a.guess_traj, a.guess_tf, a.B, b}, S.cur);
+            SW::guess_from(P, M, O, W, GuessSrc{a.guess_traj, a.guess_tf, a.res.B, b}, S.cur);
             S.from_guess = true;
           } else if (a.ref_mode != 0 && SW::load_ref(P, M, O, W, a.ref, S.cur, &mu0)) {
             S.warm = true;
@@ -515,41 +328,6 @@ static cudaError_t coop_optin() {
 // higher-order collocation kernel (NODES = 3..6, ascent_colloc.cuh): GP lanes per problem
 // ---------------------------------------------------------------------------------------
 template <int GP>
-__device__ __noinline__ void colloc_write_results(const KArgs& a, const Params& P, const colloc::Nws& W, const IpmState& S, long b) {
-  SolveOut out;
-  ipm_result(S, out);
-  const int nt = a.N + 1, m = W.L.m;
-  const long B = a.B;
-  if (W.g == 0) {
-    a.tf[b] = out.tf;
-    a.fmass[b] = P.M0 - P.fuel * (P.mflow * P.T * out.tf);
-    a.status[b] = out.status;
-    a.iters[b] = out.iters;
-    if (a.kkt) a.kkt[b] = out.kkt;
-  }
-  double* __restrict__ t = a.traj;
-  if (!t) return;
-  for (int v = W.g; v < LMATO_NVAR; v += GP) t[((long)v * nt) * B + b] = 0.0;   // node 0 pinned
-  for (int k = 1 + W.g; k <= a.N; k += GP) {
-    const double* xr = W.X(out.cur, k);
-    const double* z = xr + 6 * (m - 1);                  // the mesh node is the last collocation point of its step
-    const double ms = P.mflow * P.T * a.tau[k] * out.tf;
-    double ay, ax;
-    accel_value(P, z[0], z[2], z[4], ms, ay, ax);
-    t[((long)LMATO_V_Y * nt + k) * B + b] = z[0];
-    t[((long)LMATO_V_YDOT * nt + k) * B + b] = z[1];
-    t[((long)LMATO_V_YDOUBLEDOT * nt + k) * B + b] = ay;
-    t[((long)LMATO_V_X * nt + k) * B + b] = z[2];
-    t[((long)LMATO_V_XDOT * nt + k) * B + b] = z[3];
-    t[((long)LMATO_V_XDOUBLEDOT * nt + k) * B + b] = ax;
-    t[((long)LMATO_V_ANGLE * nt + k) * B + b] = z[4];
-    t[((long)LMATO_V_ANGLEDOT * nt + k) * B + b] = z[5];
-    t[((long)LMATO_V_MASS * nt + k) * B + b] = ms;
-    t[((long)LMATO_V_ANGLEDOUBLEDOT * nt + k) * B + b] = xr[W.L.x_u];
-  }
-}
-
-template <int GP>
 __global__ void __launch_bounds__(kCoopBlock, 1) ascent_colloc_kernel(KArgs a) {
   using SW = SweepsColloc<GP>;
   constexpr int PPW = 32 / GP;
@@ -579,7 +357,7 @@ __global__ void __launch_bounds__(kCoopBlock, 1) ascent_colloc_kernel(KArgs a) {
   while (true) {
     const bool chunk_done = !__any_sync(0xffffffffu, active);
     if (chunk_done && __any_sync(0xffffffffu, pending)) {
-      if (pending) colloc_write_results<GP>(a, P, W, S, b);
+      if (pending) write_results<SW, GP>(a.res, P, M, O.obj_scale, a.model, W, W.g, W.mask, S, b);
       pending = false;
     }
     if (!exhausted && chunk_done) {
@@ -591,12 +369,12 @@ __global__ void __launch_bounds__(kCoopBlock, 1) ascent_colloc_kernel(KArgs a) {
         if (lane == 0) chunk = atomicAdd(a.counter, 1) + gridDim.x * warps_per_block;
         chunk = __shfl_sync(0xffffffffu, chunk, 0);
       }
-      if ((long)chunk * PPW >= a.B) {
+      if ((long)chunk * PPW >= a.res.B) {
         exhausted = true;
       } else {
         b = (long)chunk * PPW + lane / GP;
-        if (b < a.B) {
-          if (W.g == 0) P = derive_params(a.params, a.B, b, a.model);
+        if (b < a.res.B) {
+          if (W.g == 0) P = derive_params(a.params, a.res.B, b, a.model);
           coop::Grp<GP>::sync(gmask);
           ipm_begin(O, S);
           variant = 0;
@@ -1010,8 +788,8 @@ lmato_status_t lmato_solve_batch(lmato_handle* h, const double* params, int64_t 
   h->ws_slots = slots;
   CUDA_TRY(cudaMemsetAsync(h->d_counter, 0, sizeof(int), st));
   KArgs a;
-  a.params = params; a.B = B; a.traj = out_traj; a.tf = out_tf; a.fmass = out_final_mass;
-  a.status = out_status; a.iters = out_iters; a.kkt = out_kkt; a.sens = h->sens_out;
+  a.params = params;
+  a.res = ResultOut{out_traj, out_tf, out_final_mass, out_status, out_iters, out_kkt, h->sens_out, (long)B};
   a.guess_traj = h->guess_traj; a.guess_tf = h->guess_tf;
   a.ws = h->d_ws; a.slots = slots; a.N = h->nt - 1; a.h = h->d_h; a.tau = h->d_tau;
   a.counter = h->d_counter;
@@ -1049,8 +827,8 @@ lmato_status_t lmato_solve_batch(lmato_handle* h, const double* params, int64_t 
     CUDA_TRY(cudaGetLastError());
     KArgs r = a;
     double* scratch = h->d_refparams + LMATO_NPARAM;
-    r.params = h->d_refparams; r.B = 1; r.traj = nullptr; r.tf = scratch; r.fmass = scratch + 1;
-    r.status = (int*)(scratch + 2); r.iters = (int*)(scratch + 3); r.kkt = scratch + 4; r.sens = nullptr;
+    r.params = h->d_refparams;
+    r.res = ResultOut{nullptr, scratch, scratch + 1, (int*)(scratch + 2), (int*)(scratch + 3), scratch + 4, nullptr, 1};
     r.guess_traj = nullptr; r.guess_tf = nullptr;
     r.ref = h->d_ref; r.ref_mode = 1;
     r.O.tol = 10.0 * h->opt.mu_ref; r.O.mu_min_factor = 0.1; r.O.n_polish = 0;

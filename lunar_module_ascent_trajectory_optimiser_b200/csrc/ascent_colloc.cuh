@@ -723,6 +723,16 @@ struct SweepsColloc {
   LM_HD static void guess_variant(const Params& P, const Mesh& M, const Options& O, const colloc::Nws& W, Scal& s, int variant) {
     colloc::colloc_init_guess<GP>(P, M, O, *W.C, W, s, variant);
   }
+  // node k of iterate `cur`: x = the six states and the control.  The multipliers of the collocation rows do not map
+  // onto one row per node, and the C ABI rejects sensitivities for NODES >= 3, so lam (if not null) is set to NaN.
+  LM_HD static void node(const colloc::Nws& W, int cur, int k, double* x, double* lam) {
+    const double* xr = W.X(cur, k);
+    if (x) {
+      for (int i = 0; i < 6; ++i) x[i] = xr[6 * (W.L.m - 1) + i];     // the mesh node is the last collocation point of its step
+      x[6] = xr[W.L.x_u];
+    }
+    if (lam) lam[0] = lam[1] = lam[2] = NAN;
+  }
   LM_HD static void remerit(const Mesh&, const Options&, const colloc::Nws&, int, double, Scal&) {}
 };
 

@@ -1337,6 +1337,16 @@ struct SweepsCoop {
                              Scal& s, double* mu) {
     return coop::coop_load_ref<GP, MOVE>(P, M, O, W, ref, s, mu);
   }
+  // node k of iterate `cur`: x = the six states and the control, lam = the multipliers of the ydot, xdot and angledot
+  // rows; either may be null
+  template <class CW>
+  LM_HD static void node(const CW& W, int cur, int k, double* x, double* lam) {
+    double r[coop::XR];
+    coop::ldv<coop::XR>(W.X(cur, k), r);
+    if (x) for (int i = 0; i < 7; ++i) x[i] = r[coop::X_Z + i];     // states, then X_U
+    if (!lam) return;
+    lam[0] = r[coop::X_LAM + 1]; lam[1] = r[coop::X_LAM + 3]; lam[2] = r[coop::X_LAM + 5];
+  }
   template <class CW>
   LM_HD static void remerit(const Mesh&, const Options&, const CW&, int, double, Scal&) {}
 };

@@ -1306,6 +1306,21 @@ LM_HD void ipm_begin(const Options& O, IpmState& S) {
   S.iters_prior = 0;
 }
 
+// Node k of iterate `cur` in a thread's workspace column with the iterate rows of SW (Sweeps7 / Sweeps8): x = the six
+// states and the control, lam = the multipliers of the ydot, xdot and angledot rows; either may be null.
+template <class SW>
+LM_HD void ws_node(const Ws& W, int cur, int k, double* x, double* lam) {
+  const double* sp = W.stage(k);
+  if (x) {
+    for (int i = 0; i < 6; ++i) x[i] = WS_AT(sp, cur * SW::NITER + SW::FZ + i);
+    x[6] = WS_AT(sp, cur * SW::NITER + SW::FU);
+  }
+  if (!lam) return;
+  lam[0] = WS_AT(sp, cur * SW::NITER + SW::FLAM + 1);
+  lam[1] = WS_AT(sp, cur * SW::NITER + SW::FLAM + 3);
+  lam[2] = WS_AT(sp, cur * SW::NITER + SW::FLAM + 5);
+}
+
 // Sweeps policy of the 7-state formulation (dcost = 0); ascent_ipm_dc.cuh provides the 8-state one.
 struct Sweeps7 {
   enum : int { NFIELDS = N_FIELDS, NITER = N_ITER, FZ = F_Z, FU = F_U, FLAM = F_LAM, REFROWS = REF_ROWS };
@@ -1332,6 +1347,7 @@ struct Sweeps7 {
                              double* mu) {
     return init_from_ref(P, M, W, ref, s, mu);
   }
+  LM_HD static void node(const Ws& W, int cur, int k, double* x, double* lam) { ws_node<Sweeps7>(W, cur, k, x, lam); }
   LM_HD static void remerit(const Mesh&, const Options&, const Ws&, int, double, Scal&) {}
 };
 

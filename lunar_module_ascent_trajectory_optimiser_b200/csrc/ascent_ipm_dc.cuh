@@ -823,6 +823,7 @@ struct Sweeps8 {
                              Scal& s, double* mu) {
     return dc::init_from_ref7(P, M, O, W, ref, s, mu);      // the reference is produced by the 7-state solve
   }
+  LM_HD static void node(const Ws& W, int cur, int k, double* x, double* lam) { ws_node<Sweeps8>(W, cur, k, x, lam); }
   LM_HD static void remerit(const Mesh&, const Options&, const Ws&, int, double, Scal&) {}
 };
 

@@ -19,6 +19,8 @@
 #pragma once
 #include <math.h>
 
+#include "../../include/lmato_b200.h"
+
 #if defined(__CUDACC__)
 #define LM_HD __host__ __device__ __forceinline__
 #define LM_D __device__ __forceinline__
@@ -69,6 +71,44 @@ struct Params {
   double mT;      // mflow * T: mass(tau) = mT * tau * tf (LO:123); read per stage, kept here so that it is a
                   // shared-memory load and not a spilled register
 };
+
+// Params of problem b from the raw parameter block [LMATO_NPARAM][B] of include/lmato_b200.h.  move: the circular
+// model with its move-suppression term (see coup5 above).
+LM_HD Params derive_params(const double* __restrict__ p, long B, long b, int model, bool move = false) {
+  // LO:50-75, 107-109
+  Params P;
+  const double G = p[LMATO_P_G * B + b], Mm = p[LMATO_P_M * B + b];
+  const double R0 = p[LMATO_P_R0 * B + b];
+  const double fuel = p[LMATO_P_FUEL_MASS * B + b];
+  const double rp = p[LMATO_P_R_PERIAPSIS * B + b], ra = p[LMATO_P_R_APOAPSIS * B + b];
+  P.GM = G * Mm;
+  P.R0 = R0;
+  P.Ft = p[LMATO_P_FT * B + b];
+  P.M0 = p[LMATO_P_M0 * B + b];
+  P.S = rp;
+  P.ms = p[LMATO_P_MASS_SCALAR * B + b];
+  P.mflow = p[LMATO_P_M_DOT * B + b] / fuel;
+  P.asc = p[LMATO_P_ANGLE_DOUBLEDOT_MAX * B + b] / 3.0;
+  P.T = p[LMATO_P_FINAL_TIME * B + b];
+  P.a_ub = p[LMATO_P_ANGLE_UB * B + b];
+  P.u_ub = p[LMATO_P_U_BOUND * B + b];
+  const double vt = sqrt(P.GM / (R0 + 0.5 * (rp + ra)));
+  P.vt2 = (vt / P.S) * (vt / P.S);
+  P.rt = (R0 + P.S) / P.S;
+  P.R0S = R0 / P.S;
+  P.tf_ub = fmin(1.0, 1.0 / (P.mflow * P.T));
+  P.fuel = fuel;
+  P.Sinv = 1.0 / P.S;
+  P.coup5 = 1.0;
+  P.mT = P.mflow * P.T;
+  if (model == LMATO_MODEL_CIRCULAR) {
+    // PDF p.27 src 69-73: the MV is the pitch angle itself; no rate or acceleration limit exists
+    P.coup5 = 0.0;
+    P.asc = move ? 0.0 : 1.0;     // with the move term the MV slot holds the pitch angle itself (mv_is_angle())
+    P.u_ub = 1e20;
+  }
+  return P;
+}
 
 // 1 in the circular model with the move term (the MV slot holds the pitch angle), else 0
 LM_HD double mv_is_angle(const Params& P) { return (P.coup5 == 0.0 && P.asc == 0.0) ? 1.0 : 0.0; }

@@ -1,10 +1,11 @@
 """The device solver's SOURCE, compiled for the host.
 
-`csrc/ascent_model.cuh`, `ascent_ipm.cuh` and `ascent_ipm_dc.cuh` are written so that g++ accepts them
-(tools/hostsim): the three sweeps, the IPM driver and the model derivatives below are the very lines the
-CUDA kernel inlines, executed by one CPU thread.  This gives the CPU-only test tier a check of the
-solver's logic against the oracle's golden vectors and of the hand-derived derivatives against finite
-differences.  It is test infrastructure only: the product has no CPU path (`_cabi.lib()` raises without
+`csrc/ascent_model.cuh`, `ascent_ipm.cuh`, `ascent_ipm_dc.cuh`, `ascent_coop.cuh`, `ascent_colloc.cuh` and
+`ascent_result.cuh` are written so that g++ accepts them (tools/hostsim): the parameter derivation, the sweeps, the
+IPM driver, the model derivatives and the result writer below are the very lines the CUDA kernels run, executed by
+one CPU thread.  This gives the CPU-only test tier a check of the solver's logic against the oracle's golden vectors,
+and of the hand-derived derivatives and the sensitivity output against finite differences.  It is test
+infrastructure only: the product has no CPU path (`_cabi.lib()` raises without
 the CUDA library), and nothing here is imported by the package.
 """
 import ctypes as C
@@ -147,6 +148,38 @@ def test_cooperative_sweeps_source_matches_goldens_and_thread_sweeps(hostsim, mo
         mine = traj[["y", "ydot", "ydoubledot", "x", "xdot", "xdoubledot", "angle", "angledot", "mass"].index(n)]
         assert np.abs(mine - ref).max() / np.abs(ref).max() < 1e-7, n
     assert np.array_equal(traj[9], traj[6]) and np.abs(traj[7]).max() == 0.0     # MV slot == angle, angledot pinned at 0
+
+
+def test_sensitivity_writer_matches_finite_differences(hostsim, monkeypatch):
+    """d tf / d parameter as the kernels' result writer (csrc/ascent_result.cuh) forms it, through the thread and the
+    cooperative workspace layouts, against the oracle's central differences (make_golden.py --sens-batch) with the
+    bounds of tests/test_gpu_kernel_matrix.py.  Both layouts read the multipliers of the same optimum."""
+    monkeypatch.delenv("CIRCULAR", raising=False)
+    monkeypatch.delenv("VREC", raising=False)
+    sg = np.load(os.path.join(GOLDEN, "sens_disp6_seed11_nt200.npz"))
+    for d, dcost in enumerate(sg["dcost"].tolist()):
+        if dcost > 0:
+            monkeypatch.setenv("WDC", repr(10.0 * dcost / 199)); monkeypatch.setenv("NPOL", "2")
+        else:
+            monkeypatch.delenv("WDC", raising=False); monkeypatch.delenv("NPOL", raising=False)
+        fd = sg["dtf"][d]                                                          # [6 problems, 4 parameters]
+        spread = np.abs(sg["tf_up"][d] - 2 * sg["tf"][d][:, None] + sg["tf_dn"][d]) / sg["step"] / np.abs(fd)
+        tol = np.full((6, 4), 3e-5 if dcost > 0 else 5e-6)
+        tol[:, 3] = 1e-5 + spread[:, 3]               # angle_doubledot_max: the quotient's one-sided spread (kinks in tf)
+        got = {}
+        for fn in ("hostsim_solve", "hostsim_solve_coop"):
+            got[fn] = np.full((6, 4), np.nan)
+            for b in range(6):
+                hostsim.hostsim_set_sensitivity_output(got[fn][b].ctypes.data_as(C.c_void_p))
+                try:
+                    assert _solve(hostsim, sg["rows"][:, b], fn=fn)[0] == 0
+                finally:
+                    hostsim.hostsim_set_sensitivity_output(None)
+            err = np.abs(got[fn] - fd) / np.abs(fd)
+            print(f"\n[sens] {fn} dcost {dcost}: worst per parameter {err.max(axis=0)} (err/tol {np.max(err / tol):.2f})")
+            assert np.all(err < tol), (fn, dcost, err, tol)
+        a, b = got["hostsim_solve"], got["hostsim_solve_coop"]
+        assert (np.abs(b - a) / np.abs(a)).max() < 1e-8, (dcost, a, b)
 
 
 def test_higher_order_collocation_source_matches_goldens(hostsim):

@@ -6,9 +6,10 @@ options, one of
     ascent_coop_kernel<G, GP, MOVE, BPS>          GP = 32 lanes per problem up to 8 problems per SM, else 8;
                                                   BPS = 2 CTAs per SM once one CTA per SM cannot hold the batch;
                                                   MOVE = 0 no DCOST, 1 DCOST, 2 the circular model with DCOST
-and every instantiation has its own start-point code (guess / guess_from / load_ref) and result writer (the thread
-kernel reads the multipliers through its workspace layout, the cooperative one sums them over the group).  The
-table below reaches each of them; a test id names the instantiation.  Batch sizes are derived from the device's SM
+and every instantiation has its own start-point code (guess / guess_from / load_ref) and reads the converged iterate
+through its own workspace layout (SW::node) for the shared result writer (csrc/ascent_result.cuh), which the
+cooperative kernels run with the problem's lanes summing over the group.  The table below reaches each of them; a
+test id names the instantiation.  Batch sizes are derived from the device's SM
 count with the dispatcher's rules, so the same table picks the same kernels on any GPU (a variant whose batch-size
 window is empty there is skipped).
 

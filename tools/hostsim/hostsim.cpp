@@ -14,21 +14,44 @@
 #include <cmath>
 #include <vector>
 #include <random>
-#include "ascent_ipm_dc.cuh"
+#include <array>
+#include "ascent_colloc.cuh"
+#include "ascent_result.cuh"
 
 using namespace lmato;
 
-static Params make_params(double Ft, double M0, double Mdot, double addm, double rp, double ra) {
-  Params P;
-  const double G = 6.674e-11, Mm = 7.346e22, R0 = 1738100.0, fuel = 2376.0, T = 470.0;
-  P.GM = G * Mm; P.R0 = R0; P.Ft = Ft; P.M0 = M0; P.S = rp; P.ms = fuel; P.mflow = Mdot / fuel;
-  P.asc = addm / 3.0; P.T = T; P.a_ub = M_PI / 3.0; P.u_ub = 1.0;
-  const double vt = std::sqrt(P.GM / (R0 + 0.5 * (rp + ra)));
-  P.vt2 = (vt / P.S) * (vt / P.S);
-  P.rt = (R0 + P.S) / P.S; P.R0S = R0 / P.S;
-  P.tf_ub = std::fmin(1.0, 1.0 / (P.mflow * T));
-  P.fuel = fuel; P.Sinv = 1.0 / P.S; P.coup5 = 1.0; P.mT = P.mflow * P.T;
-  return P;
+// Raw parameter column (include/lmato_b200.h) of the nominal problem with six of its values replaced.
+static std::array<double, LMATO_NPARAM> make_params(double Ft, double M0, double Mdot, double addm, double rp, double ra) {
+  std::array<double, LMATO_NPARAM> r;
+  r[LMATO_P_G] = 6.674e-11; r[LMATO_P_M] = 7.346e22; r[LMATO_P_R0] = 1738100.0; r[LMATO_P_FT] = Ft; r[LMATO_P_M0] = M0;
+  r[LMATO_P_M_DOT] = Mdot; r[LMATO_P_FUEL_MASS] = 2376.0; r[LMATO_P_ANGLE_DOUBLEDOT_MAX] = addm;
+  r[LMATO_P_R_PERIAPSIS] = rp; r[LMATO_P_R_APOAPSIS] = ra; r[LMATO_P_FINAL_TIME] = 470.0;
+  r[LMATO_P_MASS_SCALAR] = 2376.0; r[LMATO_P_ANGLE_UB] = M_PI / 3.0; r[LMATO_P_U_BOUND] = 1.0;
+  return r;
+}
+
+// The options every entry point starts from (those lmato_solve_batch sets, with MAX_ITER 500); each entry point then
+// applies its own environment overrides.
+static Options make_options(double tol, double obj_scale, double mu_min_factor, int n_polish, double w_dcost) {
+  Options O;
+  O.tol = tol; O.mu_init = 0.1; O.obj_scale = obj_scale; O.kappa_eps = 30.0; O.kappa_mu = 0.2; O.theta_mu = 1.5; O.theta_mu_warm = 2.0;
+  O.tau_min = 0.99; O.delta_c = 1e-8; O.tf_guess = 0.9; O.max_iter = 500; O.max_ls = 40; O.mu_min_factor = mu_min_factor;
+  O.n_polish = n_polish; O.w_dcost = w_dcost;
+  return O;
+}
+
+// the model the CIRCULAR environment variable selects
+static int model_from_env() { return getenv("CIRCULAR") ? LMATO_MODEL_CIRCULAR : LMATO_MODEL_ELLIPTICAL; }
+
+// One problem on the sweeps SW from their built-in start point, with the results written as the kernels write them
+// (B = 1, b = 0).
+template <class SW, class WS>
+static void solve_one(const ResultOut& R, const Params& P, const Mesh& M, const Options& O, int model, const WS& W) {
+  IpmState S;
+  ipm_begin(O, S);
+  SW::guess(P, M, O, W, S.cur);
+  while (!ipm_iterate_t<SW>(P, M, O, W, S)) {}
+  write_results<SW, 1>(R, P, M, O.obj_scale, model, W, 0, 1u, S, 0);
 }
 
 int main(int argc, char** argv) {
@@ -40,12 +63,9 @@ int main(int argc, char** argv) {
   std::vector<double> h(N + 1), tau(N + 1);
   for (int k = 0; k <= N; ++k) { tau[k] = (double)k / N; h[k] = k ? tau[k] - tau[k - 1] : 0.0; }
   Mesh M{N, h.data(), tau.data()};
-  Options O;
-  O.tol = 1e-10; O.mu_init = 0.1; O.obj_scale = 10.0; O.kappa_eps = 30.0; O.kappa_mu = 0.2; O.theta_mu = 1.5; O.theta_mu_warm = 2.0;
-  O.tau_min = 0.99; O.delta_c = 1e-8; O.tf_guess = 0.9; O.max_iter = 500; O.max_ls = 40; O.mu_min_factor = 1e-3; O.n_polish = 4;
+  Options O = make_options(1e-10, 10.0, 1e-3, 4, getenv("WDC") ? atof(getenv("WDC")) : 0.0);
   if (getenv("MMF")) O.mu_min_factor = atof(getenv("MMF"));
   if (getenv("NPOL")) O.n_polish = atoi(getenv("NPOL"));
-  O.w_dcost = getenv("WDC") ? atof(getenv("WDC")) : 0.0;
   if (getenv("THMU")) O.theta_mu = atof(getenv("THMU"));
   if (getenv("KMU")) O.kappa_mu = atof(getenv("KMU"));
   if (getenv("KEPS")) O.kappa_eps = atof(getenv("KEPS"));
@@ -72,7 +92,7 @@ int main(int argc, char** argv) {
     const double rp = 17703.0 * (1 + 0.10 * (2 * u[4] - 1));
     const double ra = 88615.0 * (1 + 0.10 * (2 * u[5] - 1));
     if (only >= 0 && p != only) continue;
-    Params P = make_params(Ft, M0, Mdot, addm, rp, ra);
+    Params P = derive_params(make_params(Ft, M0, Mdot, addm, rp, ra).data(), 1, 0, LMATO_MODEL_ELLIPTICAL);
     std::fill(ws.begin(), ws.end(), 0.0);
     SolveOut out;
     if (O.w_dcost > 0) {
@@ -101,6 +121,11 @@ int main(int argc, char** argv) {
   return 0;
 }
 
+// d tf / d parameter (include/lmato_b200.h, lmato_sens_t: 4 values) of the next hostsim_solve / hostsim_solve_coop
+// calls, or NULL: the counterpart of lmato_set_sensitivity_output.
+static double* g_dtf = nullptr;
+extern "C" void hostsim_set_sensitivity_output(double* dtf) { g_dtf = dtf; }
+
 // ctypes entry for developer-side comparisons against tests/golden (NOT the product path).
 extern "C" int hostsim_solve(const double* raw14, int nt, const double* time, double tol, double obj_scale,
                              double mu_min_factor, double* traj /* [10][nt] */, double* tf_out, int* iters, double* kkt) {
@@ -108,58 +133,28 @@ extern "C" int hostsim_solve(const double* raw14, int nt, const double* time, do
   std::vector<double> h(N + 1), tau(N + 1);
   for (int k = 0; k <= N; ++k) { tau[k] = time ? time[k] : (double)k / N; h[k] = k ? tau[k] - tau[k - 1] : 0.0; }
   Mesh M{N, h.data(), tau.data()};
-  Options O;
-  O.tol = tol; O.mu_init = 0.1; O.obj_scale = obj_scale; O.kappa_eps = 30.0; O.kappa_mu = 0.2; O.theta_mu = 1.5; O.theta_mu_warm = 2.0;
-  O.tau_min = 0.99; O.delta_c = 1e-8; O.tf_guess = 0.9; O.max_iter = 500; O.max_ls = 40; O.mu_min_factor = mu_min_factor; O.n_polish = getenv("NPOL") ? atoi(getenv("NPOL")) : 4;
-  O.w_dcost = getenv("WDC") ? atof(getenv("WDC")) : 0.0;
-  Params P;
-  const double* r = raw14;
-  P.GM = r[0] * r[1]; P.R0 = r[2]; P.Ft = r[3]; P.M0 = r[4]; P.S = r[8]; P.ms = r[11]; P.mflow = r[5] / r[6];
-  P.asc = r[7] / 3.0; P.T = r[10]; P.a_ub = r[12]; P.u_ub = r[13];
-  const double vt = std::sqrt(P.GM / (P.R0 + 0.5 * (r[8] + r[9])));
-  P.vt2 = (vt / P.S) * (vt / P.S); P.rt = (P.R0 + P.S) / P.S; P.R0S = P.R0 / P.S;
-  P.tf_ub = std::fmin(1.0, 1.0 / (P.mflow * P.T)); P.fuel = r[6]; P.Sinv = 1.0 / P.S; P.coup5 = 1.0; P.mT = P.mflow * P.T;
-  if (getenv("CIRCULAR")) { P.coup5 = 0.0; P.asc = 1.0; P.u_ub = 1e20; }
+  const Options O = make_options(tol, obj_scale, mu_min_factor, getenv("NPOL") ? atoi(getenv("NPOL")) : 4,
+                                 getenv("WDC") ? atof(getenv("WDC")) : 0.0);
+  const int model = model_from_env();
+  const Params P = derive_params(raw14, 1, 0, model);      // as the thread kernel: no circular move formulation
   const bool DC = O.w_dcost > 0;
   const int nfields = DC ? (int)dc::N_FIELDS : (int)N_FIELDS;
-  const int niter = DC ? (int)dc::N_ITER : (int)N_ITER;
   std::vector<double> ws((size_t)nfields * LANES * (N + 1), 0.0);
   std::vector<double> tile(2 * TILE_ROWS, 0.0);
   Ws W{ws.data(), (long)nfields * LANES, tile.data()};
-  SolveOut out;
-  if (DC) {
-    IpmState S;
-    dc::init_guess(P, M, O, W, S.cur);
-    ipm_begin(O, S);
-    while (!ipm_iterate_t<Sweeps8>(P, M, O, W, S)) {}
-    ipm_result(S, out);
-  } else {
-    ipm_solve(P, M, O, W, false, out);
-  }
-  *tf_out = out.tf; *iters = out.iters; *kkt = out.kkt;
-  for (int v = 0; v < 10; ++v) traj[v * nt] = 0.0;
-  for (int k = 1; k <= N; ++k) {
-    const double* sp = W.stage(k);
-    double z[6];
-    for (int i = 0; i < 6; ++i) z[i] = WS_AT(sp, out.cur * niter + F_Z + i);
-    const double m = P.mflow * P.T * tau[k] * out.tf;
-    double ay, ax;
-    accel_value(P, z[0], z[2], z[4], m, ay, ax);
-    const double vals[10] = {z[0], z[1], ay, z[2], z[3], ax, z[4], z[5], m, WS_AT(sp, out.cur * niter + F_U)};
-    for (int v = 0; v < 10; ++v) traj[v * nt + k] = vals[v];
-  }
-  return out.status;
+  int status;
+  double fmass;
+  const ResultOut R{traj, tf_out, &fmass, &status, iters, kkt, g_dtf, 1};
+  if (DC) solve_one<Sweeps8>(R, P, M, O, model, W);
+  else solve_one<Sweeps7>(R, P, M, O, model, W);
+  return status;
 }
 
 // Finite-difference check of the hand-derived model derivatives (ascent_model.cuh) at one point:
 // returns the largest relative error of accel_first's eight first derivatives and of the
 // second-derivative contraction used by the Hessian (accel_second) against central differences.
 extern "C" double hostsim_check_derivatives(const double* raw14, double y, double x, double a, double m) {
-  Params P;
-  const double* r = raw14;
-  P.GM = r[0] * r[1]; P.R0 = r[2]; P.Ft = r[3]; P.M0 = r[4]; P.S = r[8]; P.ms = r[11]; P.mflow = r[5] / r[6];
-  P.asc = r[7] / 3.0; P.T = r[10]; P.a_ub = r[12]; P.u_ub = r[13];
-  P.fuel = r[6]; P.Sinv = 1.0 / P.S; P.coup5 = 1.0; P.mT = P.mflow * P.T;
+  const Params P = derive_params(raw14, 1, 0, LMATO_MODEL_ELLIPTICAL);
   Accel1 f;
   accel_first(P, y, x, a, m, f);
   const double v[4] = {y, x, a, m};
@@ -199,55 +194,33 @@ extern "C" double hostsim_check_derivatives(const double* raw14, double y, doubl
 }
 
 // The cooperative sweeps (csrc/ascent_coop.cuh) run by one lane (G = 1): same entry as hostsim_solve.
-#include "ascent_coop.cuh"
 extern "C" int hostsim_solve_coop(const double* raw14, int nt, const double* time, double tol, double obj_scale,
                                   double mu_min_factor, double* traj /* [10][nt] */, double* tf_out, int* iters, double* kkt) {
   const int N = nt - 1;
   std::vector<double> h(N + 1), tau(N + 1);
   for (int k = 0; k <= N; ++k) { tau[k] = time ? time[k] : (double)k / N; h[k] = k ? tau[k] - tau[k - 1] : 0.0; }
   Mesh M{N, h.data(), tau.data()};
-  Options O;
-  O.tol = tol; O.mu_init = 0.1; O.obj_scale = obj_scale; O.kappa_eps = 30.0; O.kappa_mu = 0.2; O.theta_mu = 1.5; O.theta_mu_warm = 2.0;
-  O.tau_min = 0.99; O.delta_c = 1e-8; O.tf_guess = 0.9; O.max_iter = 500; O.max_ls = 40; O.mu_min_factor = mu_min_factor; O.n_polish = getenv("NPOL") ? atoi(getenv("NPOL")) : 4;
-  O.w_dcost = getenv("WDC") ? atof(getenv("WDC")) : 0.0;
-  Params P;
-  const double* r = raw14;
-  P.GM = r[0] * r[1]; P.R0 = r[2]; P.Ft = r[3]; P.M0 = r[4]; P.S = r[8]; P.ms = r[11]; P.mflow = r[5] / r[6];
-  P.asc = r[7] / 3.0; P.T = r[10]; P.a_ub = r[12]; P.u_ub = r[13];
-  const double vt = std::sqrt(P.GM / (P.R0 + 0.5 * (r[8] + r[9])));
-  P.vt2 = (vt / P.S) * (vt / P.S); P.rt = (P.R0 + P.S) / P.S; P.R0S = P.R0 / P.S;
-  P.tf_ub = std::fmin(1.0, 1.0 / (P.mflow * P.T)); P.fuel = r[6]; P.Sinv = 1.0 / P.S; P.coup5 = 1.0; P.mT = P.mflow * P.T;
-  if (getenv("CIRCULAR")) { P.coup5 = 0.0; P.asc = 1.0; P.u_ub = 1e20; }
+  const Options O = make_options(tol, obj_scale, mu_min_factor, getenv("NPOL") ? atoi(getenv("NPOL")) : 4,
+                                 getenv("WDC") ? atof(getenv("WDC")) : 0.0);
+  const int model = model_from_env();
   const bool DC = O.w_dcost > 0;
-  if (getenv("CIRCULAR") && DC) P.asc = 0.0;       // the circular model with its move term: the MV slot is the pitch angle
+  const Params P = derive_params(raw14, 1, 0, model, DC);   // the circular model with its move term: MV slot = pitch angle
   std::vector<double> ws((size_t)coop::coop_doubles_per_problem(nt), 0.0);
   std::vector<double> scr(coop::SCR_DOUBLES, 0.0);
   coop::Cws W{ws.data(), nt, scr.data(), 0, 1u, 1u, 0.0, 0.0, 0, 0u};
-  IpmState S;
-  ipm_begin(O, S);
+  int status;
+  double fmass;
+  const ResultOut R{traj, tf_out, &fmass, &status, iters, kkt, g_dtf, 1};
   const bool vrec = getenv("VREC") != nullptr;     // the variant that keeps W_k, g_k instead of running the adjoint recursion
-  if (DC && getenv("CIRCULAR")) { SweepsCoop<1, 1, 2, false>::guess(P, M, O, W, S.cur); while (!ipm_iterate_t<SweepsCoop<1, 1, 2, false>>(P, M, O, W, S)) {} }
-  else if (DC && vrec)  { SweepsCoop<1, 1, true, true>::guess(P, M, O, W, S.cur); while (!ipm_iterate_t<SweepsCoop<1, 1, true, true>>(P, M, O, W, S)) {} }
-  else if (DC)     { SweepsCoop<1, 1, true, false>::guess(P, M, O, W, S.cur); while (!ipm_iterate_t<SweepsCoop<1, 1, true, false>>(P, M, O, W, S)) {} }
-  else if (vrec)   { SweepsCoop<1, 1, false, true>::guess(P, M, O, W, S.cur); while (!ipm_iterate_t<SweepsCoop<1, 1, false, true>>(P, M, O, W, S)) {} }
-  else             { SweepsCoop<1, 1, false, false>::guess(P, M, O, W, S.cur); while (!ipm_iterate_t<SweepsCoop<1, 1, false, false>>(P, M, O, W, S)) {} }
-  SolveOut out;
-  ipm_result(S, out);
-  *tf_out = out.tf; *iters = out.iters; *kkt = out.kkt;
-  for (int v = 0; v < 10; ++v) traj[v * nt] = 0.0;
-  for (int k = 1; k <= N; ++k) {
-    const double* x = W.X(out.cur, k);
-    const double m = P.mflow * P.T * tau[k] * out.tf;
-    double ay, ax;
-    accel_value(P, x[0], x[2], x[4], m, ay, ax);
-    const double vals[10] = {x[0], x[1], ay, x[2], x[3], ax, x[4], x[5], m, x[coop::X_U]};
-    for (int v = 0; v < 10; ++v) traj[v * nt + k] = vals[v];
-  }
-  return out.status;
+  if (DC && model == LMATO_MODEL_CIRCULAR) solve_one<SweepsCoop<1, 1, 2, false>>(R, P, M, O, model, W);
+  else if (DC && vrec) solve_one<SweepsCoop<1, 1, true, true>>(R, P, M, O, model, W);
+  else if (DC)         solve_one<SweepsCoop<1, 1, true, false>>(R, P, M, O, model, W);
+  else if (vrec)       solve_one<SweepsCoop<1, 1, false, true>>(R, P, M, O, model, W);
+  else                 solve_one<SweepsCoop<1, 1, false, false>>(R, P, M, O, model, W);
+  return status;
 }
 
 // Higher-order collocation (csrc/ascent_colloc.cuh), GP = 1.  Ncol: row-major m x m, tauc: m points.
-#include "ascent_colloc.cuh"
 extern "C" int hostsim_solve_colloc(const double* raw14, int nt, const double* time, int nodes, const double* Ncol,
                                     const double* tauc, double tol, double obj_scale, double mu_min_factor,
                                     double* traj /* [10][nt] */, double* tf_out, int* iters, double* kkt) {
@@ -255,17 +228,8 @@ extern "C" int hostsim_solve_colloc(const double* raw14, int nt, const double* t
   std::vector<double> h(N + 1), tau(N + 1);
   for (int k = 0; k <= N; ++k) { tau[k] = time ? time[k] : (double)k / N; h[k] = k ? tau[k] - tau[k - 1] : 0.0; }
   Mesh M{N, h.data(), tau.data()};
-  Options O;
-  O.tol = tol; O.mu_init = 0.1; O.obj_scale = obj_scale; O.kappa_eps = 30.0; O.kappa_mu = 0.2; O.theta_mu = 1.5; O.theta_mu_warm = 2.0;
-  O.tau_min = 0.99; O.delta_c = 1e-8; O.tf_guess = 0.9; O.max_iter = 500; O.max_ls = 40; O.mu_min_factor = mu_min_factor; O.n_polish = getenv("NPOL") ? atoi(getenv("NPOL")) : 4;
-  O.w_dcost = 0.0;
-  Params P;
-  const double* r = raw14;
-  P.GM = r[0] * r[1]; P.R0 = r[2]; P.Ft = r[3]; P.M0 = r[4]; P.S = r[8]; P.ms = r[11]; P.mflow = r[5] / r[6];
-  P.asc = r[7] / 3.0; P.T = r[10]; P.a_ub = r[12]; P.u_ub = r[13];
-  const double vt = std::sqrt(P.GM / (P.R0 + 0.5 * (r[8] + r[9])));
-  P.vt2 = (vt / P.S) * (vt / P.S); P.rt = (P.R0 + P.S) / P.S; P.R0S = P.R0 / P.S;
-  P.tf_ub = std::fmin(1.0, 1.0 / (P.mflow * P.T)); P.fuel = r[6]; P.Sinv = 1.0 / P.S; P.coup5 = 1.0; P.mT = P.mflow * P.T;
+  const Options O = make_options(tol, obj_scale, mu_min_factor, getenv("NPOL") ? atoi(getenv("NPOL")) : 4, 0.0);
+  const Params P = derive_params(raw14, 1, 0, LMATO_MODEL_ELLIPTICAL);   // NODES >= 3: the elliptical model only
   colloc::Coll C;
   C.m = m;
   for (int i = 0; i < m; ++i) { C.tau[i] = tauc[i]; for (int j = 0; j < m; ++j) C.N[i][j] = Ncol[i * m + j]; }
@@ -273,27 +237,19 @@ extern "C" int hostsim_solve_colloc(const double* raw14, int nt, const double* t
   colloc::Nws W;
   W.base = ws.data(); W.N1 = nt; W.L.init(m); W.C = &C; W.g = 0; W.mask = 1u; W.dw = 0.0; W.pimax = 0.0; W.ls_flag = 0;
   IpmState S;
-  SolveOut out;
   const int v0 = getenv("VARIANT") ? atoi(getenv("VARIANT")) : 0;
   const int nv = getenv("VARIANT") ? v0 + 1 : (int)SweepsColloc<1>::N_STARTS;
   for (int variant = v0; variant < nv; ++variant) {        // the kernel's restart ladder
     ipm_begin(O, S);
     SweepsColloc<1>::guess_variant(P, M, O, W, S.cur, variant);
     while (!ipm_iterate_t<SweepsColloc<1>>(P, M, O, W, S)) {}
-    ipm_result(S, out);
-    if (out.status == ST_CONVERGED) break;
+    if (S.ctl.status == ST_CONVERGED) break;
   }
-  *tf_out = out.tf; *iters = out.iters; *kkt = out.kkt;
-  for (int v = 0; v < 10; ++v) traj[v * nt] = 0.0;
-  for (int k = 1; k <= N; ++k) {
-    const double* x = W.X(out.cur, k) + 6 * (m - 1);
-    const double ms = P.mflow * P.T * tau[k] * out.tf;
-    double ay, ax;
-    accel_value(P, x[0], x[2], x[4], ms, ay, ax);
-    const double vals[10] = {x[0], x[1], ay, x[2], x[3], ax, x[4], x[5], ms, W.X(out.cur, k)[W.L.x_u]};
-    for (int v = 0; v < 10; ++v) traj[v * nt + k] = vals[v];
-  }
-  return out.status;
+  int status;
+  double fmass;
+  const ResultOut R{traj, tf_out, &fmass, &status, iters, kkt, nullptr, 1};
+  write_results<SweepsColloc<1>, 1>(R, P, M, O.obj_scale, LMATO_MODEL_ELLIPTICAL, W, 0, 1u, S, 0);
+  return status;
 }
 
 // Batch warm start on the host (what lmato_solve_batch does on the device): the batch-mean problem is solved to
@@ -305,10 +261,7 @@ extern "C" double hostsim_warm_batch(int nprob, int nt, double wdc, double mu_re
   std::vector<double> h(N + 1), tau(N + 1);
   for (int k = 0; k <= N; ++k) { tau[k] = (double)k / N; h[k] = k ? tau[k] - tau[k - 1] : 0.0; }
   Mesh M{N, h.data(), tau.data()};
-  Options O;
-  O.tol = 1e-10; O.mu_init = 0.1; O.obj_scale = 10.0; O.kappa_eps = 30.0; O.kappa_mu = 0.2; O.theta_mu = 1.5; O.theta_mu_warm = 2.0;
-  O.tau_min = 0.99; O.delta_c = 1e-8; O.tf_guess = 0.9; O.max_iter = 500; O.max_ls = 40; O.mu_min_factor = 1e-3; O.n_polish = 2;
-  O.w_dcost = wdc;
+  Options O = make_options(1e-10, 10.0, 1e-3, 2, wdc);
   if (getenv("THMUW")) O.theta_mu_warm = atof(getenv("THMUW"));
   if (getenv("KEPS")) O.kappa_eps = atof(getenv("KEPS"));
   if (getenv("KMU")) O.kappa_mu = atof(getenv("KMU"));
@@ -328,7 +281,7 @@ extern "C" double hostsim_warm_batch(int nprob, int nt, double wdc, double mu_re
     const double addm = 5e-4 * std::pow(2.0, 2 * u[3] - 1);
     const double rp = 17703.0 * (1 + 0.10 * (2 * u[4] - 1));
     const double ra = 88615.0 * (1 + 0.10 * (2 * u[5] - 1));
-    Ps.push_back(make_params(Ft, M0, Mdot, addm, rp, ra));
+    Ps.push_back(derive_params(make_params(Ft, M0, Mdot, addm, rp, ra).data(), 1, 0, LMATO_MODEL_ELLIPTICAL));
     const double v[6] = {Ft, M0, Mdot, addm, rp, ra};
     for (int i = 0; i < 6; ++i) mean[i] += v[i] / nprob;
   }
@@ -336,7 +289,8 @@ extern "C" double hostsim_warm_batch(int nprob, int nt, double wdc, double mu_re
   std::vector<double> ref((size_t)dc::REF_ROWS * nt, 0.0);
   coop::Cws W{ws.data(), nt, scr.data(), 0, 1u, 1u, 0.0, 0.0, 0, 0u};
   {   // reference solve
-    Params Pm = make_params(mean[0], mean[1], mean[2], mean[3], mean[4], mean[5]);
+    const Params Pm = derive_params(make_params(mean[0], mean[1], mean[2], mean[3], mean[4], mean[5]).data(), 1, 0,
+                                    LMATO_MODEL_ELLIPTICAL);
     Options R = O;
     R.tol = 10.0 * mu_ref; R.mu_min_factor = 0.1; R.n_polish = 0; R.w_dcost = 0.0;
     IpmState S;
