@@ -162,21 +162,10 @@ __global__ void __launch_bounds__(kBlock, kBlocksPerSM) ascent_ipm_kernel(KArgs 
         b = (long)chunk * 32 + lane;
         if (b < a.res.B) {
           P = derive_params(a.params, a.res.B, b, a.model);
-          ipm_begin(O, S);
-          double mu0 = 0.0;
           // ref_mode 2: start from the batch reference.  ref_mode 1 (the reference solve itself):
           // start from the previous call's reference if the handle has one (consecutive batches of a
           // campaign have nearly the same mean, so it re-converges in one or two iterations).
-          if (a.guess_traj) {
-            SW::guess_from(P, M, O, W, GuessSrc{a.guess_traj, a.guess_tf, a.res.B, b}, S.cur);
-            S.from_guess = true;
-          } else if (a.ref_mode != 0 && SW::load_ref(P, M, O, W, a.ref, S.cur, &mu0)) {
-            S.warm = true;
-            S.ctl.mu = mu0;
-            S.ctl.tau = dmax(O.tau_min, 1.0 - mu0);
-          } else {
-            SW::guess(P, M, O, W, S.cur);
-          }
+          ipm_start<SW>(P, M, O, W, GuessSrc{a.guess_traj, a.guess_tf, a.res.B, b}, a.ref_mode != 0 ? a.ref : nullptr, S);
           active = true;
         }
       }
@@ -188,15 +177,7 @@ __global__ void __launch_bounds__(kBlock, kBlocksPerSM) ascent_ipm_kernel(KArgs 
     //  a few iterations while the warps stay close enough to share the instruction cache)
     if ((round++ % LMATO_SYNC_PERIOD) == 0 && !__syncthreads_or((active || !exhausted) ? 1 : 0)) break;
     if (active && ipm_iterate_t<SW>(P, M, O, W, S)) {
-      if ((S.warm || S.from_guess) && S.ctl.status != ST_CONVERGED) {
-        // a warm start, or a caller's start point (lmato_set_initial_guess), that did not work out: this lane
-        // restarts the same problem from the built-in roll-out.  (IPOPT would enter its feasibility restoration
-        // phase from such a point, e.g. from the reference's all-zero start values LO:39, 83-96; this solver's
-        // substitute is a start point that is dynamically feasible by construction.)
-        { const int prior = S.iters_prior + S.ctl.iter; ipm_begin(O, S); S.iters_prior = prior; }
-        SW::guess(P, M, O, W, S.cur);
-        continue;
-      }
+      if (ipm_restart<SW>(P, M, O, W, S)) continue;      // this lane restarts the same problem
       active = false;
       pending = true;      // results are written when the whole chunk is done (see above)
       // (the reference solve of the batch warm start, ref_mode 1, runs on the cooperative kernel)
@@ -271,18 +252,7 @@ __global__ void __launch_bounds__(kCoopBlock, BPS) ascent_coop_kernel(KArgs a) {
         if (b < a.res.B) {
           if (W.g == 0) P = derive_params(a.params, a.res.B, b, a.model, MOVE == 2);
           coop::Grp<GP>::sync(gmask);
-          ipm_begin(O, S);
-          double mu0 = 0.0;
-          if (a.guess_traj) {
-            SW::guess_from(P, M, O, W, GuessSrc{a.guess_traj, a.guess_tf, a.res.B, b}, S.cur);
-            S.from_guess = true;
-          } else if (a.ref_mode != 0 && SW::load_ref(P, M, O, W, a.ref, S.cur, &mu0)) {
-            S.warm = true;
-            S.ctl.mu = mu0;
-            S.ctl.tau = dmax(O.tau_min, 1.0 - mu0);
-          } else {
-            SW::guess(P, M, O, W, S.cur);
-          }
+          ipm_start<SW>(P, M, O, W, GuessSrc{a.guess_traj, a.guess_tf, a.res.B, b}, a.ref_mode != 0 ? a.ref : nullptr, S);
           active = true;
         }
       }
@@ -291,12 +261,7 @@ __global__ void __launch_bounds__(kCoopBlock, BPS) ascent_coop_kernel(KArgs a) {
     //  waits for its neighbours' line-search retries loses more than the instruction cache gains)
     if (exhausted && !__any_sync(0xffffffffu, active || pending)) break;
     if (active && ipm_iterate_t<SW>(P, M, O, W, S)) {
-      if ((S.warm || S.from_guess) && S.ctl.status != ST_CONVERGED) {
-        // a warm start or a caller's guess that did not work out: restart from the built-in roll-out
-        { const int prior = S.iters_prior + S.ctl.iter; ipm_begin(O, S); S.iters_prior = prior; }
-        SW::guess(P, M, O, W, S.cur);
-        continue;
-      }
+      if (ipm_restart<SW>(P, M, O, W, S)) continue;
       active = false;
       if (a.ref_mode == 1) {
         SolveOut out;

@@ -619,7 +619,7 @@ LM_SWEEP void colloc_eval(const Params& P, const Mesh& M, const Options& O, cons
 }
 
 // ---------------------------------------------------------------------------------------
-// start point: the bang-bang pitch-acceleration profile of init_guess() (ascent_ipm.cuh) rolled out WITH THE
+// start point: the bang-bang pitch-acceleration profile of start_rollout() (ascent_ipm.cuh) rolled out WITH THE
 // COLLOCATION RULE ITSELF: every step is first predicted by Euler sub-steps from point to point and then
 // corrected by three Newton iterations on its own collocation rows (the condensation's affine column is
 // exactly -E^-1 c), so the start is dynamically feasible and only the terminal rows and the interior push of the
@@ -662,7 +662,7 @@ LM_NOINLINE void colloc_init_guess(const Params& P, const Mesh& M, const Options
         a += dt * w;
         const double ac = dmin(dmax(a, a_lo), a_hi);
         double yn = y + dt * vy, xn = x + dt * vx, vyn = vy, vxn = vx;
-        for (int itr = 0; itr < 3; ++itr) {                     // implicit Euler sub-step, as in init_guess()
+        for (int itr = 0; itr < 3; ++itr) {                     // implicit Euler sub-step, as in start_rollout()
           double ay, ax;
           accel_value(P, yn, xn, ac, P.mflow * t, ay, ax);
           vyn = vy + dt * ay; vxn = vx + dt * ax;
@@ -689,7 +689,7 @@ LM_NOINLINE void colloc_init_guess(const Params& P, const Mesh& M, const Options
       for (int i = 0; i < L.DR; ++i) W.D(k)[i] = 0.0;
     }
   }
-  coop::coop_start_scalars(s, tf0);
+  start_scalars(s, tf0);
   Grp<GP>::sync(W.mask);
 }
 

@@ -62,6 +62,8 @@ enum : int {
   RING_DOUBLES = RING_D * RING_SB,
   SCR_DOUBLES = SCR_TR1 + SCR_TR2 + RING_DOUBLES + RING_D      // ... + one mbarrier (8 bytes) per ring slot
 };
+static_assert((int)X_LAM == NODE_LAM && (int)X_ZLA == NODE_ZLA && (int)X_ZUU == NODE_ZUU && (int)X_PP == NODE_PP &&
+              (int)X_ZPN == NODE_ZPN && NODE_N == 22 && XR == 24, "the X record holds a start node (ascent_ipm.cuh) and two pad doubles");
 
 // 128-bit moves of N (even) doubles
 template <int N>
@@ -191,6 +193,8 @@ struct CwsT {
   }
 };
 using Cws = CwsT<false>;
+template <bool STAGE_MAJOR> LM_HD int grp_lane(const CwsT<STAGE_MAJOR>& W) { return W.g; }
+template <bool STAGE_MAJOR> LM_HD unsigned grp_mask(const CwsT<STAGE_MAJOR>& W) { return W.mask; }
 LM_HD long coop_doubles_per_problem(int nt) { return (long)nt * PER_STAGE; }
 static_assert(RING_SF <= RING_SB && RING_SA <= RING_SB, "ring too small");
 
@@ -1108,121 +1112,8 @@ LM_SWEEP void coop_eval(const Params& P, const Mesh& M, const Options& O, const 
   Grp<GP>::sync(gm);
 }
 
-// ---------------------------------------------------------------------------------------
-// start points
-// ---------------------------------------------------------------------------------------
-template <class CW>
-LM_HD void coop_zero_node0(const CW& W) {
-  double zero[XR];
-#pragma unroll
-  for (int i = 0; i < XR; ++i) zero[i] = 0.0;
-  stv<XR>(W.X(0, 0), zero); stv<XR>(W.X(1, 0), zero); stv<DR>(W.D(0), zero);
-}
-
-// one stage of a start point: primal values given, multipliers and slack pair as in dc::init_guess
-template <class CW>
-LM_HD void coop_store_start(const Params& P, const Options& O, const CW& W, int k, const double* z6, double u,
-                            double uprev, bool move) {
-  double x[XR], zero[DR];
-#pragma unroll
-  for (int i = 0; i < 6; ++i) x[X_Z + i] = z6[i];
-  x[X_U] = u;
-#pragma unroll
-  for (int i = 0; i < 7; ++i) x[X_LAM + i] = 0.0;
-  x[X_ZLA] = 1.0; x[X_ZUA] = 1.0;
-  // an unbounded control (circular model) starts on the central path of its vacuous bounds
-  x[X_ZLU] = P.coup5 != 0.0 ? 1.0 : O.mu_init / (u + P.u_ub);
-  x[X_ZUU] = P.coup5 != 0.0 ? 1.0 : O.mu_init / (P.u_ub - u);
-  if (move) {
-    // slack pair on its central path for mu_init with lam_6 = 0:  z_p = z_n = w, p + n = t(v), p - n = v
-    const double wd = O.w_dcost, v = u - uprev;
-    const double tt = (O.mu_init + sqrt(O.mu_init * O.mu_init + wd * wd * v * v)) / wd;
-    x[X_PP] = 0.5 * (tt + v); x[X_PN] = 0.5 * (tt - v); x[X_ZPP] = wd; x[X_ZPN] = wd;
-  } else {
-    x[X_PP] = 1.0; x[X_PN] = 1.0; x[X_ZPP] = 0.0; x[X_ZPN] = 0.0;
-  }
-  x[22] = 0.0; x[23] = 0.0;
-  stv<XR>(W.X(0, k), x);
-#pragma unroll
-  for (int i = 0; i < DR; ++i) zero[i] = 0.0;
-  stv<DR>(W.D(k), zero);
-}
-
-LM_HD void coop_start_scalars(Scal& s, double tf0) {
-  s.tf = tf0;
-  s.zLt = 1.0; s.zUt = 1.0;
-  s.sg1 = 1e-2; s.sg2 = 1e-2; s.zs1 = 1.0; s.zs2 = 1.0; s.nu3 = 0.0;
-}
-
-// the bang-bang roll-out of init_guess() (ascent_ipm.cuh); a sequential integration, carried by every lane
-template <int G, int MOVE, class CW>
-LM_NOINLINE void coop_init_guess(const Params& P, const Mesh& M, const Options& O, const CW& W, Scal& s) {
-  const int N = M.N;
-  const double tf0 = dmin(dmax(O.tf_guess, 1e-2 * P.tf_ub), 0.99 * P.tf_ub);
-  const GuessProfile gp = guess_profile(P);
-  double y = 0, vy = 0, x = 0, vx = 0, a = 0, w = 0, t_prev = 0, u_prev = 0;
-  const double a_lo = 1e-2 * P.a_ub, a_hi = 0.99 * P.a_ub;
-  if (W.g == 0) coop_zero_node0(W);
-  for (int k = 1; k <= N; ++k) {
-    const double t = M.tau[k] * tf0 * P.T;
-    const double dt = t - t_prev;
-    const double tm = 0.5 * (t + t_prev);
-    double u = tm < gp.t1 ? gp.ulev : (tm < gp.t1 + gp.t2 ? -gp.ulev : 0.0);
-    if (P.coup5 != 0.0) {
-      w += dt * P.asc * u;
-      a += dt * w;
-    } else {
-      // circular model: pitch ramps linearly from ~34 deg (PDF p.21 Fig 9); angledot and u follow
-      const double a_new = 0.2 + 0.45 * M.tau[k];
-      if (mv_is_angle(P) != 0.0) { w = 0.0; u = dmin(dmax(a_new, a_lo), a_hi); }    // the MV is the pitch angle
-      else { w = (a_new - a) / dt; u = w / (dt * P.asc); }
-      a = a_new;
-    }
-    const double ac = dmin(dmax(a, a_lo), a_hi);
-    const double m = P.mflow * P.T * M.tau[k] * tf0;
-    double yn = y + dt * vy, xn = x + dt * vx, vyn = vy, vxn = vx;
-    for (int itr = 0; itr < 3; ++itr) {
-      double ay, ax;
-      accel_value(P, yn, xn, ac, m, ay, ax);
-      vyn = vy + dt * ay; vxn = vx + dt * ax;
-      yn = y + dt * vyn;  xn = x + dt * vxn;
-    }
-    y = yn; vy = vyn; x = xn; vx = vxn;
-    if (((k - 1) % G) == W.g) {
-      const double z6[6] = {y, vy, x, vx, ac, w};
-      coop_store_start(P, O, W, k, z6, u, u_prev, MOVE);
-    }
-    u_prev = u;
-    t_prev = t;
-  }
-  coop_start_scalars(s, tf0);
-  Grp<G>::sync(W.mask);
-}
-
-// caller-supplied start point (init_from_guess(), ascent_ipm.cuh), stage-parallel
-template <int G, int MOVE, class CW>
-LM_NOINLINE void coop_init_from_guess(const Params& P, const Mesh& M, const Options& O, const CW& W, const GuessSrc& Gs,
-                                      Scal& s) {
-  const int N = M.N, nt = N + 1;
-  const double tf0 = dmin(dmax(Gs.tf[Gs.b], 1e-2 * P.tf_ub), 0.99 * P.tf_ub);
-  const double a_lo = 1e-2 * P.a_ub, a_hi = 0.99 * P.a_ub, u_hi = 0.99 * P.u_ub;
-  if (W.g == 0) coop_zero_node0(W);
-  const bool mva = mv_is_angle(P) != 0.0;       // the MV is the pitch angle: its slot follows the angle row
-  for (int k = 1 + W.g; k <= N; k += G) {
-    const double ak = dmin(dmax(Gs.at(GuessSrc::V_ANGLE, k, nt), a_lo), a_hi);
-    const double u = mva ? ak : dmin(dmax(Gs.at(GuessSrc::V_U, k, nt), -u_hi), u_hi);
-    const double up = k > 1 ? (mva ? dmin(dmax(Gs.at(GuessSrc::V_ANGLE, k - 1, nt), a_lo), a_hi)
-                                   : dmin(dmax(Gs.at(GuessSrc::V_U, k - 1, nt), -u_hi), u_hi)) : 0.0;
-    const double z6[6] = {Gs.at(GuessSrc::V_Y, k, nt), Gs.at(GuessSrc::V_YDOT, k, nt), Gs.at(GuessSrc::V_X, k, nt),
-                          Gs.at(GuessSrc::V_XDOT, k, nt), ak, mva ? 0.0 : Gs.at(GuessSrc::V_ANGLEDOT, k, nt)};
-    coop_store_start(P, O, W, k, z6, u, up, MOVE);
-  }
-  coop_start_scalars(s, tf0);
-  Grp<G>::sync(W.mask);
-}
-
-// Reference column of the batch warm start, in the layout init_from_ref() reads (ascent_ipm.cuh: the 17 rows of the
-// 7-state iterate, then one row of scalars), so that both kernels can start from a reference produced here.
+// Reference column of the batch warm start (ascent_ipm.cuh: REF_*), so that every kernel can start from a reference
+// produced here.
 template <int G, class CW>
 LM_NOINLINE void coop_store_ref(const Params& P, const Mesh& M, const CW& W, int src, const Scal& c, double mu, bool ok,
                                 double* ref) {
@@ -1230,63 +1121,9 @@ LM_NOINLINE void coop_store_ref(const Params& P, const Mesh& M, const CW& W, int
   for (int k = 1 + W.g; k <= M.N; k += G) {
     double x[XR];
     ldv<XR>(W.X(src, k), x);
-#pragma unroll
-    for (int i = 0; i < 7; ++i) ref[(lmato::F_Z + i) * N1 + k] = x[X_Z + i];        // states, u
-#pragma unroll
-    for (int i = 0; i < 6; ++i) ref[(lmato::F_LAM + i) * N1 + k] = x[X_LAM + i];
-    ref[lmato::F_ZLA * N1 + k] = x[X_ZLA]; ref[lmato::F_ZUA * N1 + k] = x[X_ZUA];
-    ref[lmato::F_ZLU * N1 + k] = x[X_ZLU]; ref[lmato::F_ZUU * N1 + k] = x[X_ZUU];
+    ref_put_node(ref, N1, k, x);
   }
-  if (W.g == 0) {
-    double* sc = ref + lmato::N_ITER * N1;
-    sc[REF_OK] = ok ? 1.0 : 0.0; sc[REF_MU] = mu; sc[REF_S] = P.S; sc[REF_TF] = c.tf;
-    sc[REF_ZLT] = c.zLt; sc[REF_ZUT] = c.zUt; sc[REF_SG1] = c.sg1; sc[REF_SG2] = c.sg2;
-    sc[REF_ZS1] = c.zs1; sc[REF_ZS2] = c.zs2; sc[REF_NU3] = c.nu3;
-  }
-}
-
-// start from the reference column (dc::init_from_ref7): the slack pair is put on its central path for the
-// reference's moves and the multiplier of the u row follows from dual feasibility
-template <int G, int MOVE, class CW>
-LM_NOINLINE bool coop_load_ref(const Params& P, const Mesh& M, const Options& O, const CW& W, const double* ref,
-                               Scal& s, double* mu_out) {
-  const int N1 = M.N + 1;
-  const double* sc = ref + lmato::N_ITER * N1;
-  if (!(sc[REF_OK] > 0.5)) return false;
-  const double r = sc[REF_S] * P.Sinv, ri = P.S / sc[REF_S];
-  const double mu = sc[REF_MU], w = O.w_dcost;
-  if (W.g == 0) coop_zero_node0(W);
-  for (int k = 1 + W.g; k <= M.N; k += G) {
-    double x[XR], zero[DR];
-#pragma unroll
-    for (int i = 0; i < 7; ++i) x[X_Z + i] = ref[(lmato::F_Z + i) * N1 + k] * (i < 4 ? r : 1.0);
-#pragma unroll
-    for (int i = 0; i < 6; ++i) x[X_LAM + i] = ref[(lmato::F_LAM + i) * N1 + k] * (i < 4 ? ri : 1.0);
-    x[X_ZLA] = ref[lmato::F_ZLA * N1 + k]; x[X_ZUA] = ref[lmato::F_ZUA * N1 + k];
-    x[X_ZLU] = ref[lmato::F_ZLU * N1 + k]; x[X_ZUU] = ref[lmato::F_ZUU * N1 + k];
-    if (MOVE) {
-      const double u = x[X_U], up = k > 1 ? ref[lmato::F_U * N1 + k - 1] : 0.0;
-      const double v = u - up;
-      const double tt = (mu + sqrt(mu * mu + w * w * v * v)) / w;
-      const double pp = 0.5 * (tt + v), pn = 0.5 * (tt - v);
-      x[X_PP] = pp; x[X_PN] = pn; x[X_ZPP] = mu / pp; x[X_ZPN] = mu / pn;
-      x[X_LAM + 6] = w - mu / pp;
-    } else {
-      x[X_PP] = 1.0; x[X_PN] = 1.0; x[X_ZPP] = 0.0; x[X_ZPN] = 0.0;
-      x[X_LAM + 6] = 0.0;
-    }
-    x[22] = 0.0; x[23] = 0.0;
-    stv<XR>(W.X(0, k), x);
-#pragma unroll
-    for (int i = 0; i < DR; ++i) zero[i] = 0.0;
-    stv<DR>(W.D(k), zero);
-  }
-  s.tf = dmin(sc[REF_TF], 0.99 * P.tf_ub);
-  s.zLt = sc[REF_ZLT]; s.zUt = sc[REF_ZUT];
-  s.sg1 = sc[REF_SG1]; s.sg2 = sc[REF_SG2]; s.zs1 = sc[REF_ZS1]; s.zs2 = sc[REF_ZS2]; s.nu3 = sc[REF_NU3];
-  *mu_out = mu;
-  Grp<G>::sync(W.mask);
-  return true;
+  if (W.g == 0) ref_put_scalars(ref, N1, P, c, mu, ok);
 }
 
 }  // namespace coop
@@ -1296,7 +1133,7 @@ LM_NOINLINE bool coop_load_ref(const Params& P, const Mesh& M, const Options& O,
 //   GP lanes (a multiple of G, at most a warp) carry the stage-parallel phases of the same problem.
 template <int G, int GP, int MOVE, bool VREC = (GP > G)>
 struct SweepsCoop {
-  enum : int { LANES_PER_PROBLEM = GP };
+  enum : int { LANES_PER_PROBLEM = GP, MOVE_TERM = MOVE };
   template <class CW>
   LM_HD static int n_eq(const CW&, int N) { return (MOVE ? 7 : 6) * N + 3; }
   template <class CW>
@@ -1321,22 +1158,29 @@ struct SweepsCoop {
     coop::coop_eval<GP, MOVE>(P, M, O, W, src, dst, c0, ts, mu, alpha, alpha_z, alpha_lam, t);
     if (pimax) *pimax = W.pimax;
   }
+  // start points (ascent_ipm.cuh: start_rollout, ...): node k into the X record of buffer 0 with its step record
+  // zeroed; node 0 pinned at zero
   template <class CW>
-  LM_HD static void guess(const Params& P, const Mesh& M, const Options& O, const CW& W, Scal& s) {
-    coop::coop_init_guess<GP, MOVE>(P, M, O, W, s);
+  LM_HD static void store_node(const CW& W, int k, const double* x) {
+    double r[coop::XR], zero[coop::DR];
+#pragma unroll
+    for (int i = 0; i < NODE_N; ++i) r[i] = x[i];
+    r[22] = 0.0; r[23] = 0.0;
+    coop::stv<coop::XR>(W.X(0, k), r);
+#pragma unroll
+    for (int i = 0; i < coop::DR; ++i) zero[i] = 0.0;
+    coop::stv<coop::DR>(W.D(k), zero);
   }
   template <class CW>
-  LM_HD static void guess_from(const Params& P, const Mesh& M, const Options& O, const CW& W, const GuessSrc& Gs, Scal& s) {
-    coop::coop_init_from_guess<GP, MOVE>(P, M, O, W, Gs, s);
+  LM_HD static void zero_node0(const CW& W) {
+    double zero[coop::XR];
+#pragma unroll
+    for (int i = 0; i < coop::XR; ++i) zero[i] = 0.0;
+    coop::stv<coop::XR>(W.X(0, 0), zero); coop::stv<coop::XR>(W.X(1, 0), zero); coop::stv<coop::DR>(W.D(0), zero);
   }
   template <class CW>
   LM_HD static void store_ref(const Params& P, const Mesh& M, const CW& W, int src, const Scal& c, double mu, bool ok,
                               double* ref) { coop::coop_store_ref<GP>(P, M, W, src, c, mu, ok, ref); }
-  template <class CW>
-  LM_HD static bool load_ref(const Params& P, const Mesh& M, const Options& O, const CW& W, const double* ref,
-                             Scal& s, double* mu) {
-    return coop::coop_load_ref<GP, MOVE>(P, M, O, W, ref, s, mu);
-  }
   // node k of iterate `cur`: x = the six states and the control, lam = the multipliers of the ydot, xdot and angledot
   // rows; either may be null
   template <class CW>

@@ -348,46 +348,117 @@ LM_HD GuessProfile guess_profile(const Params& P) {
   return g;
 }
 
-// Row layout of an iterate in the workspace, for the start-point code shared by the 7-state sweeps (below) and
-// the 8-state sweeps with the move term (ascent_ipm_dc.cuh: Layout8).
-struct Layout7 {
-  enum : int { FZ = F_Z, FU = F_U, FLAM = F_LAM, NLAM = 6, FZLA = F_ZLA, FZUA = F_ZUA, FZLU = F_ZLU, FZUU = F_ZUU,
-               NITER = N_ITER, FDS = F_DS, FDU = F_DU, RSTEP = R_STEP, NSTEP = N_STEP,
-               MOVE = 0, FPP = 0, FPN = 0, FZPP = 0, FZPN = 0 };
+// Caller-supplied start point (SURVEY 8f.4): trajectories in the OUTPUT layout of the solver,
+// [variable][node][problem] with the ten variables in the reference's order (LO:83-100), and tf.
+struct GuessSrc {
+  const double* traj;    // [10][nt][B]
+  const double* tf;      // [B]
+  long B, b;
+  enum : int { V_Y = 0, V_YDOT = 1, V_X = 3, V_XDOT = 4, V_ANGLE = 6, V_ANGLEDOT = 7, V_U = 9 };
+  LM_HD double at(int v, int k, int nt) const { return traj[((long)v * nt + k) * B + b]; }
 };
 
-// node 0 is pinned at zero (LO:145-151): its state / step rows are literal zeros so that the sweeps can read
-// "node k-1" without a special case at k = 1 (with the move term also MV(0) = 0)
-template <class L>
-LM_HD void start_zero_node0(const Ws& W) {
-  double* s0 = W.stage(0);
-#pragma unroll
-  for (int i = 0; i < 6; ++i) { WS_AT(s0, L::FZ + i) = 0.0; WS_AT(s0, L::NITER + L::FZ + i) = 0.0; WS_AT(s0, L::FDS + i) = 0.0; }
-  if (L::MOVE) { WS_AT(s0, L::FU) = 0.0; WS_AT(s0, L::NITER + L::FU) = 0.0; WS_AT(s0, L::FDU) = 0.0; }
-}
+// ---------------------------------------------------------------------------------------
+// Warm start: every problem of a batch may start from one reference central-path point (the
+// batch-mean problem solved down to mu_ref ~ 1e-3) instead of the generic roll-out.  That skips
+// the globalisation phase (about 7 of 27 iterations); at smaller mu_ref the iterate sits too close
+// to the reference's active bounds and the method jams, so 1e-3 it is.  The reference column is
+// REF_ROWS x (N+1) doubles, ref[row * (N+1) + k]: the 17 rows of the 7-state iterate (row7() below) followed by one
+// row of scalars (node 0..).  Lengths are stored divided by the reference's distance scale S_ref = r_periapsis
+// (LO:107), so a problem rescales them to its own.
+// ---------------------------------------------------------------------------------------
+enum : int { REF_ROWS = N_ITER + 1, REF_OK = 0, REF_MU = 1, REF_S = 2, REF_TF = 3, REF_ZLT = 4, REF_ZUT = 5,
+             REF_SG1 = 6, REF_SG2 = 7, REF_ZS1 = 8, REF_ZS2 = 9, REF_NU3 = 10, REF_NSCAL = 11 };
 
-// start values of one stage: primal values as given, multipliers zero, bound multipliers 1 (an unbounded control
-// -- circular model -- starts exactly on the central path of its vacuous bounds), the move slack pair on its
-// central path for mu_init with lam_6 = 0 (z_p = z_n = w, p + n = t(v), p - n = v), step rows zero
-template <class L>
-LM_HD void start_store_stage(const Params& P, const Options& O, double* sp, const double* z6, double u, double u_prev) {
+// ---------------------------------------------------------------------------------------
+// Start points of every NODES = 2 workspace layout.  The values of a node come from start_node() (roll-out, caller's
+// start point) or ref_node() (batch reference); a layout -- the Sweeps policies Sweeps7, Sweeps8 and SweepsCoop --
+// only says where they go (SW::store_node), how node 0 is zeroed (SW::zero_node0), whether it carries the move slack
+// pair (SW::MOVE_TERM) and how many lanes share a problem (SW::LANES_PER_PROBLEM = G; the thread layouts: G = 1).
+// ---------------------------------------------------------------------------------------
+namespace coop { template <int G> struct Grp; }     // the lanes of one problem (ascent_coop.cuh)
+// this lane's index among them and their mask (the cooperative workspace: ascent_coop.cuh)
+LM_HD int grp_lane(const Ws&) { return 0; }
+LM_HD unsigned grp_mask(const Ws&) { return 1u; }
+
+// One node of a start point in the row order of the 8-state iterate (ascent_ipm_dc.cuh: dc::F_*; the cooperative X
+// record).  The 7-state iterate and the reference column hold the first NODE_N7 fields without lam_6.
+enum : int { NODE_Z = 0, NODE_U = 6, NODE_LAM = 7 /* 7 */, NODE_ZLA = 14, NODE_ZUA = 15, NODE_ZLU = 16, NODE_ZUU = 17,
+             NODE_PP = 18, NODE_PN = 19, NODE_ZPP = 20, NODE_ZPN = 21, NODE_N = 22, NODE_N7 = NODE_PP };
+// row of the 7-state iterate (and of the reference column) that holds node field f < NODE_N7, f != NODE_LAM + 6
+LM_HD constexpr int row7(int f) { return f < NODE_LAM + 6 ? f : f - 1; }
+static_assert(row7(NODE_U) == F_U && row7(NODE_LAM) == F_LAM && row7(NODE_ZLA) == F_ZLA && row7(NODE_ZUU) == F_ZUU &&
+              row7(NODE_ZUU) + 1 == N_ITER, "7-state rows");
+
+// Node k >= 1 of a cold or caller start: primal values as given, defect multipliers 0, bound multipliers 1 (an
+// unbounded control -- circular model, coup5 = 0 -- starts exactly on the central path of its vacuous bounds), and
+// with the move term the slack pair on its central path for mu_init with lam_6 = 0 (z_p = z_n = w, p + n = t(v),
+// p - n = v, v = u - u_prev).
+LM_HD void start_node(const Params& P, const Options& O, const double* z6, double u, double u_prev, bool move, double* x) {
 #pragma unroll
-  for (int i = 0; i < 6; ++i) WS_AT(sp, L::FZ + i) = z6[i];
-  WS_AT(sp, L::FU) = u;
+  for (int i = 0; i < 6; ++i) x[NODE_Z + i] = z6[i];
+  x[NODE_U] = u;
 #pragma unroll
-  for (int i = 0; i < L::NLAM; ++i) WS_AT(sp, L::FLAM + i) = 0.0;
-  WS_AT(sp, L::FZLA) = 1.0; WS_AT(sp, L::FZUA) = 1.0;
-  const bool bounded = L::MOVE || P.coup5 != 0.0;
-  WS_AT(sp, L::FZLU) = bounded ? 1.0 : O.mu_init / (u + P.u_ub);
-  WS_AT(sp, L::FZUU) = bounded ? 1.0 : O.mu_init / (P.u_ub - u);
-  if (L::MOVE) {
+  for (int i = 0; i < 7; ++i) x[NODE_LAM + i] = 0.0;
+  x[NODE_ZLA] = 1.0; x[NODE_ZUA] = 1.0;
+  x[NODE_ZLU] = P.coup5 != 0.0 ? 1.0 : O.mu_init / (u + P.u_ub);
+  x[NODE_ZUU] = P.coup5 != 0.0 ? 1.0 : O.mu_init / (P.u_ub - u);
+  if (move) {
     const double wd = O.w_dcost, v = u - u_prev;
     const double tt = (O.mu_init + sqrt(O.mu_init * O.mu_init + wd * wd * v * v)) / wd;
-    WS_AT(sp, L::FPP) = 0.5 * (tt + v); WS_AT(sp, L::FPN) = 0.5 * (tt - v);
-    WS_AT(sp, L::FZPP) = wd; WS_AT(sp, L::FZPN) = wd;
+    x[NODE_PP] = 0.5 * (tt + v); x[NODE_PN] = 0.5 * (tt - v); x[NODE_ZPP] = wd; x[NODE_ZPN] = wd;
+  } else {
+    x[NODE_PP] = 1.0; x[NODE_PN] = 1.0; x[NODE_ZPP] = 0.0; x[NODE_ZPN] = 0.0;
   }
+}
+
+// Node k >= 1 from the reference column: lengths rescaled by r = S_ref / S and the multipliers of their rows by
+// ri = S / S_ref.  The reference is a solve without the move term (at mu_ref ~ 1e-3 >> w the two central paths
+// practically coincide): with the move term the slack pair is put exactly on its own central path for mu_ref and the
+// reference's moves (z_p + z_n = 2w, p z_p = n z_n = mu) and lam_6 = w - z_p follows from dual feasibility.
+LM_HD void ref_node(const double* ref, int N1, int k, double r, double ri, double mu, double w, bool move, double* x) {
 #pragma unroll
-  for (int i = 0; i < L::NSTEP; ++i) WS_AT(sp, L::RSTEP + i) = 0.0;
+  for (int f = 0; f < NODE_N7; ++f)
+    if (f != NODE_LAM + 6) x[f] = ref[row7(f) * N1 + k];
+#pragma unroll
+  for (int i = 0; i < 4; ++i) { x[NODE_Z + i] *= r; x[NODE_LAM + i] *= ri; }    // y, vy, x, vx and their rows
+  if (move) {
+    const double v = x[NODE_U] - (k > 1 ? ref[row7(NODE_U) * N1 + k - 1] : 0.0);
+    const double tt = (mu + sqrt(mu * mu + w * w * v * v)) / w;
+    const double pp = 0.5 * (tt + v), pn = 0.5 * (tt - v);
+    x[NODE_PP] = pp; x[NODE_PN] = pn; x[NODE_ZPP] = mu / pp; x[NODE_ZPN] = mu / pn;
+    x[NODE_LAM + 6] = w - mu / pp;
+  } else {
+    x[NODE_PP] = 1.0; x[NODE_PN] = 1.0; x[NODE_ZPP] = 0.0; x[NODE_ZPN] = 0.0;
+    x[NODE_LAM + 6] = 0.0;
+  }
+}
+
+// node k of a converged reference solve into the reference column
+LM_HD void ref_put_node(double* ref, int N1, int k, const double* x) {
+#pragma unroll
+  for (int f = 0; f < NODE_N7; ++f)
+    if (f != NODE_LAM + 6) ref[row7(f) * N1 + k] = x[f];
+}
+
+LM_HD void ref_put_scalars(double* ref, int N1, const Params& P, const Scal& c, double mu, bool ok) {
+  double* sc = ref + N_ITER * N1;
+  sc[REF_OK] = ok ? 1.0 : 0.0; sc[REF_MU] = mu; sc[REF_S] = P.S; sc[REF_TF] = c.tf;
+  sc[REF_ZLT] = c.zLt; sc[REF_ZUT] = c.zUt; sc[REF_SG1] = c.sg1; sc[REF_SG2] = c.sg2;
+  sc[REF_ZS1] = c.zs1; sc[REF_ZS2] = c.zs2; sc[REF_NU3] = c.nu3;
+}
+
+// The start scalars, the barrier parameter mu and the length ratios r, ri of a start from the reference column, or
+// false if the column holds no reference.
+LM_HD bool ref_scalars(const Params& P, const double* ref, int N1, Scal& s, double& mu, double& r, double& ri) {
+  const double* sc = ref + N_ITER * N1;
+  if (!(sc[REF_OK] > 0.5)) return false;
+  r = sc[REF_S] * P.Sinv; ri = P.S / sc[REF_S];
+  mu = sc[REF_MU];
+  s.tf = dmin(sc[REF_TF], 0.99 * P.tf_ub);
+  s.zLt = sc[REF_ZLT]; s.zUt = sc[REF_ZUT];
+  s.sg1 = sc[REF_SG1]; s.sg2 = sc[REF_SG2]; s.zs1 = sc[REF_ZS1]; s.zs2 = sc[REF_ZS2]; s.nu3 = sc[REF_NU3];
+  return true;
 }
 
 LM_HD void start_scalars(Scal& s, double tf0) {
@@ -396,27 +467,30 @@ LM_HD void start_scalars(Scal& s, double tf0) {
   s.sg1 = 1e-2; s.sg2 = 1e-2; s.zs1 = 1.0; s.zs2 = 1.0; s.nu3 = 0.0;
 }
 
-template <class L>
-LM_HD void init_guess_t(const Params& P, const Mesh& M, const Options& O, const Ws& W, Scal& s) {
-  const int N = M.N;
+// The built-in start point: the roll-out of guess_profile(), a sequential integration carried by each of the G lanes
+// of the problem (lane g stores the nodes k with (k - 1) % G == g).
+template <class SW, class WS>
+LM_NOINLINE void start_rollout(const Params& P, const Mesh& M, const Options& O, const WS& W, Scal& s) {
+  constexpr int G = SW::LANES_PER_PROBLEM;
+  const int N = M.N, g = grp_lane(W);
   const double tf0 = dmin(dmax(O.tf_guess, 1e-2 * P.tf_ub), 0.99 * P.tf_ub);
-  const GuessProfile g = guess_profile(P);
+  const GuessProfile gp = guess_profile(P);
   double y = 0, vy = 0, x = 0, vx = 0, a = 0, w = 0, t_prev = 0, u_prev = 0;
   const double a_lo = 1e-2 * P.a_ub, a_hi = 0.99 * P.a_ub;
-  start_zero_node0<L>(W);
+  if (g == 0) SW::zero_node0(W);
   for (int k = 1; k <= N; ++k) {
     const double t = M.tau[k] * tf0 * P.T;
     const double dt = t - t_prev;
     const double tm = 0.5 * (t + t_prev);
-    double u = tm < g.t1 ? g.ulev : (tm < g.t1 + g.t2 ? -g.ulev : 0.0);
+    double u = tm < gp.t1 ? gp.ulev : (tm < gp.t1 + gp.t2 ? -gp.ulev : 0.0);
     if (P.coup5 != 0.0) {
       w += dt * P.asc * u;
       a += dt * w;
     } else {
       // circular model: pitch ramps linearly from ~34 deg (PDF p.21 Fig 9); angledot and u follow
       const double a_new = 0.2 + 0.45 * M.tau[k];
-      w = (a_new - a) / dt;
-      u = w / (dt * P.asc);
+      if (mv_is_angle(P) != 0.0) { w = 0.0; u = dmin(dmax(a_new, a_lo), a_hi); }    // the MV is the pitch angle
+      else { w = (a_new - a) / dt; u = w / (dt * P.asc); }
       a = a_new;
     }
     const double ac = dmin(dmax(a, a_lo), a_hi);
@@ -430,52 +504,63 @@ LM_HD void init_guess_t(const Params& P, const Mesh& M, const Options& O, const 
       yn = y + dt * vyn;  xn = x + dt * vxn;
     }
     y = yn; vy = vyn; x = xn; vx = vxn;
-    const double z6[6] = {y, vy, x, vx, ac, w};
-    start_store_stage<L>(P, O, W.stage(k), z6, u, u_prev);
+    if (((k - 1) % G) == g) {
+      const double z6[6] = {y, vy, x, vx, ac, w};
+      double xk[NODE_N];
+      start_node(P, O, z6, u, u_prev, SW::MOVE_TERM != 0, xk);
+      SW::store_node(W, k, xk);
+    }
     u_prev = u;
     t_prev = t;
   }
   start_scalars(s, tf0);
+  coop::Grp<G>::sync(grp_mask(W));
 }
 
-LM_NOINLINE void init_guess(const Params& P, const Mesh& M, const Options& O, const Ws& W, Scal& s) {
-  init_guess_t<Layout7>(P, M, O, W, s);
-}
-
-// Caller-supplied start point (SURVEY 8f.4): trajectories in the OUTPUT layout of the solver,
-// [variable][node][problem] with the ten variables in the reference's order (LO:83-100), and tf.
-struct GuessSrc {
-  const double* traj;    // [10][nt][B]
-  const double* tf;      // [B]
-  long B, b;
-  enum : int { V_Y = 0, V_YDOT = 1, V_X = 3, V_XDOT = 4, V_ANGLE = 6, V_ANGLEDOT = 7, V_U = 9 };
-  LM_HD double at(int v, int k, int nt) const { return traj[((long)v * nt + k) * B + b]; }
-};
-
-// The primal values are taken as given and only pushed into the interior of their bounds (IPOPT's
-// bound_push); multipliers and slacks start as in the cold start, so iteration 0 is again the
-// least-squares multiplier estimate.  Node 0 is pinned whatever the guess says (LO:145-151).
-template <class L>
-LM_HD void init_from_guess_t(const Params& P, const Mesh& M, const Options& O, const Ws& W, const GuessSrc& G, Scal& s) {
-  const int N = M.N, nt = N + 1;
-  const double tf0 = dmin(dmax(G.tf[G.b], 1e-2 * P.tf_ub), 0.99 * P.tf_ub);
+// Caller-supplied start point, stage-parallel over the G lanes.  The primal values are taken as given and only pushed
+// into the interior of their bounds (IPOPT's bound_push); multipliers and slacks start as in the roll-out, so
+// iteration 0 is again the least-squares multiplier estimate.  Node 0 is pinned whatever the guess says (LO:145-151).
+template <class SW, class WS>
+LM_NOINLINE void start_from_guess(const Params& P, const Mesh& M, const Options& O, const WS& W, const GuessSrc& Gs,
+                                  Scal& s) {
+  constexpr int G = SW::LANES_PER_PROBLEM;
+  const int N = M.N, nt = N + 1, g = grp_lane(W);
+  const double tf0 = dmin(dmax(Gs.tf[Gs.b], 1e-2 * P.tf_ub), 0.99 * P.tf_ub);
   const double a_lo = 1e-2 * P.a_ub, a_hi = 0.99 * P.a_ub, u_hi = 0.99 * P.u_ub;
-  start_zero_node0<L>(W);
-  double u_prev = 0.0;
-  for (int k = 1; k <= N; ++k) {
-    const double u = dmin(dmax(G.at(GuessSrc::V_U, k, nt), -u_hi), u_hi);
-    const double z6[6] = {G.at(GuessSrc::V_Y, k, nt), G.at(GuessSrc::V_YDOT, k, nt), G.at(GuessSrc::V_X, k, nt),
-                          G.at(GuessSrc::V_XDOT, k, nt), dmin(dmax(G.at(GuessSrc::V_ANGLE, k, nt), a_lo), a_hi),
-                          G.at(GuessSrc::V_ANGLEDOT, k, nt)};
-    start_store_stage<L>(P, O, W.stage(k), z6, u, u_prev);
-    u_prev = u;
+  if (g == 0) SW::zero_node0(W);
+  const bool mva = mv_is_angle(P) != 0.0;       // the MV is the pitch angle: its slot follows the angle row
+  for (int k = 1 + g; k <= N; k += G) {
+    const double ak = dmin(dmax(Gs.at(GuessSrc::V_ANGLE, k, nt), a_lo), a_hi);
+    const double u = mva ? ak : dmin(dmax(Gs.at(GuessSrc::V_U, k, nt), -u_hi), u_hi);
+    const double up = k > 1 ? (mva ? dmin(dmax(Gs.at(GuessSrc::V_ANGLE, k - 1, nt), a_lo), a_hi)
+                                   : dmin(dmax(Gs.at(GuessSrc::V_U, k - 1, nt), -u_hi), u_hi)) : 0.0;
+    const double z6[6] = {Gs.at(GuessSrc::V_Y, k, nt), Gs.at(GuessSrc::V_YDOT, k, nt), Gs.at(GuessSrc::V_X, k, nt),
+                          Gs.at(GuessSrc::V_XDOT, k, nt), ak, mva ? 0.0 : Gs.at(GuessSrc::V_ANGLEDOT, k, nt)};
+    double xk[NODE_N];
+    start_node(P, O, z6, u, up, SW::MOVE_TERM != 0, xk);
+    SW::store_node(W, k, xk);
   }
   start_scalars(s, tf0);
+  coop::Grp<G>::sync(grp_mask(W));
 }
 
-LM_NOINLINE void init_from_guess(const Params& P, const Mesh& M, const Options& O, const Ws& W, const GuessSrc& G,
-                                 Scal& s) {
-  init_from_guess_t<Layout7>(P, M, O, W, G, s);
+// Start from the reference column, stage-parallel over the G lanes; false (nothing written) if it holds none.
+template <class SW, class WS>
+LM_NOINLINE bool start_from_ref(const Params& P, const Mesh& M, const Options& O, const WS& W, const double* ref,
+                                Scal& s, double* mu_out) {
+  constexpr int G = SW::LANES_PER_PROBLEM;
+  const int N1 = M.N + 1, g = grp_lane(W);
+  double mu, r, ri;
+  if (!ref_scalars(P, ref, N1, s, mu, r, ri)) return false;
+  if (g == 0) SW::zero_node0(W);
+  for (int k = 1 + g; k <= M.N; k += G) {
+    double xk[NODE_N];
+    ref_node(ref, N1, k, r, ri, mu, O.w_dcost, SW::MOVE_TERM != 0, xk);
+    SW::store_node(W, k, xk);
+  }
+  *mu_out = mu;
+  coop::Grp<G>::sync(grp_mask(W));
+  return true;
 }
 
 // ---------------------------------------------------------------------------------------
@@ -575,49 +660,6 @@ LM_HD void stage_hessian(const Params& P, const Accel1& f, const StageJac& J, do
     q.q4 = -zla + zua;
     q.R = 1.0; q.r = -zlu + zuu; q.sig = 0.0;
   }
-}
-
-// ---------------------------------------------------------------------------------------
-// Warm start: every problem of a batch may start from one reference central-path point (the
-// batch-mean problem solved down to mu_ref ~ 1e-3) instead of the generic roll-out.  That skips
-// the globalisation phase (about 7 of 27 iterations); at smaller mu_ref the iterate sits too close
-// to the reference's active bounds and the method jams, so 1e-3 it is.  The reference column is
-// REF_ROWS x (N+1) doubles: the 17 iterate rows followed by one row of scalars (node 0..).
-// ---------------------------------------------------------------------------------------
-enum : int { REF_ROWS = N_ITER + 1, REF_OK = 0, REF_MU = 1, REF_S = 2, REF_TF = 3, REF_ZLT = 4, REF_ZUT = 5,
-             REF_SG1 = 6, REF_SG2 = 7, REF_ZS1 = 8, REF_ZS2 = 9, REF_NU3 = 10, REF_NSCAL = 11 };
-
-// ref[(row * (N+1)) + k]; written by the cooperative kernel's reference solve (coop_store_ref)
-// Start point of one problem from the reference column (lengths are stored divided by the
-// reference's distance scale S_ref = r_periapsis, LO:107, so they are rescaled to this problem's).
-LM_NOINLINE bool init_from_ref(const Params& P, const Mesh& M, const Ws& W, const double* ref, Scal& s,
-                               double* mu_out) {
-  const int N1 = M.N + 1;
-  const double* sc = ref + N_ITER * N1;
-  if (!(sc[REF_OK] > 0.5)) return false;
-  const double r = sc[REF_S] * P.Sinv, ri = P.S / sc[REF_S];
-  {
-    double* s0 = W.stage(0);
-#pragma unroll
-    for (int i = 0; i < 6; ++i) { WS_AT(s0, F_Z + i) = 0.0; WS_AT(s0, N_ITER + F_Z + i) = 0.0; WS_AT(s0, F_DS + i) = 0.0; }
-  }
-  for (int k = 1; k <= M.N; ++k) {
-    double* sp = W.stage(k);
-#pragma unroll
-    for (int f = 0; f < N_ITER; ++f) {
-      double v = ref[f * N1 + k];
-      if (f < 4) v *= r;                               // y, vy, x, vx
-      else if (f >= F_LAM && f < F_LAM + 4) v *= ri;   // multipliers of those rows
-      WS_AT(sp, f) = v;
-    }
-#pragma unroll
-    for (int i = 0; i < N_STEP; ++i) WS_AT(sp, R_STEP + i) = 0.0;
-  }
-  s.tf = dmin(sc[REF_TF], 0.99 * P.tf_ub);
-  s.zLt = sc[REF_ZLT]; s.zUt = sc[REF_ZUT];
-  s.sg1 = sc[REF_SG1]; s.sg2 = sc[REF_SG2]; s.zs1 = sc[REF_ZS1]; s.zs2 = sc[REF_ZS2]; s.nu3 = sc[REF_NU3];
-  *mu_out = sc[REF_MU];
-  return true;
 }
 
 // ---------------------------------------------------------------------------------------
@@ -1306,6 +1348,40 @@ LM_HD void ipm_begin(const Options& O, IpmState& S) {
   S.iters_prior = 0;
 }
 
+// Start of one problem on the sweeps SW: the caller's start point if G has one (lmato_set_initial_guess), else the
+// batch reference if `ref` holds one (it then also gives the barrier parameter), else the built-in roll-out.
+template <class SW, class WS>
+LM_HD void ipm_start(const Params& P, const Mesh& M, const Options& O, const WS& W, const GuessSrc& G, const double* ref,
+                     IpmState& S) {
+  ipm_begin(O, S);
+  double mu0 = 0.0;
+  if (G.traj) {
+    start_from_guess<SW>(P, M, O, W, G, S.cur);
+    S.from_guess = true;
+  } else if (ref && start_from_ref<SW>(P, M, O, W, ref, S.cur, &mu0)) {
+    S.warm = true;
+    S.ctl.mu = mu0;
+    S.ctl.tau = dmax(O.tau_min, 1.0 - mu0);
+  } else {
+    start_rollout<SW>(P, M, O, W, S.cur);
+  }
+}
+
+// After ipm_iterate_t has finished a problem: a warm start, or a caller's start point, that did not converge is
+// restarted from the built-in roll-out, with the iterations spent so far reported with the rest.  (IPOPT would enter
+// its feasibility restoration phase from such a point, e.g. from the reference's all-zero start values LO:39, 83-96;
+// this solver's substitute is a start point that is dynamically feasible by construction.)  Returns true if it
+// restarted.
+template <class SW, class WS>
+LM_HD bool ipm_restart(const Params& P, const Mesh& M, const Options& O, const WS& W, IpmState& S) {
+  if (!(S.warm || S.from_guess) || S.ctl.status == ST_CONVERGED) return false;
+  const int prior = S.iters_prior + S.ctl.iter;
+  ipm_begin(O, S);
+  S.iters_prior = prior;
+  start_rollout<SW>(P, M, O, W, S.cur);
+  return true;
+}
+
 // Node k of iterate `cur` in a thread's workspace column with the iterate rows of SW (Sweeps7 / Sweeps8): x = the six
 // states and the control, lam = the multipliers of the ydot, xdot and angledot rows; either may be null.
 template <class SW>
@@ -1323,7 +1399,8 @@ LM_HD void ws_node(const Ws& W, int cur, int k, double* x, double* lam) {
 
 // Sweeps policy of the 7-state formulation (dcost = 0); ascent_ipm_dc.cuh provides the 8-state one.
 struct Sweeps7 {
-  enum : int { NFIELDS = N_FIELDS, NITER = N_ITER, FZ = F_Z, FU = F_U, FLAM = F_LAM, REFROWS = REF_ROWS };
+  enum : int { NFIELDS = N_FIELDS, NITER = N_ITER, FZ = F_Z, FU = F_U, FLAM = F_LAM, REFROWS = REF_ROWS, MOVE_TERM = 0,
+               LANES_PER_PROBLEM = 1 };
   LM_HD static int n_eq(const Ws&, int N) { return 6 * N + 3; }
   LM_HD static int n_bd(const Ws&, int N) { return 4 * N + 4; }
   LM_HD static bool backward(const Params& P, const Mesh& M, const Options& O, const Ws& W, int src, const Scal& c0,
@@ -1339,13 +1416,21 @@ struct Sweeps7 {
                          double alpha_lam, int mode, Scal& t, double* pimax) {
     eval_pass(P, M, O, W, src, dst, c0, ts, mu, dw, alpha, alpha_z, alpha_lam, mode, t, pimax);
   }
-  LM_HD static void guess(const Params& P, const Mesh& M, const Options& O, const Ws& W, Scal& s) { init_guess(P, M, O, W, s); }
-  LM_HD static void guess_from(const Params& P, const Mesh& M, const Options& O, const Ws& W, const GuessSrc& G, Scal& s) {
-    init_from_guess(P, M, O, W, G, s);
+  // start points (start_rollout, start_from_guess, start_from_ref): node k into this layout's rows, node 0 pinned at
+  // zero (LO:145-151: its state and step rows are literal zeros, so that the sweeps read "node k-1" without a special
+  // case at k = 1)
+  LM_HD static void store_node(const Ws& W, int k, const double* x) {
+    double* sp = W.stage(k);
+#pragma unroll
+    for (int f = 0; f < NODE_N7; ++f)
+      if (f != NODE_LAM + 6) WS_AT(sp, row7(f)) = x[f];
+#pragma unroll
+    for (int i = 0; i < N_STEP; ++i) WS_AT(sp, R_STEP + i) = 0.0;
   }
-  LM_HD static bool load_ref(const Params& P, const Mesh& M, const Options&, const Ws& W, const double* ref, Scal& s,
-                             double* mu) {
-    return init_from_ref(P, M, W, ref, s, mu);
+  LM_HD static void zero_node0(const Ws& W) {
+    double* s0 = W.stage(0);
+#pragma unroll
+    for (int i = 0; i < 6; ++i) { WS_AT(s0, F_Z + i) = 0.0; WS_AT(s0, N_ITER + F_Z + i) = 0.0; WS_AT(s0, F_DS + i) = 0.0; }
   }
   LM_HD static void node(const Ws& W, int cur, int k, double* x, double* lam) { ws_node<Sweeps7>(W, cur, k, x, lam); }
   LM_HD static void remerit(const Mesh&, const Options&, const Ws&, int, double, Scal&) {}
@@ -1505,23 +1590,9 @@ LM_HD bool ipm_iterate_t(const Params& P, const Mesh& M, const Options& O, const
   return false;
 }
 
-LM_HD bool ipm_iterate(const Params& P, const Mesh& M, const Options& O, const Ws& W, IpmState& S) {
-  return ipm_iterate_t<Sweeps7>(P, M, O, W, S);
-}
-
 LM_HD void ipm_result(const IpmState& S, SolveOut& out) {
   out.tf = S.cur.tf; out.status = S.ctl.status; out.iters = S.iters_prior + S.ctl.iter; out.kkt = S.err0; out.mu = S.ctl.mu;
   out.cur = S.src;
-}
-
-// One complete solve of one problem (host simulator; the kernel interleaves ipm_iterate with barriers).
-LM_HD void ipm_solve(const Params& P, const Mesh& M, const Options& O, const Ws& W, bool have_guess,
-                     SolveOut& out) {
-  IpmState S;
-  if (!have_guess) init_guess(P, M, O, W, S.cur);
-  ipm_begin(O, S);
-  while (!ipm_iterate(P, M, O, W, S)) {}
-  ipm_result(S, out);
 }
 
 }  // namespace lmato

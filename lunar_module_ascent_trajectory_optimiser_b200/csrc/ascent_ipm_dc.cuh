@@ -81,69 +81,8 @@ LM_HD void solveET8(const StageJac& J, double* g) {
   g[0] = w0; g[1] = w1; g[2] = w2; g[3] = w3; g[4] = w4; g[5] = w5; g[6] = w6; g[7] = w7;
 }
 
-// ---------------------------------------------------------------------------------------
-// start points: the code shared with the 7-state sweeps (ascent_ipm.cuh: init_guess_t / init_from_guess_t), on
-// this layout
-struct Layout8 {
-  enum : int { FZ = F_Z, FU = F_U, FLAM = F_LAM, NLAM = 7, FZLA = F_ZLA, FZUA = F_ZUA, FZLU = F_ZLU, FZUU = F_ZUU,
-               NITER = N_ITER, FDS = F_DS, FDU = F_DU, RSTEP = R_STEP, NSTEP = N_STEP,
-               MOVE = 1, FPP = F_PP, FPN = F_PN, FZPP = F_ZPP, FZPN = F_ZPN };
-};
-LM_NOINLINE void init_guess(const Params& P, const Mesh& M, const Options& O, const Ws& W, Scal& s) {
-  init_guess_t<Layout8>(P, M, O, W, s);
-}
-
-// Start from a reference column produced by the (cheaper) 7-state solve of the batch-mean problem without
-// the move term: at mu_ref ~ 1e-3 >> w the two central paths practically coincide.  The slack pair is put
-// exactly on its own central path for the reference's moves (z_p + z_n = 2w, p z_p = n z_n = mu) and the
-// multiplier of the u row follows from dual feasibility, lam_6 = w - z_p.
-LM_NOINLINE bool init_from_ref7(const Params& P, const Mesh& M, const Options& O, const Ws& W, const double* ref,
-                                Scal& s, double* mu_out) {
-  const int N1 = M.N + 1;
-  const int NI7 = lmato::N_ITER;                       // 17 rows in the 7-state layout
-  const double* sc = ref + NI7 * N1;
-  if (!(sc[REF_OK] > 0.5)) return false;
-  const double r = sc[REF_S] * P.Sinv, ri = P.S / sc[REF_S];
-  const double mu = sc[REF_MU], w = O.w_dcost;
-  {
-    double* s0 = W.stage(0);
-#pragma unroll
-    for (int i = 0; i < 6; ++i) { WS_AT(s0, F_Z + i) = 0.0; WS_AT(s0, N_ITER + F_Z + i) = 0.0; WS_AT(s0, F_DS + i) = 0.0; }
-    WS_AT(s0, F_U) = 0.0; WS_AT(s0, N_ITER + F_U) = 0.0; WS_AT(s0, F_DU) = 0.0;
-  }
-  double u_prev = 0.0;
-  for (int k = 1; k <= M.N; ++k) {
-    double* sp = W.stage(k);
-#pragma unroll
-    for (int f = 0; f < 7; ++f) WS_AT(sp, f) = ref[f * N1 + k] * (f < 4 ? r : 1.0);                 // states, u
-#pragma unroll
-    for (int i = 0; i < 6; ++i) WS_AT(sp, F_LAM + i) = ref[(lmato::F_LAM + i) * N1 + k] * (i < 4 ? ri : 1.0);
-    WS_AT(sp, F_ZLA) = ref[lmato::F_ZLA * N1 + k]; WS_AT(sp, F_ZUA) = ref[lmato::F_ZUA * N1 + k];
-    WS_AT(sp, F_ZLU) = ref[lmato::F_ZLU * N1 + k]; WS_AT(sp, F_ZUU) = ref[lmato::F_ZUU * N1 + k];
-    const double u = ref[lmato::F_U * N1 + k];
-    const double v = u - u_prev;
-    const double tt = (mu + sqrt(mu * mu + w * w * v * v)) / w;
-    const double pp = 0.5 * (tt + v), pn = 0.5 * (tt - v);
-    WS_AT(sp, F_PP) = pp; WS_AT(sp, F_PN) = pn;
-    WS_AT(sp, F_ZPP) = mu / pp; WS_AT(sp, F_ZPN) = mu / pn;
-    WS_AT(sp, F_LAM + 6) = w - mu / pp;
-#pragma unroll
-    for (int i = 0; i < N_STEP; ++i) WS_AT(sp, R_STEP + i) = 0.0;
-    u_prev = u;
-  }
-  s.tf = dmin(sc[REF_TF], 0.99 * P.tf_ub);
-  s.zLt = sc[REF_ZLT]; s.zUt = sc[REF_ZUT];
-  s.sg1 = sc[REF_SG1]; s.sg2 = sc[REF_SG2]; s.zs1 = sc[REF_ZS1]; s.zs2 = sc[REF_ZS2]; s.nu3 = sc[REF_NU3];
-  *mu_out = mu;
-  return true;
-}
-
-// Caller-supplied start point (see ascent_ipm.cuh: init_from_guess), 8-state layout: the move slack pair
-// is put on its central path for the guess's control moves.
-LM_NOINLINE void init_from_guess(const Params& P, const Mesh& M, const Options& O, const Ws& W, const GuessSrc& G,
-                                 Scal& s) {
-  init_from_guess_t<Layout8>(P, M, O, W, G, s);
-}
+static_assert((int)F_LAM == NODE_LAM && (int)F_ZLA == NODE_ZLA && (int)F_ZUU == NODE_ZUU && (int)F_PP == NODE_PP &&
+              (int)F_ZPN == NODE_ZPN && (int)N_ITER == NODE_N, "the 8-state rows are the rows of a start node (ascent_ipm.cuh)");
 
 // ---------------------------------------------------------------------------------------
 // Staging tiles (see ascent_ipm.cuh: tl_*): which rows each sweep reads per stage and where they sit
@@ -799,7 +738,8 @@ LM_SWEEP void riccati_forward(const Params& P, const Mesh& M, const Options& O, 
 
 // Sweeps policy of the 8-state (DCOST) formulation.
 struct Sweeps8 {
-  enum : int { NFIELDS = dc::N_FIELDS, NITER = dc::N_ITER, FZ = dc::F_Z, FU = dc::F_U, FLAM = dc::F_LAM, REFROWS = dc::REF_ROWS };
+  enum : int { NFIELDS = dc::N_FIELDS, NITER = dc::N_ITER, FZ = dc::F_Z, FU = dc::F_U, FLAM = dc::F_LAM, REFROWS = dc::REF_ROWS,
+               MOVE_TERM = 1, LANES_PER_PROBLEM = 1 };
   LM_HD static int n_eq(const Ws&, int N) { return 7 * N + 3; }
   LM_HD static int n_bd(const Ws&, int N) { return 6 * N + 4; }
   LM_HD static bool backward(const Params& P, const Mesh& M, const Options& O, const Ws& W, int src, const Scal& c0,
@@ -815,13 +755,18 @@ struct Sweeps8 {
                          double alpha_lam, int mode, Scal& t, double* pimax) {
     dc::eval_pass(P, M, O, W, src, dst, c0, ts, mu, dw, alpha, alpha_z, alpha_lam, mode, t, pimax);
   }
-  LM_HD static void guess(const Params& P, const Mesh& M, const Options& O, const Ws& W, Scal& s) { dc::init_guess(P, M, O, W, s); }
-  LM_HD static void guess_from(const Params& P, const Mesh& M, const Options& O, const Ws& W, const GuessSrc& G, Scal& s) {
-    dc::init_from_guess(P, M, O, W, G, s);
+  // start points (ascent_ipm.cuh: start_rollout, ...): node k into the 8-state rows; node 0 pinned at zero, MV(0) = 0
+  LM_HD static void store_node(const Ws& W, int k, const double* x) {
+    double* sp = W.stage(k);
+#pragma unroll
+    for (int f = 0; f < NODE_N; ++f) WS_AT(sp, f) = x[f];
+#pragma unroll
+    for (int i = 0; i < dc::N_STEP; ++i) WS_AT(sp, dc::R_STEP + i) = 0.0;
   }
-  LM_HD static bool load_ref(const Params& P, const Mesh& M, const Options& O, const Ws& W, const double* ref,
-                             Scal& s, double* mu) {
-    return dc::init_from_ref7(P, M, O, W, ref, s, mu);      // the reference is produced by the 7-state solve
+  LM_HD static void zero_node0(const Ws& W) {
+    double* s0 = W.stage(0);
+#pragma unroll
+    for (int i = 0; i < 7; ++i) { WS_AT(s0, dc::F_Z + i) = 0.0; WS_AT(s0, dc::N_ITER + dc::F_Z + i) = 0.0; WS_AT(s0, dc::F_DS + i) = 0.0; }
   }
   LM_HD static void node(const Ws& W, int cur, int k, double* x, double* lam) { ws_node<Sweeps8>(W, cur, k, x, lam); }
   LM_HD static void remerit(const Mesh&, const Options&, const Ws&, int, double, Scal&) {}

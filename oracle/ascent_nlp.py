@@ -526,7 +526,7 @@ class AscentNLP:
         83-96), which needs IPOPT's full restoration phase.  Otherwise: a dynamically
         consistent roll-out of a bang-bang pitch-acceleration profile (+0.9 until t1, -0.9
         until t1+t2, then 0), the shape of Angle_vs_Time.png.  The product builds the same
-        start on the device (csrc/ascent_ipm.cuh: init_guess) -- restated here, not shared."""
+        start on the device (csrc/ascent_ipm.cuh: start_rollout) -- restated here, not shared."""
         nm, p, K, nv = self.nm, self.p, self.K, self.nv
         x = np.zeros(self.n)
         if tf0 is None:

@@ -214,3 +214,63 @@ def test_higher_order_collocation_source_matches_goldens(hostsim):
         st, tf, it, traj = solve(g["rows"][:, b], int(g["disp_nt"]), 3)
         assert st == 0 and abs(tf - g["disp_tf"][b]) / tf < 1e-9
         assert _rel(traj, g["disp_traj"][b])[:9].max() < 1e-5
+
+
+def test_start_points_on_every_layout(hostsim, monkeypatch):
+    """Start points through the kernels' own ipm_start / ipm_restart on both thread layouts (hostsim_solve: Sweeps8
+    with DCOST, Sweeps7 without) and the cooperative layout (hostsim_solve_coop: MOVE 1 / 0): the batch reference of
+    hostsim_reference (the ref_mode 1 solve), a caller's start point, an all-zero start point that has to be
+    restarted from the roll-out, and a reference column that holds no reference (REF_OK = 0)."""
+    monkeypatch.delenv("CIRCULAR", raising=False)
+    monkeypatch.delenv("VREC", raising=False)
+    nt, ref_rows = 200, 23                 # the reference buffer as the handle sizes it (the 8-state REF_ROWS)
+    ptr = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
+    for fixture, dcost in (("elliptical_dcost1e-5_disp4_seed11_nt200.npz", True),
+                           ("elliptical_dispersions8_seed11_nt200.npz", False)):
+        g = np.load(os.path.join(GOLDEN, fixture))
+        rows, gold_tf, gold_traj = g["rows"][:, :4], g["tf"][:4], g["traj"][:4]
+        if dcost:
+            monkeypatch.setenv("WDC", repr(10.0 * 1e-5 / 199)); monkeypatch.setenv("NPOL", "2")
+        else:
+            monkeypatch.delenv("WDC", raising=False); monkeypatch.delenv("NPOL", raising=False)
+        ref = np.zeros((ref_rows, nt))
+        mean = np.ascontiguousarray(rows.mean(axis=1))              # the batch-mean problem (mean_params_kernel)
+        assert hostsim.hostsim_reference(ptr(mean), nt, C.c_double(1e-3), ptr(ref)) == 0
+        no_ref = np.zeros((ref_rows, nt))
+        # the same reference stored at twice the distance scale S_ref: lengths halved, the multipliers of their rows
+        # doubled (csrc/ascent_ipm.cuh: rows F_LAM = 7.., scalar row N_ITER = 17, REF_S = 2).  Every factor is a power
+        # of two, so the reader's rescaling must give the same start point bit for bit.
+        rescaled = ref.copy()
+        rescaled[0:4] /= 2; rescaled[7:11] *= 2; rescaled[17, 2] *= 2
+
+        def solve(fn, b, traj=None, tf=None, column=None):
+            hostsim.hostsim_set_start(ptr(traj), ptr(tf), ptr(column))
+            try:
+                return _solve(hostsim, rows[:, b], nt=nt, fn=fn)
+            finally:
+                hostsim.hostsim_set_start(None, None, None)
+
+        warm = {}
+        for fn in ("hostsim_solve", "hostsim_solve_coop"):
+            cold = [solve(fn, b) for b in range(4)]
+            warm[fn] = [solve(fn, b, column=ref) for b in range(4)]
+            for b in range(4):
+                assert cold[b][0] == 0 and warm[fn][b][0] == 0, (fn, b)
+                assert abs(warm[fn][b][1] - gold_tf[b]) / gold_tf[b] < 1e-8, (fn, b)
+                st, tf, it, traj = solve(fn, b, column=rescaled)
+                assert (st, tf, it) == warm[fn][b][:3] and np.array_equal(traj, warm[fn][b][3]), (fn, b)
+                # a caller's start point: the solution of the neighbouring problem
+                n = b ^ 1
+                st, tf, it, _ = solve(fn, b, np.ascontiguousarray(gold_traj[n]), np.array([gold_tf[n]]))
+                assert st == 0 and abs(tf - gold_tf[b]) / gold_tf[b] < 1e-8, (fn, b)
+                # an all-zero start point fails and is restarted from the roll-out: the cold optimum, more iterations
+                st, tf, it, _ = solve(fn, b, np.zeros((10, nt)), np.zeros(1))
+                assert st == 0 and abs(tf - cold[b][1]) / cold[b][1] < 1e-8 and it > cold[b][2], (fn, b, it, cold[b][2])
+                # a reference column without a reference: the cold start, bit for bit
+                st, tf, it, traj = solve(fn, b, column=no_ref)
+                assert (st, tf, it) == cold[b][:3] and np.array_equal(traj, cold[b][3]), (fn, b)
+            its_warm, its_cold = np.mean([w[2] for w in warm[fn]]), np.mean([c[2] for c in cold])
+            print(f"\n[start] {fixture} {fn}: iterations warm {its_warm:.2f} cold {its_cold:.2f}")
+            assert its_warm < its_cold, (fn, its_warm, its_cold)
+        for a, c in zip(warm["hostsim_solve"], warm["hostsim_solve_coop"]):
+            assert abs(a[1] - c[1]) / a[1] < 1e-11 and abs(a[2] - c[2]) <= 1, (a[:3], c[:3])

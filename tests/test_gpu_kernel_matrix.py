@@ -6,9 +6,10 @@ options, one of
     ascent_coop_kernel<G, GP, MOVE, BPS>          GP = 32 lanes per problem up to 8 problems per SM, else 8;
                                                   BPS = 2 CTAs per SM once one CTA per SM cannot hold the batch;
                                                   MOVE = 0 no DCOST, 1 DCOST, 2 the circular model with DCOST
-and every instantiation has its own start-point code (guess / guess_from / load_ref) and reads the converged iterate
-through its own workspace layout (SW::node) for the shared result writer (csrc/ascent_result.cuh), which the
-cooperative kernels run with the problem's lanes summing over the group.  The table below reaches each of them; a
+and every instantiation writes the shared start points (start_rollout / start_from_guess / start_from_ref) through its
+own workspace layout (SW::store_node) and reads the converged iterate through it (SW::node) for the shared result writer
+(csrc/ascent_result.cuh), which the cooperative kernels run with the problem's lanes summing over the group.  The
+table below reaches each of them; a
 test id names the instantiation.  Batch sizes are derived from the device's SM
 count with the dispatcher's rules, so the same table picks the same kernels on any GPU (a variant whose batch-size
 window is empty there is skipped).
@@ -266,7 +267,7 @@ START_POINTS = [("thread-sweeps8", "thread", 0, 1e-5), ("thread-sweeps7", "threa
 
 @pytest.mark.parametrize("vid,kernel,lanes,dcost", START_POINTS, ids=[s[0] for s in START_POINTS])
 def test_start_points(lm, golden_dir, vid, kernel, lanes, dcost):
-    """`guess=` on each kernel's own guess_from: the fixture problems started from the solutions of the same problems
+    """`guess=` on each kernel (start_from_guess through its own layout): the fixture problems started from the solutions of the same problems
     at +0.5 % thrust reach the oracle's optimum in fewer iterations than from the cold start; on the thread kernel an
     all-zero start point is abandoned and the problem restarted from the roll-out, which reaches the cold optimum."""
     if dcost > 0:

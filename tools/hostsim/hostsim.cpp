@@ -43,14 +43,26 @@ static Options make_options(double tol, double obj_scale, double mu_min_factor, 
 // the model the CIRCULAR environment variable selects
 static int model_from_env() { return getenv("CIRCULAR") ? LMATO_MODEL_CIRCULAR : LMATO_MODEL_ELLIPTICAL; }
 
-// One problem on the sweeps SW from their built-in start point, with the results written as the kernels write them
-// (B = 1, b = 0).
+// Start point of the next hostsim_solve / hostsim_solve_coop calls (B = 1, b = 0): a caller's start point
+// (guess_traj [10][nt] in the output layout, guess_tf), the counterpart of lmato_set_initial_guess, and a reference
+// column ([REF_ROWS][nt], as hostsim_reference writes it), the counterpart of the handle's warm-start reference.  Any
+// of them may be NULL; with neither a guess nor a reference holding REF_OK the solve starts from the roll-out.
+static const double* g_guess_traj = nullptr;
+static const double* g_guess_tf = nullptr;
+static const double* g_ref = nullptr;
+extern "C" void hostsim_set_start(const double* guess_traj, const double* guess_tf, const double* ref) {
+  g_guess_traj = guess_traj; g_guess_tf = guess_tf; g_ref = ref;
+}
+
+// One problem on the sweeps SW, started and restarted as the kernels do (ipm_start / ipm_restart), with the results
+// written as the kernels write them (B = 1, b = 0).
 template <class SW, class WS>
 static void solve_one(const ResultOut& R, const Params& P, const Mesh& M, const Options& O, int model, const WS& W) {
   IpmState S;
-  ipm_begin(O, S);
-  SW::guess(P, M, O, W, S.cur);
-  while (!ipm_iterate_t<SW>(P, M, O, W, S)) {}
+  ipm_start<SW>(P, M, O, W, GuessSrc{g_guess_traj, g_guess_tf, 1, 0}, g_ref, S);
+  do {
+    while (!ipm_iterate_t<SW>(P, M, O, W, S)) {}
+  } while (ipm_restart<SW>(P, M, O, W, S));
   write_results<SW, 1>(R, P, M, O.obj_scale, model, W, 0, 1u, S, 0);
 }
 
@@ -78,6 +90,7 @@ int main(int argc, char** argv) {
   std::vector<double> ws((size_t)nfields * LANES * (N + 1), 0.0);   // one warp block, lane 0 used
   std::vector<double> tile(2 * TILE_ROWS, 0.0);
   Ws W{ws.data(), (long)nfields * LANES, tile.data()};
+  std::vector<double> traj((size_t)LMATO_NVAR * nt);
   std::mt19937_64 rng(11);
   std::uniform_real_distribution<double> U(0.0, 1.0);
   int nfail = 0, itsum = 0, itmax = 0;
@@ -94,27 +107,20 @@ int main(int argc, char** argv) {
     if (only >= 0 && p != only) continue;
     Params P = derive_params(make_params(Ft, M0, Mdot, addm, rp, ra).data(), 1, 0, LMATO_MODEL_ELLIPTICAL);
     std::fill(ws.begin(), ws.end(), 0.0);
-    SolveOut out;
-    if (O.w_dcost > 0) {
-      IpmState S;
-      dc::init_guess(P, M, O, W, S.cur);
-      ipm_begin(O, S);
-      while (!ipm_iterate_t<Sweeps8>(P, M, O, W, S)) {}
-      ipm_result(S, out);
-    } else {
-      ipm_solve(P, M, O, W, false, out);
-    }
-    itsum += out.iters; if (out.iters > itmax) itmax = out.iters;
-    if (out.status != 0) ++nfail;
-    if (verbose || nprob <= 20 || out.status != 0)
-      printf("p %4d status %d iters %3d kkt %.2e mu %.1e tf %.10f tf_s %.8f  (Ft %.1f M0 %.1f Mdot %.4f addm %.2e rp %.0f ra %.0f)\n",
-             p, out.status, out.iters, out.kkt, out.mu, out.tf, out.tf * P.T, Ft, M0, Mdot, addm, rp, ra);
+    int status, iters;
+    double tf, kkt, fmass;
+    const ResultOut R{traj.data(), &tf, &fmass, &status, &iters, &kkt, nullptr, 1};
+    if (O.w_dcost > 0) solve_one<Sweeps8>(R, P, M, O, LMATO_MODEL_ELLIPTICAL, W);
+    else solve_one<Sweeps7>(R, P, M, O, LMATO_MODEL_ELLIPTICAL, W);
+    itsum += iters; if (iters > itmax) itmax = iters;
+    if (status != 0) ++nfail;
+    if (verbose || nprob <= 20 || status != 0)
+      printf("p %4d status %d iters %3d kkt %.2e tf %.10f tf_s %.8f  (Ft %.1f M0 %.1f Mdot %.4f addm %.2e rp %.0f ra %.0f)\n",
+             p, status, iters, kkt, tf, tf * P.T, Ft, M0, Mdot, addm, rp, ra);
     if (p == 0 && nprob == 1) {
-      const int b = out.cur;
-      const double* sp = W.stage(N);
-      printf("final y %.9f x %.9f vy %.9f vx %.9f\n", WS_AT(sp, b * N_ITER + F_Z + 0) * P.S, WS_AT(sp, b * N_ITER + F_Z + 2) * P.S,
-             WS_AT(sp, b * N_ITER + F_Z + 1) * P.S, WS_AT(sp, b * N_ITER + F_Z + 3) * P.S);
-      printf("final mass %.9f\n", P.M0 - P.fuel * P.mflow * P.T * out.tf);
+      printf("final y %.9f x %.9f vy %.9f vx %.9f\n", traj[LMATO_V_Y * nt + N] * P.S, traj[LMATO_V_X * nt + N] * P.S,
+             traj[LMATO_V_YDOT * nt + N] * P.S, traj[LMATO_V_XDOT * nt + N] * P.S);
+      printf("final mass %.9f\n", fmass);
     }
   }
   printf("solved %d problems: %d failures, mean iters %.1f, max %d\n", nprob, nfail, (double)itsum / nprob, itmax);
@@ -252,9 +258,35 @@ extern "C" int hostsim_solve_colloc(const double* raw14, int nt, const double* t
   return status;
 }
 
+// The reference solve of the batch warm start (lmato_solve_batch's ref_mode 1 launch) for the problem raw14 on a
+// uniform mesh of nt nodes: the cooperative sweeps without the move term, solved down to mu_ref (tol = 10 mu_ref,
+// mu_min_factor 0.1, no polish), started from the reference already in ref_out if it holds one, then stored there
+// ([REF_ROWS][nt]).  Returns the solve's status.
+extern "C" int hostsim_reference(const double* raw14, int nt, double mu_ref, double* ref_out) {
+  const int N = nt - 1;
+  std::vector<double> h(N + 1), tau(N + 1);
+  for (int k = 0; k <= N; ++k) { tau[k] = (double)k / N; h[k] = k ? tau[k] - tau[k - 1] : 0.0; }
+  Mesh M{N, h.data(), tau.data()};
+  Options O = make_options(10.0 * mu_ref, 10.0, 0.1, 0, 0.0);
+  if (getenv("KEPS")) O.kappa_eps = atof(getenv("KEPS"));
+  if (getenv("KMU")) O.kappa_mu = atof(getenv("KMU"));
+  const Params P = derive_params(raw14, 1, 0, model_from_env());
+  std::vector<double> ws((size_t)coop::coop_doubles_per_problem(nt), 0.0), scr(coop::SCR_DOUBLES, 0.0);
+  coop::Cws W{ws.data(), nt, scr.data(), 0, 1u, 1u, 0.0, 0.0, 0, 0u};
+  using SW = SweepsCoop<1, 1, false, false>;
+  IpmState S;
+  ipm_start<SW>(P, M, O, W, GuessSrc{nullptr, nullptr, 1, 0}, ref_out, S);
+  do {
+    while (!ipm_iterate_t<SW>(P, M, O, W, S)) {}
+  } while (ipm_restart<SW>(P, M, O, W, S));
+  SW::store_ref(P, M, W, S.src, S.cur, S.ctl.mu, S.ctl.status == ST_CONVERGED, ref_out);
+  return S.ctl.status;
+}
+
 // Batch warm start on the host (what lmato_solve_batch does on the device): the batch-mean problem is solved to
-// mu_ref by the cooperative sweeps without the move term and stored as the reference; every dispersed problem
-// then starts from it.  Returns the mean iteration count; used to study barrier-update strategies on the CPU.
+// mu_ref by hostsim_reference, and every dispersed problem then starts from that reference on the cooperative sweeps
+// (with the move term if wdc > 0).  It leaves no start point set (hostsim_set_start).  Returns the mean iteration
+// count; used to study barrier-update strategies on the CPU.
 //   hostsim_warm_batch(nprob, nt, wdc, mu_ref, out_iters[nprob], out_status[nprob], out_tf[nprob])
 extern "C" double hostsim_warm_batch(int nprob, int nt, double wdc, double mu_ref, int* out_iters, int* out_status, double* out_tf) {
   const int N = nt - 1;
@@ -285,39 +317,18 @@ extern "C" double hostsim_warm_batch(int nprob, int nt, double wdc, double mu_re
     const double v[6] = {Ft, M0, Mdot, addm, rp, ra};
     for (int i = 0; i < 6; ++i) mean[i] += v[i] / nprob;
   }
-  std::vector<double> ws((size_t)coop::coop_doubles_per_problem(nt), 0.0), scr(coop::SCR_DOUBLES, 0.0);
   std::vector<double> ref((size_t)dc::REF_ROWS * nt, 0.0);
+  hostsim_reference(make_params(mean[0], mean[1], mean[2], mean[3], mean[4], mean[5]).data(), nt, mu_ref, ref.data());
+  std::vector<double> ws((size_t)coop::coop_doubles_per_problem(nt), 0.0), scr(coop::SCR_DOUBLES, 0.0);
   coop::Cws W{ws.data(), nt, scr.data(), 0, 1u, 1u, 0.0, 0.0, 0, 0u};
-  {   // reference solve
-    const Params Pm = derive_params(make_params(mean[0], mean[1], mean[2], mean[3], mean[4], mean[5]).data(), 1, 0,
-                                    LMATO_MODEL_ELLIPTICAL);
-    Options R = O;
-    R.tol = 10.0 * mu_ref; R.mu_min_factor = 0.1; R.n_polish = 0; R.w_dcost = 0.0;
-    IpmState S;
-    ipm_begin(R, S);
-    SweepsCoop<1, 1, false, false>::guess(Pm, M, R, W, S.cur);
-    while (!ipm_iterate_t<SweepsCoop<1, 1, false, false>>(Pm, M, R, W, S)) {}
-    SolveOut out; ipm_result(S, out);
-    SweepsCoop<1, 1, false, false>::store_ref(Pm, M, W, out.cur, S.cur, S.ctl.mu, out.status == ST_CONVERGED, ref.data());
-  }
-  double itsum = 0;
+  hostsim_set_start(nullptr, nullptr, ref.data());
+  double itsum = 0, fmass;
   for (int p = 0; p < nprob; ++p) {
-    IpmState S;
-    ipm_begin(O, S);
-    double mu0 = 0.0;
-    SolveOut out;
-    if (wdc > 0) {
-      SweepsCoop<1, 1, true, false>::load_ref(Ps[p], M, O, W, ref.data(), S.cur, &mu0);
-      S.warm = true; S.ctl.mu = mu0; S.ctl.tau = dmax(O.tau_min, 1.0 - mu0);
-      while (!ipm_iterate_t<SweepsCoop<1, 1, true, false>>(Ps[p], M, O, W, S)) {}
-    } else {
-      SweepsCoop<1, 1, false, false>::load_ref(Ps[p], M, O, W, ref.data(), S.cur, &mu0);
-      S.warm = true; S.ctl.mu = mu0; S.ctl.tau = dmax(O.tau_min, 1.0 - mu0);
-      while (!ipm_iterate_t<SweepsCoop<1, 1, false, false>>(Ps[p], M, O, W, S)) {}
-    }
-    ipm_result(S, out);
-    out_iters[p] = out.iters; out_status[p] = out.status; out_tf[p] = out.tf;
-    itsum += out.iters;
+    const ResultOut R{nullptr, out_tf + p, &fmass, out_status + p, out_iters + p, nullptr, nullptr, 1};
+    if (wdc > 0) solve_one<SweepsCoop<1, 1, true, false>>(R, Ps[p], M, O, LMATO_MODEL_ELLIPTICAL, W);
+    else solve_one<SweepsCoop<1, 1, false, false>>(R, Ps[p], M, O, LMATO_MODEL_ELLIPTICAL, W);
+    itsum += out_iters[p];
   }
+  hostsim_set_start(nullptr, nullptr, nullptr);
   return itsum / nprob;
 }
