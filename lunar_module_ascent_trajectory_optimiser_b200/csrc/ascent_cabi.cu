@@ -1,6 +1,6 @@
 // C ABI + kernels of the batched ascent solver (sm_100a).  See include/lmato_b200.h.
 //
-// Two kernels solve the same NLP with the same IPM driver (ipm_iterate_t, ascent_ipm.cuh):
+// Three kernels solve the same NLP with the same IPM driver (ipm_iterate_t, ascent_ipm.cuh):
 //   ascent_ipm_kernel   ONE PROBLEM PER THREAD, persistent warps, for batches that fill the GPU (>= ~1 wave of
 //                       148 x 256 problems).  The stage data of a problem (55-67 doubles x nt) streams through a
 //                       workspace in HBM laid out [stage][warp][field][lane]: every access of a warp is one
@@ -10,7 +10,9 @@
 //                       1 024 / 4 096-problem configurations, a 65 536 batch strong-scaled over 8 GPUs.  Model
 //                       evaluation is stage-parallel over the group and stored per stage; the Riccati recursion
 //                       runs on the stored records with the cost-to-go distributed by rows over the group.
-// Both claim problems from a device-side queue and never return to the host during a solve (barrier updates,
+//   ascent_colloc_kernel 8 OR 32 LANES PER PROBLEM (ascent_colloc.cuh), the general path for NODES = 3..6.
+// Each kernel sets up its shared constants and its workspace view and then runs one loop, solve_queue: it claims
+// problems from a device-side queue and never returns to the host during a solve (barrier updates,
 // fraction-to-boundary, filter line search and convergence masks live in the owning lanes).  Tensor cores are
 // not used: the stage blocks are 8x8 FP64 and the recursion over stages is sequential (DESIGN.md).
 #include <cuda_runtime.h>
@@ -101,6 +103,98 @@ static_assert(GuessSrc::V_Y == LMATO_V_Y && GuessSrc::V_YDOT == LMATO_V_YDOT && 
               GuessSrc::V_ANGLEDOT == LMATO_V_ANGLEDOT && GuessSrc::V_U == LMATO_V_ANGLEDOUBLEDOT,
               "the guess uses the output layout of include/lmato_b200.h");
 
+// How a warp leaves the problem queue of solve_queue.
+enum QueueExit {
+  kBlockBarrier,   // a block-wide vote every LMATO_SYNC_PERIOD-th round, which also keeps the warps of a CTA in step
+  kWarpVote        // each warp on its own, once the queue is empty and its last chunk is written
+};
+
+// The persistent problem queue of every solve kernel.  A warp holds a chunk of 32 / GP problems, GP =
+// SW::LANES_PER_PROBLEM lanes each (1 in the thread kernel); its groups run the IPM driver in lock step (same sweep at
+// the same time, each with its own lane mask), finished problems wait until the warp's whole chunk is done, then the
+// warp claims the next chunk.  IpmState (filter, barrier parameter, ...) is carried redundantly by the GP lanes of a
+// problem: every decision of the driver is a function of group-uniform values.  P is this problem's slot of the
+// kernel's shared Params; g and mask are this lane's index and lane mask in its group, as write_results takes them.
+// The driver is inlined here with one call site each of ipm_start, ipm_iterate_t, ipm_restart and write_results
+// (DESIGN.md section 3a).
+template <class SW, QueueExit EXIT, class WS>
+__device__ __forceinline__ void solve_queue(const KArgs& a, Params& P, const Mesh& M, const Options& O, const WS& W,
+                                            int g, unsigned mask) {
+  constexpr int GP = SW::LANES_PER_PROBLEM;
+  constexpr int PPW = 32 / GP;                 // problems per warp
+  const int lane = threadIdx.x & 31;
+  IpmState S;
+  bool active = false;        // this lane holds an unfinished problem
+  bool pending = false;       // this lane holds a finished problem whose results are not written yet
+  bool exhausted = false;     // the queue is empty (warp-uniform)
+  bool first = true;
+  long b = -1;
+  unsigned round = 0;
+  while (true) {
+    // ---- a warp whose problems are all finished claims the next chunk (warp-uniform branch) ----
+    const bool chunk_done = !__any_sync(0xffffffffu, active);
+    // ---- a finished chunk writes its results with all 32 lanes together: every row of the
+    //      [variable][node][problem] output is then one coalesced store per warp (the output
+    //      may be pinned host memory written over PCIe while the other warps keep computing) ----
+    if (chunk_done && __any_sync(0xffffffffu, pending)) {
+      if (pending) write_results<SW, GP>(a.res, P, M, O.obj_scale, a.model, W, g, mask, S, b);
+      pending = false;
+    }
+    if (!exhausted && chunk_done) {
+      // first chunk: static round-robin over CTAs (spreads a small batch over all SMs);
+      // afterwards: the device-wide queue
+      int chunk = 0;
+      if (first) {
+        chunk = (threadIdx.x / 32) * gridDim.x + blockIdx.x;
+        first = false;
+      } else {
+        if (lane == 0) chunk = atomicAdd(a.counter, 1) + gridDim.x * (kBlock / 32);
+        chunk = __shfl_sync(0xffffffffu, chunk, 0);
+      }
+      if ((long)chunk * PPW >= a.res.B) {
+        exhausted = true;
+      } else {
+        b = (long)chunk * PPW + lane / GP;
+        if (b < a.res.B) {
+          if (g == 0) P = derive_params(a.params, a.res.B, b, a.model, SW::MOVE_TERM == 2);
+          coop::Grp<GP>::sync(mask);
+          // ref_mode 2: start from the batch reference.  ref_mode 1 (the reference solve itself):
+          // start from the previous call's reference if the handle has one (consecutive batches of a
+          // campaign have nearly the same mean, so it re-converges in one or two iterations).
+          ipm_start<SW>(P, M, O, W, GuessSrc{a.guess_traj, a.guess_tf, a.res.B, b}, a.ref_mode != 0 ? a.ref : nullptr, S);
+          active = true;
+        }
+      }
+    }
+    if constexpr (EXIT == kBlockBarrier) {
+      // ---- all eight warps of the SM start each iteration together: they then run the same sweep
+      //      (same code) at the same time, which keeps the 32 KB instruction cache effective ----
+      // (every LMATO_SYNC_PERIOD-th round: a barrier per iteration costs more in waiting than it
+      //  gains, because line-search retries differ between warps; the imbalance averages out over
+      //  a few iterations while the warps stay close enough to share the instruction cache)
+      if ((round++ % LMATO_SYNC_PERIOD) == 0 && !__syncthreads_or((active || !exhausted) ? 1 : 0)) break;
+    } else {
+      // (no block barrier per iteration here: the warps of an SM are few and their sweeps are short; a warp that
+      //  waits for its neighbours' line-search retries loses more than the instruction cache gains)
+      if (exhausted && !__any_sync(0xffffffffu, active || pending)) break;
+    }
+    if (active && ipm_iterate_t<SW>(P, M, O, W, S)) {
+      if (ipm_restart<SW>(P, M, O, W, S)) continue;      // this problem restarts from another start point
+      active = false;
+      if constexpr (SW::STORES_REF) {
+        // ref_mode 1, the reference solve of the batch warm start: store the reference, write no results
+        if (a.ref_mode == 1) {
+          SolveOut out;
+          ipm_result(S, out);
+          SW::store_ref(P, M, W, out.cur, S.cur, S.ctl.mu, out.status == ST_CONVERGED, a.ref);
+          continue;
+        }
+      }
+      pending = true;      // results are written when the whole chunk is done (see above)
+    }
+  }
+}
+
 // SW = Sweeps7 (dcost = 0) or Sweeps8 (with the reference's move-suppression term, LO:99)
 template <class SW>
 __global__ void __launch_bounds__(kBlock, kBlocksPerSM) ascent_ipm_kernel(KArgs a) {
@@ -112,9 +206,6 @@ __global__ void __launch_bounds__(kBlock, kBlocksPerSM) ascent_ipm_kernel(KArgs 
   __shared__ Mesh sM;
   if (threadIdx.x == 0) { sO = a.O; sM = Mesh{a.N, a.h, a.tau}; }
   __syncthreads();
-  const Options& O = sO;
-  const Mesh& M = sM;
-  Params& P = sP[threadIdx.x].p;
   const long slot = (long)blockIdx.x * blockDim.x + threadIdx.x;
   const int lane = threadIdx.x & 31;
   const long nwarps = a.slots / LANES;
@@ -126,63 +217,8 @@ __global__ void __launch_bounds__(kBlock, kBlocksPerSM) ascent_ipm_kernel(KArgs 
   // (24-byte stride: conflict-free per half warp)
   Ws* sW = reinterpret_cast<Ws*>(sTiles + (size_t)(kBlock / 32) * 2 * TILE_ROWS * LANES);   // after the tiles
   sW[threadIdx.x] = Ws{a.ws + ((slot / LANES) * SW::NFIELDS) * LANES + lane, nwarps * SW::NFIELDS * LANES, tile0};
-  const Ws& W = sW[threadIdx.x];
-  IpmState S;
-  bool active = false;        // this lane holds an unfinished problem
-  bool pending = false;       // this lane holds a finished problem whose results are not written yet
-  bool exhausted = false;     // the queue is empty (warp-uniform)
-  bool first = true;
-  long b = -1;
-  const int warps_per_block = kBlock / 32;
-  unsigned round = 0;
-  while (true) {
-    // ---- a warp whose 32 problems are all finished claims the next 32 (warp-uniform branch) ----
-    const bool chunk_done = !__any_sync(0xffffffffu, active);
-    // ---- a finished chunk writes its results with all 32 lanes together: every row of the
-    //      [variable][node][problem] output is then one coalesced 256-byte store per warp (the output
-    //      may be pinned host memory written over PCIe while the other warps keep computing) ----
-    if (chunk_done && __any_sync(0xffffffffu, pending)) {
-      if (pending) write_results<SW, 1>(a.res, P, M, O.obj_scale, a.model, W, 0, 1u << lane, S, b);
-      pending = false;
-    }
-    if (!exhausted && chunk_done) {
-      // first chunk: static round-robin over CTAs (spreads a small batch over all SMs);
-      // afterwards: the device-wide queue
-      int chunk = 0;
-      if (first) {
-        chunk = (threadIdx.x / 32) * gridDim.x + blockIdx.x;
-        first = false;
-      } else {
-        if (lane == 0) chunk = atomicAdd(a.counter, 1) + gridDim.x * warps_per_block;
-        chunk = __shfl_sync(0xffffffffu, chunk, 0);
-      }
-      if ((long)chunk * 32 >= a.res.B) {
-        exhausted = true;
-      } else {
-        b = (long)chunk * 32 + lane;
-        if (b < a.res.B) {
-          P = derive_params(a.params, a.res.B, b, a.model);
-          // ref_mode 2: start from the batch reference.  ref_mode 1 (the reference solve itself):
-          // start from the previous call's reference if the handle has one (consecutive batches of a
-          // campaign have nearly the same mean, so it re-converges in one or two iterations).
-          ipm_start<SW>(P, M, O, W, GuessSrc{a.guess_traj, a.guess_tf, a.res.B, b}, a.ref_mode != 0 ? a.ref : nullptr, S);
-          active = true;
-        }
-      }
-    }
-    // ---- all eight warps of the SM start each iteration together: they then run the same sweep
-    //      (same code) at the same time, which keeps the 32 KB instruction cache effective ----
-    // (every LMATO_SYNC_PERIOD-th round: a barrier per iteration costs more in waiting than it
-    //  gains, because line-search retries differ between warps; the imbalance averages out over
-    //  a few iterations while the warps stay close enough to share the instruction cache)
-    if ((round++ % LMATO_SYNC_PERIOD) == 0 && !__syncthreads_or((active || !exhausted) ? 1 : 0)) break;
-    if (active && ipm_iterate_t<SW>(P, M, O, W, S)) {
-      if (ipm_restart<SW>(P, M, O, W, S)) continue;      // this lane restarts the same problem
-      active = false;
-      pending = true;      // results are written when the whole chunk is done (see above)
-      // (the reference solve of the batch warm start, ref_mode 1, runs on the cooperative kernel)
-    }
-  }
+  // (the reference solve of the batch warm start, ref_mode 1, runs on the cooperative kernel)
+  solve_queue<SW, kBlockBarrier>(a, sP[threadIdx.x].p, sM, sO, sW[threadIdx.x], 0, 1u << lane);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -192,12 +228,9 @@ constexpr int kCoopBlock = 256;
 constexpr int kCoopBlocksPerSM = 2;
 constexpr int kCoopG = 8;
 constexpr int kCoopScrStride = coop::SCR_DOUBLES;       // per group: record ring + transpose tiles (even: 16-byte aligned)
+static_assert(kCoopBlock == kBlock, "solve_queue counts kBlock / 32 warps in every CTA");
 static size_t coop_smem(int gp) { return sizeof(double) * (size_t)(kCoopBlock / gp) * kCoopScrStride; }
 
-// A warp holds 32/GP problems; its groups run the IPM driver in lock step (same sweep at the same time, each
-// with its own lane mask), finished groups idle until the warp's chunk is done, then the warp claims the next
-// chunk from the device-wide queue.  IpmState (filter, barrier parameter, ...) is carried redundantly by the
-// GP lanes of a group: every decision of the driver is a function of group-uniform values.
 //   GP = 8 : four problems per warp, for batches that can fill the GPU that way;
 //   GP = 32: the whole warp works on one problem (the stage-parallel phases are four times shorter), for
 //            the latency regime: up to a few problems per SM.
@@ -205,7 +238,6 @@ static size_t coop_smem(int gp) { return sizeof(double) * (size_t)(kCoopBlock / 
 template <int G, int GP, int MOVE, int BPS>      // MOVE: 0 no move term, 1 move term (LO:99), 2 the circular model's (MV = angle)
 __global__ void __launch_bounds__(kCoopBlock, BPS) ascent_coop_kernel(KArgs a) {
   using SW = SweepsCoop<G, GP, MOVE>;
-  constexpr int PPW = 32 / GP;                 // problems per warp
   constexpr int GPB = kCoopBlock / GP;         // groups per block
   __shared__ ParamsSlot sP[GPB];
   __shared__ Options sO;
@@ -213,65 +245,17 @@ __global__ void __launch_bounds__(kCoopBlock, BPS) ascent_coop_kernel(KArgs a) {
   extern __shared__ __align__(16) double sScr[];    // [GPB][kCoopScrStride]
   if (threadIdx.x == 0) { sO = a.O; sM = Mesh{a.N, a.h, a.tau}; }
   __syncthreads();
-  const Options& O = sO;
-  const Mesh& M = sM;
   const int lane = threadIdx.x & 31;
   const int grp = threadIdx.x / GP;
   const unsigned gmask = GP == 32 ? 0xffffffffu : (((1u << GP) - 1u) << ((lane / GP) * GP));
   const unsigned smask = ((1u << G) - 1u) << ((lane / GP) * GP);
-  Params& P = sP[grp].p;
   const long slot = (long)blockIdx.x * GPB + grp;
   // workspace layout by regime (ascent_coop.cuh, CwsT): stage-major blocks when a whole warp walks one problem
   const coop::CwsT<(GP == 32)> W{a.ws + slot * coop::coop_doubles_per_problem(a.N + 1), a.N + 1, sScr + grp * kCoopScrStride,
                                  lane % GP, gmask, smask, 0.0, 0.0, 0, 0u};
   if (W.g == 0) coop::ring_init_barriers(W.bars());      // the mbarriers of this group's record ring
   __syncthreads();
-  IpmState S;
-  bool active = false, pending = false, exhausted = false, first = true;
-  long b = -1;
-  const int warps_per_block = kCoopBlock / 32;
-  while (true) {
-    const bool chunk_done = !__any_sync(0xffffffffu, active);
-    if (chunk_done && __any_sync(0xffffffffu, pending)) {
-      if (pending) write_results<SW, GP>(a.res, P, M, O.obj_scale, a.model, W, W.g, W.mask, S, b);
-      pending = false;
-    }
-    if (!exhausted && chunk_done) {
-      int chunk = 0;
-      if (first) {
-        chunk = (threadIdx.x / 32) * gridDim.x + blockIdx.x;     // static round-robin: spreads a small batch over all SMs
-        first = false;
-      } else {
-        if (lane == 0) chunk = atomicAdd(a.counter, 1) + gridDim.x * warps_per_block;
-        chunk = __shfl_sync(0xffffffffu, chunk, 0);
-      }
-      if ((long)chunk * PPW >= a.res.B) {
-        exhausted = true;
-      } else {
-        b = (long)chunk * PPW + lane / GP;
-        if (b < a.res.B) {
-          if (W.g == 0) P = derive_params(a.params, a.res.B, b, a.model, MOVE == 2);
-          coop::Grp<GP>::sync(gmask);
-          ipm_start<SW>(P, M, O, W, GuessSrc{a.guess_traj, a.guess_tf, a.res.B, b}, a.ref_mode != 0 ? a.ref : nullptr, S);
-          active = true;
-        }
-      }
-    }
-    // (no block barrier per iteration here: the warps of an SM are few and their sweeps are short; a warp that
-    //  waits for its neighbours' line-search retries loses more than the instruction cache gains)
-    if (exhausted && !__any_sync(0xffffffffu, active || pending)) break;
-    if (active && ipm_iterate_t<SW>(P, M, O, W, S)) {
-      if (ipm_restart<SW>(P, M, O, W, S)) continue;
-      active = false;
-      if (a.ref_mode == 1) {
-        SolveOut out;
-        ipm_result(S, out);
-        SW::store_ref(P, M, W, out.cur, S.cur, S.ctl.mu, out.status == ST_CONVERGED, a.ref);
-        continue;
-      }
-      pending = true;
-    }
-  }
+  solve_queue<SW, kWarpVote>(a, sP[grp].p, sM, sO, W, W.g, W.mask);
 }
 
 template <int GP, int BPS>
@@ -294,8 +278,6 @@ static cudaError_t coop_optin() {
 // ---------------------------------------------------------------------------------------
 template <int GP>
 __global__ void __launch_bounds__(kCoopBlock, 1) ascent_colloc_kernel(KArgs a) {
-  using SW = SweepsColloc<GP>;
-  constexpr int PPW = 32 / GP;
   constexpr int GPB = kCoopBlock / GP;
   __shared__ ParamsSlot sP[GPB];
   __shared__ Options sO;
@@ -303,65 +285,15 @@ __global__ void __launch_bounds__(kCoopBlock, 1) ascent_colloc_kernel(KArgs a) {
   __shared__ colloc::Coll sC;
   if (threadIdx.x == 0) { sO = a.O; sM = Mesh{a.N, a.h, a.tau}; sC = *a.coll; }
   __syncthreads();
-  const Options& O = sO;
-  const Mesh& M = sM;
   const int lane = threadIdx.x & 31;
   const int grp = threadIdx.x / GP;
   const unsigned gmask = GP == 32 ? 0xffffffffu : (((1u << GP) - 1u) << ((lane / GP) * GP));
-  Params& P = sP[grp].p;
   const long slot = (long)blockIdx.x * GPB + grp;
   colloc::Nws W;
   W.L.init(sC.m);
   W.base = a.ws + slot * colloc::colloc_doubles_per_problem(a.N + 1, sC.m);
   W.N1 = a.N + 1; W.C = &sC; W.g = lane % GP; W.mask = gmask; W.dw = 0.0; W.pimax = 0.0; W.ls_flag = 0;
-  IpmState S;
-  int variant = 0;
-  bool active = false, pending = false, exhausted = false, first = true;
-  long b = -1;
-  const int warps_per_block = kCoopBlock / 32;
-  while (true) {
-    const bool chunk_done = !__any_sync(0xffffffffu, active);
-    if (chunk_done && __any_sync(0xffffffffu, pending)) {
-      if (pending) write_results<SW, GP>(a.res, P, M, O.obj_scale, a.model, W, W.g, W.mask, S, b);
-      pending = false;
-    }
-    if (!exhausted && chunk_done) {
-      int chunk = 0;
-      if (first) {
-        chunk = (threadIdx.x / 32) * gridDim.x + blockIdx.x;
-        first = false;
-      } else {
-        if (lane == 0) chunk = atomicAdd(a.counter, 1) + gridDim.x * warps_per_block;
-        chunk = __shfl_sync(0xffffffffu, chunk, 0);
-      }
-      if ((long)chunk * PPW >= a.res.B) {
-        exhausted = true;
-      } else {
-        b = (long)chunk * PPW + lane / GP;
-        if (b < a.res.B) {
-          if (W.g == 0) P = derive_params(a.params, a.res.B, b, a.model);
-          coop::Grp<GP>::sync(gmask);
-          ipm_begin(O, S);
-          variant = 0;
-          SW::guess_variant(P, M, O, W, S.cur, variant);
-          active = true;
-        }
-      }
-    }
-    if (exhausted && !__any_sync(0xffffffffu, active || pending)) break;
-    if (active && ipm_iterate_t<SW>(P, M, O, W, S)) {
-      if (S.ctl.status != ST_CONVERGED && S.ctl.status != ST_MAX_ITER && variant + 1 < (int)SW::N_STARTS) {
-        // no restoration phase: a problem that fails from one start point is restarted from the next
-        const int it_used = S.ctl.iter;
-        ipm_begin(O, S);
-        S.ctl.iter = it_used; S.ctl.iter_best = it_used;      // MAX_ITER (LO:28) bounds the whole ladder
-        SW::guess_variant(P, M, O, W, S.cur, ++variant);
-        continue;
-      }
-      active = false;
-      pending = true;
-    }
-  }
+  solve_queue<SweepsColloc<GP>, kWarpVote>(a, sP[grp].p, sM, sO, W, W.g, W.mask);
 }
 
 // FP64 FMA peak: 8 independent chains per thread, no memory traffic.

@@ -698,6 +698,7 @@ LM_NOINLINE void colloc_init_guess(const Params& P, const Mesh& M, const Options
 // Sweeps policy of the higher-order collocation path for the IPM driver (ipm_iterate_t).
 template <int GP>
 struct SweepsColloc {
+  enum : int { LANES_PER_PROBLEM = GP, MOVE_TERM = 0, STORES_REF = 0 };
   LM_HD static int n_eq(const colloc::Nws& W, int N) { return 6 * W.L.m * N + 3; }
   LM_HD static int n_bd(const colloc::Nws& W, int N) { return (2 * W.L.m + 2) * N + 4; }
   LM_HD static bool backward(const Params& P, const Mesh& M, const Options& O, const colloc::Nws& W, int src, const Scal& c0,
@@ -715,10 +716,7 @@ struct SweepsColloc {
     colloc::colloc_eval<GP>(P, M, O, *W.C, W, src, dst, c0, ts, mu, alpha, alpha_z, alpha_lam, t);
     if (pimax) *pimax = W.pimax;
   }
-  LM_HD static void guess(const Params& P, const Mesh& M, const Options& O, const colloc::Nws& W, Scal& s) {
-    colloc::colloc_init_guess<GP>(P, M, O, *W.C, W, s, 0);
-  }
-  // further start points for a problem that failed from the first (this solver has no restoration phase)
+  // the start points of the ladder, tried in turn by ipm_start / ipm_restart below (this solver has no restoration phase)
   enum : int { N_STARTS = 4 };
   LM_HD static void guess_variant(const Params& P, const Mesh& M, const Options& O, const colloc::Nws& W, Scal& s, int variant) {
     colloc::colloc_init_guess<GP>(P, M, O, *W.C, W, s, variant);
@@ -735,5 +733,29 @@ struct SweepsColloc {
   }
   LM_HD static void remerit(const Mesh&, const Options&, const colloc::Nws&, int, double, Scal&) {}
 };
+
+// Start of one problem on the collocation workspace: the first rung of the start ladder (colloc_init_guess).  The
+// caller's start point and the batch reference are not read: the C ABI rejects a start point for NODES >= 3 and never
+// sets a reference for them.
+template <class SW>
+LM_HD void ipm_start(const Params& P, const Mesh& M, const Options& O, const colloc::Nws& W, const GuessSrc&, const double*,
+                     IpmState& S) {
+  ipm_begin(O, S);
+  S.start = 0;
+  SW::guess_variant(P, M, O, W, S.cur, 0);
+}
+
+// A problem that failed from one rung of the ladder is restarted from the next, unless it stopped at MAX_ITER or no
+// rung is left.  The iteration count carries on, so that MAX_ITER (LO:28) bounds the whole ladder and the reported
+// iterations include the abandoned starts.  Returns true if it restarted.
+template <class SW>
+LM_HD bool ipm_restart(const Params& P, const Mesh& M, const Options& O, const colloc::Nws& W, IpmState& S) {
+  if (S.ctl.status == ST_CONVERGED || S.ctl.status == ST_MAX_ITER || S.start + 1 >= (int)SW::N_STARTS) return false;
+  const int it_used = S.ctl.iter;
+  ipm_begin(O, S);
+  S.ctl.iter = it_used; S.ctl.iter_best = it_used;
+  SW::guess_variant(P, M, O, W, S.cur, ++S.start);
+  return true;
+}
 
 }  // namespace lmato

@@ -1133,7 +1133,7 @@ LM_NOINLINE void coop_store_ref(const Params& P, const Mesh& M, const CW& W, int
 //   GP lanes (a multiple of G, at most a warp) carry the stage-parallel phases of the same problem.
 template <int G, int GP, int MOVE, bool VREC = (GP > G)>
 struct SweepsCoop {
-  enum : int { LANES_PER_PROBLEM = GP, MOVE_TERM = MOVE };
+  enum : int { LANES_PER_PROBLEM = GP, MOVE_TERM = MOVE, STORES_REF = 1 };    // STORES_REF: has store_ref
   template <class CW>
   LM_HD static int n_eq(const CW&, int N) { return (MOVE ? 7 : 6) * N + 3; }
   template <class CW>

@@ -1318,6 +1318,8 @@ enum : int { PH_LSQ = 0, PH_NEWTON = 1 };
 struct IpmState {
   bool warm;        // start point carries its own multipliers (skip the least-squares estimate)
   bool from_guess;  // start point supplied by the caller (lmato_set_initial_guess)
+  unsigned char start;   // rung of the collocation start ladder (ascent_colloc.cuh), set by its ipm_start only; one
+                         // byte, so that it fills padding and IpmState keeps its size on every other kernel's stack
   int iters_prior;  // iterations of an abandoned warm / caller-supplied start of the same problem (reported with the rest)
   Scal cur;
   Ctl ctl;
@@ -1400,7 +1402,7 @@ LM_HD void ws_node(const Ws& W, int cur, int k, double* x, double* lam) {
 // Sweeps policy of the 7-state formulation (dcost = 0); ascent_ipm_dc.cuh provides the 8-state one.
 struct Sweeps7 {
   enum : int { NFIELDS = N_FIELDS, NITER = N_ITER, FZ = F_Z, FU = F_U, FLAM = F_LAM, REFROWS = REF_ROWS, MOVE_TERM = 0,
-               LANES_PER_PROBLEM = 1 };
+               LANES_PER_PROBLEM = 1, STORES_REF = 0 };
   LM_HD static int n_eq(const Ws&, int N) { return 6 * N + 3; }
   LM_HD static int n_bd(const Ws&, int N) { return 4 * N + 4; }
   LM_HD static bool backward(const Params& P, const Mesh& M, const Options& O, const Ws& W, int src, const Scal& c0,

@@ -739,7 +739,7 @@ LM_SWEEP void riccati_forward(const Params& P, const Mesh& M, const Options& O, 
 // Sweeps policy of the 8-state (DCOST) formulation.
 struct Sweeps8 {
   enum : int { NFIELDS = dc::N_FIELDS, NITER = dc::N_ITER, FZ = dc::F_Z, FU = dc::F_U, FLAM = dc::F_LAM, REFROWS = dc::REF_ROWS,
-               MOVE_TERM = 1, LANES_PER_PROBLEM = 1 };
+               MOVE_TERM = 1, LANES_PER_PROBLEM = 1, STORES_REF = 0 };
   LM_HD static int n_eq(const Ws&, int N) { return 7 * N + 3; }
   LM_HD static int n_bd(const Ws&, int N) { return 6 * N + 4; }
   LM_HD static bool backward(const Params& P, const Mesh& M, const Options& O, const Ws& W, int src, const Scal& c0,

@@ -2,8 +2,9 @@
 
 `csrc/ascent_model.cuh`, `ascent_ipm.cuh`, `ascent_ipm_dc.cuh`, `ascent_coop.cuh`, `ascent_colloc.cuh` and
 `ascent_result.cuh` are written so that g++ accepts them (tools/hostsim): the parameter derivation, the sweeps, the
-IPM driver, the model derivatives and the result writer below are the very lines the CUDA kernels run, executed by
-one CPU thread.  This gives the CPU-only test tier a check of the solver's logic against the oracle's golden vectors,
+IPM driver with its start and restart steps (`ipm_start` / `ipm_restart`, the collocation start ladder included),
+the model derivatives and the result writer below are the very lines the CUDA kernels run, executed by one CPU
+thread.  Only the kernels' problem queue (`solve_queue`) is not run here.  This gives the CPU-only test tier a check of the solver's logic against the oracle's golden vectors,
 and of the hand-derived derivatives and the sensitivity output against finite differences.  It is test
 infrastructure only: the product has no CPU path (`_cabi.lib()` raises without
 the CUDA library), and nothing here is imported by the package.
@@ -214,6 +215,26 @@ def test_higher_order_collocation_source_matches_goldens(hostsim):
         st, tf, it, traj = solve(g["rows"][:, b], int(g["disp_nt"]), 3)
         assert st == 0 and abs(tf - g["disp_tf"][b]) / tf < 1e-9
         assert _rel(traj, g["disp_traj"][b])[:9].max() < 1e-5
+
+
+def test_collocation_start_ladder_counts_every_start(hostsim, monkeypatch):
+    """The collocation start ladder (ascent_colloc.cuh: ipm_start / ipm_restart) as the kernel runs it.  From a burn
+    time guess of 0.1 the nominal problem at NODES = 3, nt = 60 fails from every start without reaching MAX_ITER, so
+    the ladder runs to its last start; the first start alone takes 31 iterations before its line search fails, and
+    the reported count covers all starts, not only the last."""
+    from oracle.ascent_nlp import collocation_matrix
+    monkeypatch.delenv("NPOL", raising=False)
+    monkeypatch.setenv("TF0", "0.1")
+    nt, nodes = 60, 3
+    t_or, N_or = collocation_matrix(nodes)
+    tau, Nc = np.ascontiguousarray(t_or[1:], dtype=np.float64), np.ascontiguousarray(N_or, dtype=np.float64)
+    traj = np.empty((10, nt)); tf, it, kkt = C.c_double(), C.c_int(), C.c_double()
+    st = hostsim.hostsim_solve_colloc(NOMINAL.ctypes.data_as(C.c_void_p), nt, None, nodes, Nc.ctypes.data_as(C.c_void_p),
+                                      tau.ctypes.data_as(C.c_void_p), C.c_double(1e-10), C.c_double(10.0),
+                                      C.c_double(1e-3), traj.ctypes.data_as(C.c_void_p), C.byref(tf), C.byref(it),
+                                      C.byref(kkt))
+    assert st not in (0, 1), (st, it.value)          # neither converged nor stopped at MAX_ITER: the ladder ran out
+    assert it.value >= 31, it.value
 
 
 def test_start_points_on_every_layout(hostsim, monkeypatch):

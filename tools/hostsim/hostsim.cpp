@@ -226,7 +226,8 @@ extern "C" int hostsim_solve_coop(const double* raw14, int nt, const double* tim
   return status;
 }
 
-// Higher-order collocation (csrc/ascent_colloc.cuh), GP = 1.  Ncol: row-major m x m, tauc: m points.
+// Higher-order collocation (csrc/ascent_colloc.cuh), GP = 1, with the kernel's start ladder.  Ncol: row-major m x m,
+// tauc: m points.  TF0 sets tf_guess.
 extern "C" int hostsim_solve_colloc(const double* raw14, int nt, const double* time, int nodes, const double* Ncol,
                                     const double* tauc, double tol, double obj_scale, double mu_min_factor,
                                     double* traj /* [10][nt] */, double* tf_out, int* iters, double* kkt) {
@@ -234,7 +235,8 @@ extern "C" int hostsim_solve_colloc(const double* raw14, int nt, const double* t
   std::vector<double> h(N + 1), tau(N + 1);
   for (int k = 0; k <= N; ++k) { tau[k] = time ? time[k] : (double)k / N; h[k] = k ? tau[k] - tau[k - 1] : 0.0; }
   Mesh M{N, h.data(), tau.data()};
-  const Options O = make_options(tol, obj_scale, mu_min_factor, getenv("NPOL") ? atoi(getenv("NPOL")) : 4, 0.0);
+  Options O = make_options(tol, obj_scale, mu_min_factor, getenv("NPOL") ? atoi(getenv("NPOL")) : 4, 0.0);
+  if (getenv("TF0")) O.tf_guess = atof(getenv("TF0"));
   const Params P = derive_params(raw14, 1, 0, LMATO_MODEL_ELLIPTICAL);   // NODES >= 3: the elliptical model only
   colloc::Coll C;
   C.m = m;
@@ -242,19 +244,10 @@ extern "C" int hostsim_solve_colloc(const double* raw14, int nt, const double* t
   std::vector<double> ws((size_t)colloc::colloc_doubles_per_problem(nt, m), 0.0);
   colloc::Nws W;
   W.base = ws.data(); W.N1 = nt; W.L.init(m); W.C = &C; W.g = 0; W.mask = 1u; W.dw = 0.0; W.pimax = 0.0; W.ls_flag = 0;
-  IpmState S;
-  const int v0 = getenv("VARIANT") ? atoi(getenv("VARIANT")) : 0;
-  const int nv = getenv("VARIANT") ? v0 + 1 : (int)SweepsColloc<1>::N_STARTS;
-  for (int variant = v0; variant < nv; ++variant) {        // the kernel's restart ladder
-    ipm_begin(O, S);
-    SweepsColloc<1>::guess_variant(P, M, O, W, S.cur, variant);
-    while (!ipm_iterate_t<SweepsColloc<1>>(P, M, O, W, S)) {}
-    if (S.ctl.status == ST_CONVERGED) break;
-  }
   int status;
   double fmass;
   const ResultOut R{traj, tf_out, &fmass, &status, iters, kkt, nullptr, 1};
-  write_results<SweepsColloc<1>, 1>(R, P, M, O.obj_scale, LMATO_MODEL_ELLIPTICAL, W, 0, 1u, S, 0);
+  solve_one<SweepsColloc<1>>(R, P, M, O, LMATO_MODEL_ELLIPTICAL, W);
   return status;
 }
 
