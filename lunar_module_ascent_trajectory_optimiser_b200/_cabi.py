@@ -68,7 +68,7 @@ def build_library(force: bool = False, verbose: bool = False) -> str:
     every source; ``LAST_BUILD`` says which)."""
     import time as _time
     srcs = [os.path.join(CSRC, f) for f in ("ascent_cabi.cu", "ascent_ipm.cuh", "ascent_ipm_dc.cuh", "ascent_coop.cuh", "ascent_colloc.cuh",
-                                            "ascent_model.cuh", "ascent_result.cuh")]
+                                            "ascent_model.cuh", "ascent_result.cuh", "ascent_plan.h")]
     srcs.append(os.path.join(INCLUDE, "lmato_b200.h"))
     if not force and os.path.exists(LIB_PATH):
         if all(os.path.getmtime(LIB_PATH) >= os.path.getmtime(s) for s in srcs):

@@ -25,6 +25,7 @@
 
 #include "../../include/lmato_b200.h"
 #include "ascent_colloc.cuh"
+#include "ascent_plan.h"
 #include "ascent_result.cuh"
 
 using namespace lmato;
@@ -46,19 +47,11 @@ void set_err(const char* fmt, const char* a = "", const char* b = "") {
     }                                                                         \
   } while (0)
 
-// One CTA of 256 threads (8 warps) per SM: 255 registers x 256 threads fills the register file.
 #ifndef LMATO_SYNC_PERIOD
 #define LMATO_SYNC_PERIOD 1
 #endif
-constexpr int kBlock = 256;
-constexpr int kBlocksPerSM = 1;
 // dynamic shared memory: the staging tiles, then one workspace view per thread
 constexpr size_t kTileSmem = (size_t)(kBlock / 32) * 2 * TILE_ROWS * LANES * sizeof(double) + kBlock * sizeof(Ws);
-// Batch warm start: one reference solve of the batch-mean problem (cooperative kernel, one group) against ~6 saved
-// iterations per problem.  Measured with the reference solve on the cooperative kernel (1.8 ms on the first call of a
-// handle, 0.2 ms afterwards): 512 problems 7.2 ms cold, 7.3 ms warm on the first call, 5.5 ms on later calls; from
-// 1 024 problems up the first call wins as well (tools/gpu_warm_threshold.py).
-constexpr long kWarmStartMinBatch = 512;
 
 struct KArgs {
   const double* params;  // [NPARAM][B]
@@ -224,12 +217,9 @@ __global__ void __launch_bounds__(kBlock, kBlocksPerSM) ascent_ipm_kernel(KArgs 
 // ---------------------------------------------------------------------------------------
 // cooperative kernel: G lanes per problem (ascent_coop.cuh)
 // ---------------------------------------------------------------------------------------
-constexpr int kCoopBlock = 256;
-constexpr int kCoopBlocksPerSM = 2;
-constexpr int kCoopG = 8;
 constexpr int kCoopScrStride = coop::SCR_DOUBLES;       // per group: record ring + transpose tiles (even: 16-byte aligned)
 static_assert(kCoopBlock == kBlock, "solve_queue counts kBlock / 32 warps in every CTA");
-static size_t coop_smem(int gp) { return sizeof(double) * (size_t)(kCoopBlock / gp) * kCoopScrStride; }
+constexpr size_t coop_smem(int gp) { return sizeof(double) * (size_t)(kCoopBlock / gp) * kCoopScrStride; }
 
 //   GP = 8 : four problems per warp, for batches that can fill the GPU that way;
 //   GP = 32: the whole warp works on one problem (the stage-parallel phases are four times shorter), for
@@ -258,21 +248,6 @@ __global__ void __launch_bounds__(kCoopBlock, BPS) ascent_coop_kernel(KArgs a) {
   solve_queue<SW, kWarpVote>(a, sP[grp].p, sM, sO, W, W.g, W.mask);
 }
 
-template <int GP, int BPS>
-static void coop_launch(int move, long grid, cudaStream_t st, const KArgs& a) {
-  if (move == 2) ascent_coop_kernel<kCoopG, GP, 2, BPS><<<(int)grid, kCoopBlock, coop_smem(GP), st>>>(a);
-  else if (move == 1) ascent_coop_kernel<kCoopG, GP, 1, BPS><<<(int)grid, kCoopBlock, coop_smem(GP), st>>>(a);
-  else ascent_coop_kernel<kCoopG, GP, 0, BPS><<<(int)grid, kCoopBlock, coop_smem(GP), st>>>(a);
-}
-template <int GP, int BPS>
-static cudaError_t coop_optin() {
-  cudaError_t e = cudaFuncSetAttribute(ascent_coop_kernel<kCoopG, GP, 2, BPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coop_smem(GP));
-  if (e != cudaSuccess) return e;
-  e = cudaFuncSetAttribute(ascent_coop_kernel<kCoopG, GP, 1, BPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coop_smem(GP));
-  if (e != cudaSuccess) return e;
-  return cudaFuncSetAttribute(ascent_coop_kernel<kCoopG, GP, 0, BPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coop_smem(GP));
-}
-
 // ---------------------------------------------------------------------------------------
 // higher-order collocation kernel (NODES = 3..6, ascent_colloc.cuh): GP lanes per problem
 // ---------------------------------------------------------------------------------------
@@ -294,6 +269,52 @@ __global__ void __launch_bounds__(kCoopBlock, 1) ascent_colloc_kernel(KArgs a) {
   W.base = a.ws + slot * colloc::colloc_doubles_per_problem(a.N + 1, sC.m);
   W.N1 = a.N + 1; W.C = &sC; W.g = lane % GP; W.mask = gmask; W.dw = 0.0; W.pimax = 0.0; W.ls_flag = 0;
   solve_queue<SweepsColloc<GP>, kWarpVote>(a, sP[grp].p, sM, sO, W, W.g, W.mask);
+}
+
+// Every solve-kernel instantiation a launch plan (ascent_plan.h) can name, with its launch shape.  The thread kernel's
+// staging tiles and the cooperative kernel's record rings need the opt-in shared-memory size (thread kernel: 158 KB
+// dynamic + 42 KB static per CTA).
+struct SolveKernel {
+  KernelKey key;
+  void (*fn)(KArgs);
+  int block;
+  size_t smem;         // dynamic shared memory
+};
+#define COOP_KERNEL(GP, MOVE, BPS) {{kCoopKernel, GP, BPS, MOVE}, ascent_coop_kernel<kCoopG, GP, MOVE, BPS>, kCoopBlock, coop_smem(GP)}
+const SolveKernel kSolveKernels[] = {
+  {{kThreadKernel, 1, kBlocksPerSM, 0}, ascent_ipm_kernel<Sweeps7>, kBlock, kTileSmem},
+  {{kThreadKernel, 1, kBlocksPerSM, 1}, ascent_ipm_kernel<Sweeps8>, kBlock, kTileSmem},
+  COOP_KERNEL(8, 0, 1), COOP_KERNEL(8, 1, 1), COOP_KERNEL(8, 2, 1),
+  COOP_KERNEL(8, 0, 2), COOP_KERNEL(8, 1, 2), COOP_KERNEL(8, 2, 2),
+  COOP_KERNEL(32, 0, 1), COOP_KERNEL(32, 1, 1), COOP_KERNEL(32, 2, 1),
+  COOP_KERNEL(32, 0, 2), COOP_KERNEL(32, 1, 2), COOP_KERNEL(32, 2, 2),
+  {{kCollocKernel, 8, 1, 0}, ascent_colloc_kernel<8>, kCoopBlock, 0},
+  {{kCollocKernel, 32, 1, 0}, ascent_colloc_kernel<32>, kCoopBlock, 0},
+};
+#undef COOP_KERNEL
+
+// Launches the table's kernel for `key` on `grid` CTAs.
+lmato_status_t launch(const KernelKey& key, long grid, cudaStream_t st, const KArgs& a) {
+  for (const SolveKernel& k : kSolveKernels)
+    if (k.key == key) {
+      k.fn<<<(int)grid, k.block, k.smem, st>>>(a);
+      CUDA_TRY(cudaGetLastError());
+      return LMATO_OK;
+    }
+  set_err("lmato_solve_batch: no solve kernel is instantiated for the launch plan");
+  return LMATO_ERR_INVALID;
+}
+
+// Makes *p hold at least `bytes` bytes of device memory, freeing and reallocating it when it is smaller.  A caller
+// whose old buffer may still be in use on the device waits for that before it asks for more.
+cudaError_t grow(double** p, size_t* cap, size_t bytes) {
+  if (bytes <= *cap) return cudaSuccess;
+  const cudaError_t e = cudaFree(*p);
+  *p = nullptr; *cap = 0;
+  if (e != cudaSuccess) return e;
+  const cudaError_t m = cudaMalloc(p, bytes);
+  if (m == cudaSuccess) *cap = bytes;
+  return m;
 }
 
 // FP64 FMA peak: 8 independent chains per thread, no memory traffic.
@@ -363,7 +384,6 @@ struct lmato_handle {
   double* d_tau = nullptr;
   double* d_ws = nullptr;
   size_t ws_bytes = 0;
-  long ws_slots = 0;
   int* d_counter = nullptr;
   // staging for the host-buffer entry point
   double* d_params = nullptr; size_t params_bytes = 0;
@@ -379,7 +399,6 @@ struct lmato_handle {
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   cudaStream_t last_stream = nullptr;
   bool timed = false;
-  bool last_coop = false;         // which kernel the last solve used
   colloc::Coll coll;              // collocation rule for NODES >= 3 ...
   colloc::Coll* d_coll = nullptr; // ... and its device copy
 };
@@ -432,13 +451,8 @@ static lmato_status_t create_device_state(lmato_handle* H, const std::vector<dou
   cudaDeviceProp prop;
   CUDA_TRY(cudaGetDeviceProperties(&prop, H->device));
   H->sm_count = prop.multiProcessorCount;
-  // the staging tiles need the opt-in shared-memory size (158 KB dynamic + 42 KB static per CTA)
-  CUDA_TRY(cudaFuncSetAttribute(ascent_ipm_kernel<Sweeps7>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTileSmem));
-  CUDA_TRY(cudaFuncSetAttribute(ascent_ipm_kernel<Sweeps8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTileSmem));
-  CUDA_TRY((coop_optin<8, 1>()));
-  CUDA_TRY((coop_optin<8, 2>()));
-  CUDA_TRY((coop_optin<32, 1>()));
-  CUDA_TRY((coop_optin<32, 2>()));
+  for (const SolveKernel& k : kSolveKernels)
+    if (k.smem > 0) CUDA_TRY(cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.smem));
   CUDA_TRY(cudaMalloc(&H->d_h, sizeof(double) * nt));
   CUDA_TRY(cudaMalloc(&H->d_tau, sizeof(double) * nt));
   CUDA_TRY(cudaMemcpy(H->d_h, h.data(), sizeof(double) * nt, cudaMemcpyHostToDevice));
@@ -460,25 +474,7 @@ const char* lmato_last_error(void) { return g_err; }
 const char* lmato_version(void) { return "lmato_b200 0.1 (sm_100a)"; }
 
 void lmato_default_options(lmato_options* o) {
-  if (!o) return;
-  o->tol = 1e-10;
-  o->mu_init = 0.1;
-  o->obj_scale = 10.0;
-  o->tf_guess = 0.9;
-  o->delta_c = 1e-8;
-  o->mu_min_factor = 1e-3;
-  o->n_polish = -1;           // automatic: 2 with the DCOST term, 4 without (DESIGN.md "Tolerance")
-  o->warm_start = 1;
-  o->mu_ref = 1e-3;
-  o->dcost = 1e-5;            // LO:99
-  o->kappa_eps = 30.0;
-  o->objective_nodes = 0;     // 0 = nt - 1
-  o->kernel = LMATO_KERNEL_AUTO;
-  o->coop_lanes = 0;
-  o->otol = 1e-3;             // LO:31
-  o->rtol = 1e-3;             // LO:32
-  o->max_iter = 20000;   // LO:28
-  o->max_ls = 40;
+  if (o) *o = default_options();
 }
 
 lmato_status_t lmato_create(lmato_handle** out, int32_t device, int32_t nt, const double* time,
@@ -549,68 +545,9 @@ lmato_status_t lmato_set_options(lmato_handle* h, const lmato_options* o) {
   return LMATO_OK;
 }
 
-// The move-suppression term: DCOST on the MV angledoubledot of the elliptical model (LO:99), on the MV angle of the
-// circular model (PDF p.27 src 69-73).  The circular model with the term is carried by the cooperative kernel only.
-static bool dcost_active(const lmato_handle* h) { return h->opt.dcost > 0.0; }
-static bool circular_move(const lmato_handle* h) { return h->model == LMATO_MODEL_CIRCULAR && dcost_active(h); }
-
-// Which kernel solves a batch of B problems.  One thread per problem needs ~1 wave (SMs x 256 problems) to fill
-// the GPU and streams the least HBM traffic per problem; eight lanes per problem fill it with an eighth of that
-// and shorten the critical path of every problem, at ~2.5x the traffic.  Measured cross-over on B200 at nt = 200:
-// between 16 384 and 32 768 problems (profiles/README.md).
-constexpr int64_t kCoopMaxBatch = 6144;
-static bool use_coop(const lmato_handle* h, int64_t B) {
-  if (circular_move(h)) return true;
-  if (h->opt.kernel == LMATO_KERNEL_COOP) return true;
-  if (h->opt.kernel == LMATO_KERNEL_THREAD) return false;
-  return B <= kCoopMaxBatch;
-}
-static int fields_for(const lmato_handle* h) { return dcost_active(h) ? (int)dc::N_FIELDS : (int)N_FIELDS; }
-
-static long slots_for(const lmato_handle* h, int64_t B) {
-  // one CTA per SM, but never more CTAs than 32-problem chunks
-  const long chunks = (B + 31) / 32;
-  const long grid = chunks < (long)h->sm_count * kBlocksPerSM ? (chunks > 0 ? chunks : 1) : (long)h->sm_count * kBlocksPerSM;
-  return grid * kBlock;
-}
-// cooperative kernel: lanes per problem in the stage-parallel phases.  A whole warp per problem while that still
-// gives every SM at most ~8 warps (the latency regime), otherwise 8 lanes (four problems per warp).
-static int coop_gp_for(const lmato_handle* h, int64_t B) {
-  if (h->opt.coop_lanes == 8 || h->opt.coop_lanes == 32) return h->opt.coop_lanes;
-  return B <= (int64_t)h->sm_count * 8 ? 32 : 8;
-}
-// CTAs per SM: one (255 registers per thread) while one CTA per SM holds the whole batch, else two
-static int coop_bps_for(const lmato_handle* h, int64_t B, int gp) {
-  return B <= (int64_t)h->sm_count * (kCoopBlock / gp) ? 1 : kCoopBlocksPerSM;
-}
-// CTAs of 256 threads = 256/GP groups; a warp's chunk is 32/GP problems
-static long coop_grid_for(const lmato_handle* h, int64_t B, int gp) {
-  const long chunks = (B + (32 / gp) - 1) / (32 / gp);
-  const long cap = (long)h->sm_count * coop_bps_for(h, B, gp);
-  return chunks < cap ? (chunks > 0 ? chunks : 1) : cap;
-}
-static size_t coop_ws_bytes(const lmato_handle* h, long grid, int gp) {
-  return sizeof(double) * (size_t)coop::coop_doubles_per_problem(h->nt) * (size_t)(grid * (kCoopBlock / gp));
-}
-static int colloc_gp_for(const lmato_handle* h, int64_t B) { return B <= (int64_t)h->sm_count * 8 ? 32 : 8; }
-static long colloc_grid_for(const lmato_handle* h, int64_t B, int gp) {
-  const long chunks = (B + (32 / gp) - 1) / (32 / gp);
-  const long cap = (long)h->sm_count;
-  return chunks < cap ? (chunks > 0 ? chunks : 1) : cap;
-}
-static size_t ws_bytes_for(const lmato_handle* h, int64_t B) {
-  if (h->nodes > 2) {
-    const int gp = colloc_gp_for(h, B);
-    return sizeof(double) * (size_t)colloc::colloc_doubles_per_problem(h->nt, h->nodes - 1) *
-           (size_t)(colloc_grid_for(h, B, gp) * (kCoopBlock / gp));
-  }
-  if (use_coop(h, B)) { const int gp = coop_gp_for(h, B); return coop_ws_bytes(h, coop_grid_for(h, B, gp), gp); }
-  return sizeof(double) * (size_t)fields_for(h) * (size_t)h->nt * (size_t)slots_for(h, B);
-}
-
 lmato_status_t lmato_workspace_bytes(lmato_handle* h, int64_t B, int64_t* bytes) {
   if (!h || !bytes || B < 0) { set_err("lmato_workspace_bytes: bad argument"); return LMATO_ERR_INVALID; }
-  *bytes = (int64_t)ws_bytes_for(h, B);
+  *bytes = (int64_t)plan_solve(h->sm_count, h->nt, h->nodes, h->model, h->opt, B, h->guess_traj != nullptr, B).ws_bytes;
   return LMATO_OK;
 }
 
@@ -637,10 +574,10 @@ static bool host_can_address(const void* p) {
   return attr.type != cudaMemoryTypeDevice;
 }
 
-lmato_status_t lmato_solve_batch(lmato_handle* h, const double* params, int64_t B,
-                                 double* out_traj, double* out_tf, double* out_final_mass,
-                                 int32_t* out_status, int32_t* out_iters, double* out_kkt,
-                                 void* stream) {
+// lmato_solve_batch for B problems that belong to a batch of warm_batch problems (ascent_plan.h, plan_solve).
+static lmato_status_t solve_batch(lmato_handle* h, const double* params, int64_t B, double* out_traj, double* out_tf,
+                                  double* out_final_mass, int32_t* out_status, int32_t* out_iters, double* out_kkt,
+                                  cudaStream_t st, int64_t warm_batch) {
   if (!h) { set_err("lmato_solve_batch: NULL handle"); return LMATO_ERR_INVALID; }
   if (B < 0) { set_err("lmato_solve_batch: negative batch"); return LMATO_ERR_INVALID; }
   if (B == 0) return LMATO_OK;
@@ -654,72 +591,30 @@ lmato_status_t lmato_solve_batch(lmato_handle* h, const double* params, int64_t 
             "(lmato_solve_batch takes DEVICE pointers; use lmato_solve_batch_host for host buffers)");
     return LMATO_ERR_INVALID;
   }
-  cudaStream_t st = (cudaStream_t)stream;
-  // Every solve on a handle shares its workspace, work-queue counter and warm-start reference.  A solve issued on
-  // a different stream than the previous one first waits (on the device) for that one to finish.
-  if (h->timed && st != h->last_stream) CUDA_TRY(cudaStreamWaitEvent(st, h->ev1, 0));
-  const bool hi_order = h->nodes > 2;        // NODES >= 3: the general collocation kernel
-  if (hi_order && (h->sens_out || h->guess_traj)) {
+  if (h->nodes > 2 && (h->sens_out || h->guess_traj)) {
     set_err("lmato_solve_batch: sensitivities and caller-supplied start points are implemented for NODES = 2 only");
     return LMATO_ERR_UNSUPPORTED;
   }
-  const bool coopk = !hi_order && use_coop(h, B);
-  const long slots = slots_for(h, B);
-  const int gp = coop_gp_for(h, B);
-  const long cgrid = coop_grid_for(h, B, gp);
-  const bool use_dc = dcost_active(h) && !hi_order;   // the l1 move term is carried by the NODES = 2 kernels only
-  // (no batch warm start for the circular model with its move term: the reference column of the 7-state solve
-  //  carries a different MV)
-  const bool warm = !hi_order && !h->guess_traj && !circular_move(h) &&
-                    (h->opt.warm_start == 2 || (h->opt.warm_start == 1 && B >= kWarmStartMinBatch));
-  size_t need = ws_bytes_for(h, B);
-  if (warm) { const size_t r = coop_ws_bytes(h, 1, 32); if (r > need) need = r; }     // the reference solve: one warp of one CTA
-  if (need > h->ws_bytes) {
-    if (h->d_ws) {
-      if (h->timed) CUDA_TRY(cudaEventSynchronize(h->ev1));     // the previous solve may still be using it
-      CUDA_TRY(cudaFree(h->d_ws)); h->d_ws = nullptr; h->ws_bytes = 0;
-    }
-    CUDA_TRY(cudaMalloc(&h->d_ws, need));
-    h->ws_bytes = need;
-  }
-  h->ws_slots = slots;
+  // Every solve on a handle shares its workspace, work-queue counter and warm-start reference.  A solve issued on
+  // a different stream than the previous one first waits (on the device) for that one to finish.
+  if (h->timed && st != h->last_stream) CUDA_TRY(cudaStreamWaitEvent(st, h->ev1, 0));
+  const LaunchPlan plan = plan_solve(h->sm_count, h->nt, h->nodes, h->model, h->opt, B, h->guess_traj != nullptr, warm_batch);
+  if (plan.alloc_bytes > h->ws_bytes && h->timed) CUDA_TRY(cudaEventSynchronize(h->ev1));   // the previous solve may still be using it
+  CUDA_TRY(grow(&h->d_ws, &h->ws_bytes, plan.alloc_bytes));
   CUDA_TRY(cudaMemsetAsync(h->d_counter, 0, sizeof(int), st));
   KArgs a;
   a.params = params;
   a.res = ResultOut{out_traj, out_tf, out_final_mass, out_status, out_iters, out_kkt, h->sens_out, (long)B};
   a.guess_traj = h->guess_traj; a.guess_tf = h->guess_tf;
-  a.ws = h->d_ws; a.slots = slots; a.N = h->nt - 1; a.h = h->d_h; a.tau = h->d_tau;
+  a.ws = h->d_ws; a.slots = plan.slots; a.N = h->nt - 1; a.h = h->d_h; a.tau = h->d_tau;
   a.counter = h->d_counter;
   a.model = h->model;
-  // OTOL / RTOL (LO:31-32): how APMonitor maps them onto IPOPT's `tol` is not verifiable here, so the rule is
-  // the conservative one: the solve runs to the tightest of tol, otol and rtol (defaults 1e-10, 1e-3, 1e-3).
-  double tol = h->opt.tol;
-  if (h->opt.otol > 0.0 && h->opt.otol < tol) tol = h->opt.otol;
-  if (h->opt.rtol > 0.0 && h->opt.rtol < tol) tol = h->opt.rtol;
-  a.O.tol = tol; a.O.mu_init = h->opt.mu_init; a.O.obj_scale = h->opt.obj_scale;
-  // barrier decrease exponent: IPOPT's 1.5 from the cold start, 2 from the batch warm start.  Measured on the
-  // benchmark batch (warm): 1.3 / 1.5 / 1.7 / 2.0 / 2.5 / 3.0 -> 91 / 96 / 95 / 88 / 88 / 115 ms; from the cold
-  // start 2.0 costs 0.7 iterations more than 1.5.  kappa_mu and tau_min do not matter.
-  a.O.kappa_eps = h->opt.kappa_eps; a.O.kappa_mu = 0.2; a.O.theta_mu = 1.5; a.O.tau_min = 0.99;
-  a.O.delta_c = h->opt.delta_c; a.O.tf_guess = h->opt.tf_guess;
-  a.O.max_iter = h->opt.max_iter; a.O.max_ls = h->opt.max_ls;
-  a.O.mu_min_factor = h->opt.mu_min_factor;
-  a.O.n_polish = h->opt.n_polish >= 0 ? h->opt.n_polish : (use_dc ? 2 : 4);
-  // ... 2 from the warm start WITH the move term only.  Without it the control on the singular arc is a nearly flat
-  // direction, and the jump 1e-6 -> 1e-12 leaves a few problems in 10 000 on an error plateau until the stall guard
-  // gives the warm attempt up -- each holding its warp: 65 536 problems, dcost = 0: 260-560 ms with 2, 66 ms with 1.5.
-  a.O.theta_mu_warm = use_dc ? 2.0 : 1.5;
-  {
-    const int on = h->opt.objective_nodes > 0 ? h->opt.objective_nodes : h->nt - 1;
-    a.O.w_dcost = use_dc ? h->opt.obj_scale * h->opt.dcost / (double)on : 0.0;
-  }
   a.ref = nullptr; a.ref_mode = 0;
+  a.O = solve_options(h->opt, h->nt, plan.use_dc);
+  a.coll = h->d_coll;
   CUDA_TRY(cudaEventRecord(h->ev0, st));
-  // (a caller-supplied guess replaces the batch warm start)
-  if (warm) {
-    // reference problem = batch mean, solved down to mu_ref only by ONE group of the cooperative kernel without
-    // the move term (at mu_ref >> w it is immaterial): ~10 iterations from the cold start on the first call,
-    // 1-2 from the previous call's reference afterwards
+  if (plan.warm) {
+    // the reference problem is the batch mean, solved by ONE group of the cooperative kernel
     mean_params_kernel<<<LMATO_NPARAM, 256, 0, st>>>(params, B, h->d_refparams);
     CUDA_TRY(cudaGetLastError());
     KArgs r = a;
@@ -728,36 +623,27 @@ lmato_status_t lmato_solve_batch(lmato_handle* h, const double* params, int64_t 
     r.res = ResultOut{nullptr, scratch, scratch + 1, (int*)(scratch + 2), (int*)(scratch + 3), scratch + 4, nullptr, 1};
     r.guess_traj = nullptr; r.guess_tf = nullptr;
     r.ref = h->d_ref; r.ref_mode = 1;
-    r.O.tol = 10.0 * h->opt.mu_ref; r.O.mu_min_factor = 0.1; r.O.n_polish = 0;
-    r.O.w_dcost = 0.0;
-    coop_launch<32, 1>(0, 1, st, r);
-    CUDA_TRY(cudaGetLastError());
+    r.O = reference_options(a.O, h->opt.mu_ref);
+    const lmato_status_t rc = launch(KernelKey{kCoopKernel, 32, 1, 0}, 1, st, r);
+    if (rc != LMATO_OK) return rc;
     CUDA_TRY(cudaMemsetAsync(h->d_counter, 0, sizeof(int), st));
     a.ref = h->d_ref; a.ref_mode = 2;
     h->launches += 2;
   }
-  a.coll = h->d_coll;
-  if (hi_order) {
-    const int cgp = colloc_gp_for(h, B);
-    const int cg = (int)colloc_grid_for(h, B, cgp);
-    if (cgp == 32) ascent_colloc_kernel<32><<<cg, kCoopBlock, 0, st>>>(a);
-    else ascent_colloc_kernel<8><<<cg, kCoopBlock, 0, st>>>(a);
-  } else if (coopk) {
-    const int bps = coop_bps_for(h, B, gp);
-    const int mv = !use_dc ? 0 : circular_move(h) ? 2 : 1;
-    if (gp == 32) { if (bps == 1) coop_launch<32, 1>(mv, cgrid, st, a); else coop_launch<32, 2>(mv, cgrid, st, a); }
-    else          { if (bps == 1) coop_launch<8, 1>(mv, cgrid, st, a); else coop_launch<8, 2>(mv, cgrid, st, a); }
-  } else {
-    const int grid = (int)(slots / kBlock);
-    if (use_dc) ascent_ipm_kernel<Sweeps8><<<grid, kBlock, kTileSmem, st>>>(a);
-    else ascent_ipm_kernel<Sweeps7><<<grid, kBlock, kTileSmem, st>>>(a);
-  }
-  CUDA_TRY(cudaGetLastError());
+  const lmato_status_t rc = launch(plan.kernel, plan.grid, st, a);
+  if (rc != LMATO_OK) return rc;
   CUDA_TRY(cudaEventRecord(h->ev1, st));
   h->last_stream = st; h->timed = true;
-  h->last_coop = coopk;
   h->launches += 1;
   return LMATO_OK;
+}
+
+lmato_status_t lmato_solve_batch(lmato_handle* h, const double* params, int64_t B,
+                                 double* out_traj, double* out_tf, double* out_final_mass,
+                                 int32_t* out_status, int32_t* out_iters, double* out_kkt,
+                                 void* stream) {
+  return solve_batch(h, params, B, out_traj, out_tf, out_final_mass, out_status, out_iters, out_kkt,
+                     (cudaStream_t)stream, B);
 }
 
 lmato_status_t lmato_last_kernel_ms(lmato_handle* h, double* ms) {
@@ -794,12 +680,7 @@ lmato_status_t lmato_solve_batch_host(lmato_handle* h, const double* params, int
   }
   CUDA_TRY(cudaSetDevice(h->device));
   const size_t pbytes = sizeof(double) * LMATO_NPARAM * (size_t)B;
-  if (pbytes > h->params_bytes) {
-    if (h->d_params) CUDA_TRY(cudaFree(h->d_params));
-    h->d_params = nullptr; h->params_bytes = 0;
-    CUDA_TRY(cudaMalloc(&h->d_params, pbytes));
-    h->params_bytes = pbytes;
-  }
+  CUDA_TRY(grow(&h->d_params, &h->params_bytes, pbytes));
   // The per-node trajectories are 16 KB per problem (1 GB for 65 536 problems).  If the caller's
   // buffer is pinned the kernel writes them there directly, chunk by chunk as problems finish, so the
   // transfer over PCIe overlaps the solve; a pageable buffer is filled by a copy after the kernel.
@@ -815,12 +696,7 @@ lmato_status_t lmato_solve_batch_host(lmato_handle* h, const double* params, int
   const size_t sens_n = sens_host ? (size_t)LMATO_NSENS * (size_t)B : 0;
   // layout of d_out: traj (only when staged) | sens | tf | fmass | kkt | status | iters
   const size_t obytes = sizeof(double) * (traj_stage + sens_n + 3 * (size_t)B) + sizeof(int32_t) * 2 * (size_t)B;
-  if (obytes > h->out_bytes) {
-    if (h->d_out) CUDA_TRY(cudaFree(h->d_out));
-    h->d_out = nullptr; h->out_bytes = 0;
-    CUDA_TRY(cudaMalloc(&h->d_out, obytes));
-    h->out_bytes = obytes;
-  }
+  CUDA_TRY(grow(&h->d_out, &h->out_bytes, obytes));
   double* d_traj = out_traj ? (traj_alias ? traj_alias : h->d_out) : nullptr;
   double* d_sens = sens_host ? h->d_out + traj_stage : nullptr;
   double* d_tf = h->d_out + traj_stage + sens_n;
@@ -836,12 +712,7 @@ lmato_status_t lmato_solve_batch_host(lmato_handle* h, const double* params, int
   if (guess_traj_host) {
     const size_t gn = (size_t)LMATO_NVAR * h->nt * (size_t)B;
     const size_t gbytes = sizeof(double) * (gn + (size_t)B);
-    if (gbytes > h->guess_bytes) {
-      if (h->d_guess) CUDA_TRY(cudaFree(h->d_guess));
-      h->d_guess = nullptr; h->guess_bytes = 0;
-      CUDA_TRY(cudaMalloc(&h->d_guess, gbytes));
-      h->guess_bytes = gbytes;
-    }
+    CUDA_TRY(grow(&h->d_guess, &h->guess_bytes, gbytes));
     CUDA_TRY(cudaMemcpyAsync(h->d_guess, guess_traj_host, sizeof(double) * gn, cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(h->d_guess + gn, guess_tf_host, sizeof(double) * (size_t)B, cudaMemcpyHostToDevice, st));
     h->guess_traj = h->d_guess; h->guess_tf = h->d_guess + gn;
@@ -1035,32 +906,21 @@ lmato_status_t lmato_multi_solve_host(lmato_multi* m, const double* params, int6
     s.n = (B * (g + 1)) / G - s.lo;
     if (s.n == 0) continue;
     CUDA_TRY(cudaSetDevice(h->device));
-    // the shards of one batch keep the batch warm start even when a shard alone is small
-    const int32_t ws_saved = h->opt.warm_start;
-    if (ws_saved == 1 && B >= kWarmStartMinBatch) h->opt.warm_start = 2;
     const size_t pbytes = sizeof(double) * LMATO_NPARAM * (size_t)s.n;
-    if (pbytes > m->params_bytes[g]) {
-      CUDA_TRY(cudaStreamSynchronize(m->st[g]));
-      cudaFree(m->d_params[g]); m->d_params[g] = nullptr; m->params_bytes[g] = 0;
-      CUDA_TRY(cudaMalloc(&m->d_params[g], pbytes));
-      m->params_bytes[g] = pbytes;
-    }
     const size_t traj_n = out_traj ? (size_t)LMATO_NVAR * nt * (size_t)s.n : 0;
     const size_t obytes = sizeof(double) * (traj_n + 3 * (size_t)s.n) + sizeof(int32_t) * 2 * (size_t)s.n;
-    if (obytes > m->out_bytes[g]) {
-      CUDA_TRY(cudaStreamSynchronize(m->st[g]));
-      cudaFree(m->d_out[g]); m->d_out[g] = nullptr; m->out_bytes[g] = 0;
-      CUDA_TRY(cudaMalloc(&m->d_out[g], obytes));
-      m->out_bytes[g] = obytes;
-    }
+    // the previous solve on this stream may still be using the buffers
+    if (pbytes > m->params_bytes[g] || obytes > m->out_bytes[g]) CUDA_TRY(cudaStreamSynchronize(m->st[g]));
+    CUDA_TRY(grow(&m->d_params[g], &m->params_bytes[g], pbytes));
+    CUDA_TRY(grow(&m->d_out[g], &m->out_bytes[g], obytes));
     s.traj = out_traj ? m->d_out[g] : nullptr;
     s.tf = m->d_out[g] + traj_n; s.fm = s.tf + s.n; s.kkt = s.fm + s.n;
     s.st = (int32_t*)(s.kkt + s.n); s.it = s.st + s.n;
     // columns [lo, lo+n) of the row-major [NPARAM][B] block
     CUDA_TRY(cudaMemcpy2DAsync(m->d_params[g], sizeof(double) * s.n, params + s.lo, sizeof(double) * B,
                                sizeof(double) * s.n, LMATO_NPARAM, cudaMemcpyHostToDevice, m->st[g]));
-    const lmato_status_t rc = lmato_solve_batch(h, m->d_params[g], s.n, s.traj, s.tf, s.fm, s.st, s.it, s.kkt, m->st[g]);
-    h->opt.warm_start = ws_saved;
+    // the shards of one batch keep the batch warm start even when a shard alone is small
+    const lmato_status_t rc = solve_batch(h, m->d_params[g], s.n, s.traj, s.tf, s.fm, s.st, s.it, s.kkt, m->st[g], B);
     if (rc != LMATO_OK) return rc;
   }
   // phase 2: every device writes its slice of the host arrays

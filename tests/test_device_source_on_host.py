@@ -4,7 +4,8 @@
 `ascent_result.cuh` are written so that g++ accepts them (tools/hostsim): the parameter derivation, the sweeps, the
 IPM driver with its start and restart steps (`ipm_start` / `ipm_restart`, the collocation start ladder included),
 the model derivatives and the result writer below are the very lines the CUDA kernels run, executed by one CPU
-thread.  Only the kernels' problem queue (`solve_queue`) is not run here.  This gives the CPU-only test tier a check of the solver's logic against the oracle's golden vectors,
+thread.  Only the kernels' problem queue (`solve_queue`) is not run here.  The launch plan of `ascent_plan.h`
+(which kernel, grid and workspace a batch gets) is checked here too.  This gives the CPU-only test tier a check of the solver's logic against the oracle's golden vectors,
 and of the hand-derived derivatives and the sensitivity output against finite differences.  It is test
 infrastructure only: the product has no CPU path (`_cabi.lib()` raises without
 the CUDA library), and nothing here is imported by the package.
@@ -295,3 +296,69 @@ def test_start_points_on_every_layout(hostsim, monkeypatch):
             assert its_warm < its_cold, (fn, its_warm, its_cold)
         for a, c in zip(warm["hostsim_solve"], warm["hostsim_solve_coop"]):
             assert abs(a[1] - c[1]) / a[1] < 1e-11 and abs(a[2] - c[2]) <= 1, (a[:3], c[:3])
+
+
+def test_launch_plan_matches_the_dispatch_rules(hostsim):
+    """plan_solve (csrc/ascent_plan.h), the library's choice of kernel, grid, workspace and warm start, against the
+    rules written out in tests/dispatch_rules.py, which the GPU kernel matrix uses to reach every kernel variant: on
+    three SM counts, for every variant of that matrix at its batch size, and for every kernel / lanes / model / DCOST
+    setting one below, at and one above each window edge."""
+    from dispatch_rules import COOP_MAX_BATCH, VARIANTS, V
+    L, nt = hostsim, 200
+    keys = ("kind", "lanes", "bps", "move", "grid", "slots", "ws", "alloc", "warm", "use_dc")
+
+    def plan(S, B, v, nodes=2, warm_start=1, guess=False, warm_batch=None):
+        out = (C.c_int64 * len(keys))()
+        L.hostsim_plan(S, nt, nodes, 1 if v.model == "circular" else 0, {"auto": 0, "thread": 1, "coop": 2}[v.kernel],
+                       v.coop_lanes, C.c_double(v.dcost), warm_start, C.c_int64(B), int(guess),
+                       C.c_int64(B if warm_batch is None else warm_batch), out)
+        return dict(zip(keys, out))
+
+    coop_doubles = 258 * nt       # DESIGN.md section 3b: X[2][24] + D[16] + M[2][52] + K[10] + H[8] + V[72] per stage
+    ref_ws = 8 * coop_doubles * (256 // 32)      # the warm start's reference solve: one warp of one CTA
+    grid = lambda B, lanes, cap: min(max(-(-B * lanes // 32), 1), cap)
+    for S in (148, 132, 100):
+        edges = sorted({0, 1} | {e + d for e in (8 * S, 32 * S, COOP_MAX_BATCH) for d in (-1, 0, 1)})
+        cases = [(v, v.batch(S)) for v in VARIANTS if v.batch(S) is not None]
+        for model, dcost in (("elliptical", 1e-5), ("elliptical", 0.0), ("circular", 1e-5), ("circular", 0.0)):
+            for kernel in ("auto", "thread", "coop"):
+                for lanes in (0, 8, 32):
+                    cases += [(V("", None, model, dcost, kernel, lanes), B) for B in edges]
+        for v, B in cases:
+            p, exp = plan(S, B, v), v.expect(S, B)
+            tag = (S, B, v.id, v.model, v.dcost, v.kernel, v.coop_lanes)
+            assert p["use_dc"] == (v.dcost > 0), tag
+            assert p["slots"] == 256 * grid(B, 1, S), tag
+            if exp[0] == "thread":
+                assert (p["kind"], p["lanes"], p["bps"], p["move"]) == (0, 1, 1, int(exp[1] == 8)), (tag, p)
+                assert p["grid"] == grid(B, 1, S), tag
+                assert p["ws"] == 8 * (67 if v.dcost > 0 else 55) * nt * 256 * p["grid"], (tag, p)
+            else:
+                assert (p["kind"], p["lanes"], p["bps"], p["move"]) == (1,) + exp[1:], (tag, p, exp)
+                assert p["grid"] == grid(B, exp[1], S * exp[2]), (tag, p)
+                assert p["ws"] == 8 * coop_doubles * p["grid"] * (256 // exp[1]), (tag, p)
+            warm = not (v.model == "circular" and v.dcost > 0) and B >= 512
+            assert p["warm"] == warm, (tag, p)
+            assert p["alloc"] == (max(p["ws"], ref_ws) if warm else p["ws"]), (tag, p)
+        # NODES = 3..6: the collocation kernel, whatever the kernel options say; no move term, no warm start
+        for nodes in (3, 4, 5, 6):
+            colloc_doubles = plan(S, 1, V("", 1), nodes)["ws"] // (8 * 8)
+            for kernel, lanes in (("auto", 0), ("thread", 0), ("coop", 8)):
+                for B in edges:
+                    p = plan(S, B, V("", None, kernel=kernel, coop_lanes=lanes), nodes, warm_start=2)
+                    gp = 32 if B <= 8 * S else 8
+                    assert (p["kind"], p["lanes"], p["bps"], p["move"], p["use_dc"], p["warm"]) == (2, gp, 1, 0, 0, 0), (S, B, p)
+                    assert p["grid"] == grid(B, gp, S) and p["slots"] == 256 * grid(B, 1, S), (S, B, p)
+                    assert p["ws"] == p["alloc"] == 8 * colloc_doubles * p["grid"] * (256 // gp), (S, B, p)
+    # the warm start: warm_start 0 / 1 / 2 around 512 problems, a caller's start point, the circular model with its
+    # move term, and a 300-problem shard of a 1 024-problem batch
+    S, v = 148, V("", None)
+    for B in (511, 512):
+        assert [plan(S, B, v, warm_start=w)["warm"] for w in (0, 1, 2)] == [0, int(B >= 512), 1], B
+        assert plan(S, B, v, warm_start=2, guess=True)["warm"] == 0
+        assert plan(S, B, V("", None, "circular"), warm_start=2)["warm"] == 0
+        assert plan(S, B, V("", None, "circular", 0.0), warm_start=2)["warm"] == 1
+    assert plan(S, 300, v, warm_batch=1024)["warm"] == 1 and plan(S, 300, v, warm_batch=511)["warm"] == 0
+    assert plan(S, 300, v, warm_start=0, warm_batch=1024)["warm"] == 0
+    p = plan(S, 1, v, warm_start=2)                   # one warp of one CTA, as the reference solve
+    assert p["warm"] == 1 and p["alloc"] == p["ws"] == ref_ws, p

@@ -1,7 +1,6 @@
 """Every kernel instantiation that `lmato_solve_batch` can launch, against the oracle.
 
-The dispatcher (csrc/ascent_cabi.cu: use_coop, coop_gp_for, coop_bps_for) picks, by batch size, DCOST, model and
-options, one of
+The launch plan (csrc/ascent_plan.h: plan_solve) picks, by batch size, DCOST, model and options, one of
     ascent_ipm_kernel<Sweeps7 | Sweeps8>          one problem per thread (above 6 144 problems, or kernel="thread")
     ascent_coop_kernel<G, GP, MOVE, BPS>          GP = 32 lanes per problem up to 8 problems per SM, else 8;
                                                   BPS = 2 CTAs per SM once one CTA per SM cannot hold the batch;
@@ -11,8 +10,9 @@ own workspace layout (SW::store_node) and reads the converged iterate through it
 (csrc/ascent_result.cuh), which the cooperative kernels run with the problem's lanes summing over the group.  The
 table below reaches each of them; a
 test id names the instantiation.  Batch sizes are derived from the device's SM
-count with the dispatcher's rules, so the same table picks the same kernels on any GPU (a variant whose batch-size
-window is empty there is skipped).
+count with the dispatch rules of tests/dispatch_rules.py, which test_device_source_on_host.py checks against
+plan_solve itself, so the same table picks the same kernels on any GPU (a variant whose batch-size window is empty
+there is skipped).
 
 Each batch carries known problems: the seed-11 dispersions are prefix-stable, so `dispersed_params(B, seed=11)` starts
 with the rows of the oracle fixtures, and copies of the nominal problem (problem 0 of every such batch) sit at warp,
@@ -27,6 +27,8 @@ import numpy as np
 import pytest
 import torch
 
+from dispatch_rules import VARIANTS
+
 pytestmark = pytest.mark.gpu
 
 VAR_ROWS = ["y", "ydot", "ydoubledot", "x", "xdot", "xdoubledot", "angle", "angledot", "mass",
@@ -34,8 +36,6 @@ VAR_ROWS = ["y", "ydot", "ydoubledot", "x", "xdot", "xdoubledot", "angle", "angl
 CIRCULAR_ROWS = ["y", "ydot", "ydoubledot", "x", "xdot", "xdoubledot", "mass", "angle"]   # the model's Vars and MV
 SENS_NAMES = ["Ft", "M0", "M_dot", "angle_doubledot_max"]
 STATE_RTOL = 1e-4
-COOP_MAX_BATCH = 6144         # kCoopMaxBatch: AUTO runs the cooperative kernel up to this batch size
-COOP_BLOCK = 256              # kCoopBlock
 # d tf / d (Ft, M0, M_dot) against the oracle's central differences, relative, per regime: ten times the worst error
 # measured over all variants on a B200 (1000 W): 2.9e-6 with DCOST, 5.3e-7 without, 1.2e-8 for the circular model.
 SENS_RTOL = {"dcost": 3e-5, "nodcost": 5e-6, "circular": 1.2e-7}
@@ -43,66 +43,6 @@ SENS_RTOL = {"dcost": 3e-5, "nodcost": 5e-6, "circular": 1.2e-7}
 # by 1.5e-3 between relative steps of 1e-3 and 2.5e-4), so the oracle's quotient carries an error up to its
 # one-sided spread |forward - backward| / |central|, which is added to this floor
 SENS_ADDM_RTOL = 1e-5
-
-
-def _gp(S, B, lanes=0):
-    """coop_gp_for: lanes per problem."""
-    return lanes if lanes else (32 if B <= 8 * S else 8)
-
-
-def _bps(S, B, gp):
-    """coop_bps_for: CTAs per SM."""
-    return 1 if B <= S * (COOP_BLOCK // gp) else 2
-
-
-def _coop_window(S, gp, bps, cap=COOP_MAX_BATCH):
-    """Batch sizes (lo, hi] for which AUTO picks coop<gp, bps> (lanes chosen by size)."""
-    lo, hi = (0, 8 * S) if gp == 32 else (8 * S, cap)
-    if gp == 8:
-        lo, hi = (lo, min(hi, 32 * S)) if bps == 1 else (max(lo, 32 * S), hi)
-    return lo, hi
-
-
-def _top(window):
-    """The largest batch of the window that still leaves a partial last chunk (two short of the top)."""
-    lo, hi = window
-    return hi - 2 if hi - 2 > lo else None
-
-
-class V:
-    def __init__(self, vid, B, model="elliptical", dcost=1e-5, kernel="auto", coop_lanes=0):
-        self.id, self.B, self.model, self.dcost, self.kernel, self.coop_lanes = vid, B, model, dcost, kernel, coop_lanes
-
-    def batch(self, S):
-        return self.B(S) if callable(self.B) else self.B
-
-    def expect(self, S, B):
-        """(kernel, GP, BPS, MOVE) the dispatcher must pick for B on a device with S SMs."""
-        coop = (self.model == "circular" and self.dcost > 0) or self.kernel == "coop" or \
-               (self.kernel == "auto" and B <= COOP_MAX_BATCH)
-        if not coop:
-            return ("thread", 8 if self.dcost > 0 else 7)
-        gp = _gp(S, B, self.coop_lanes)
-        move = 0 if self.dcost == 0 else (2 if self.model == "circular" else 1)
-        return ("coop", gp, _bps(S, B, gp), move)
-
-
-VARIANTS = [
-    V("thread-sweeps8", 65536),                                   # the benchmark's configuration (AUTO)
-    V("thread-sweeps7", 1000, dcost=0.0, kernel="thread"),
-    V("coop-gp32-bps1-move0", lambda S: _top(_coop_window(S, 32, 1)), dcost=0.0),
-    V("coop-gp32-bps1-move1", lambda S: _top(_coop_window(S, 32, 1))),
-    V("coop-gp8-bps1-move0", lambda S: _top(_coop_window(S, 8, 1)), dcost=0.0),
-    V("coop-gp8-bps1-move1", lambda S: _top(_coop_window(S, 8, 1))),
-    V("coop-gp8-bps2-move0", lambda S: _top(_coop_window(S, 8, 2)), dcost=0.0),
-    V("coop-gp8-bps2-move1", lambda S: _top(_coop_window(S, 8, 2))),
-    V("coop-gp32-bps2-move1", lambda S: 8 * S + 62 if 8 * S + 62 <= COOP_MAX_BATCH else None, coop_lanes=32),
-    V("circular-coop-gp32-bps1-move2", 1, model="circular"),
-    V("circular-coop-gp8-bps1-move2", lambda S: _top(_coop_window(S, 8, 1, cap=32 * S)), model="circular"),
-    V("circular-coop-gp8-bps2-move2", lambda S: max(COOP_MAX_BATCH - 2, 32 * S + 30), model="circular"),
-    V("circular-thread-sweeps7", 1000, model="circular", dcost=0.0, kernel="thread"),
-    V("circular-coop-gp8-bps1-move0", lambda S: _top(_coop_window(S, 8, 1)), model="circular", dcost=0.0),
-]
 
 
 @pytest.fixture(scope="module")

@@ -16,6 +16,7 @@
 #include <random>
 #include <array>
 #include "ascent_colloc.cuh"
+#include "ascent_plan.h"
 #include "ascent_result.cuh"
 
 using namespace lmato;
@@ -30,13 +31,20 @@ static std::array<double, LMATO_NPARAM> make_params(double Ft, double M0, double
   return r;
 }
 
-// The options every entry point starts from (those lmato_solve_batch sets, with MAX_ITER 500); each entry point then
-// applies its own environment overrides.
-static Options make_options(double tol, double obj_scale, double mu_min_factor, int n_polish, double w_dcost) {
-  Options O;
-  O.tol = tol; O.mu_init = 0.1; O.obj_scale = obj_scale; O.kappa_eps = 30.0; O.kappa_mu = 0.2; O.theta_mu = 1.5; O.theta_mu_warm = 2.0;
-  O.tau_min = 0.99; O.delta_c = 1e-8; O.tf_guess = 0.9; O.max_iter = 500; O.max_ls = 40; O.mu_min_factor = mu_min_factor;
-  O.n_polish = n_polish; O.w_dcost = w_dcost;
+// The options every entry point starts from: the library's solve_options on its defaults, with the solve running to
+// exactly `tol` (no OTOL / RTOL) and MAX_ITER 500; each entry point then applies its own environment overrides.  Three
+// departures from the library are kept on purpose, so that host results stay comparable with earlier ones:
+//   - w_dcost is the raw move weight `wdc` (WDC), not obj_scale * dcost / objective_nodes;
+//   - n_polish is the caller's (4 unless NPOL is set, 2 in hostsim_warm_batch), where the library's automatic value
+//     is 2 with the move term and 4 without;
+//   - theta_mu_warm is 2.0 with and without the move term (the library: 1.5 without).
+static Options make_options(int nt, double tol, double obj_scale, double mu_min_factor, int n_polish, double wdc) {
+  lmato_options o = default_options();
+  o.tol = tol; o.otol = 0.0; o.rtol = 0.0; o.obj_scale = obj_scale; o.mu_min_factor = mu_min_factor; o.max_iter = 500;
+  o.n_polish = n_polish;
+  Options O = solve_options(o, nt, wdc > 0);
+  O.w_dcost = wdc;
+  O.theta_mu_warm = 2.0;
   return O;
 }
 
@@ -75,7 +83,7 @@ int main(int argc, char** argv) {
   std::vector<double> h(N + 1), tau(N + 1);
   for (int k = 0; k <= N; ++k) { tau[k] = (double)k / N; h[k] = k ? tau[k] - tau[k - 1] : 0.0; }
   Mesh M{N, h.data(), tau.data()};
-  Options O = make_options(1e-10, 10.0, 1e-3, 4, getenv("WDC") ? atof(getenv("WDC")) : 0.0);
+  Options O = make_options(nt, 1e-10, 10.0, 1e-3, 4, getenv("WDC") ? atof(getenv("WDC")) : 0.0);
   if (getenv("MMF")) O.mu_min_factor = atof(getenv("MMF"));
   if (getenv("NPOL")) O.n_polish = atoi(getenv("NPOL"));
   if (getenv("THMU")) O.theta_mu = atof(getenv("THMU"));
@@ -139,7 +147,7 @@ extern "C" int hostsim_solve(const double* raw14, int nt, const double* time, do
   std::vector<double> h(N + 1), tau(N + 1);
   for (int k = 0; k <= N; ++k) { tau[k] = time ? time[k] : (double)k / N; h[k] = k ? tau[k] - tau[k - 1] : 0.0; }
   Mesh M{N, h.data(), tau.data()};
-  const Options O = make_options(tol, obj_scale, mu_min_factor, getenv("NPOL") ? atoi(getenv("NPOL")) : 4,
+  const Options O = make_options(nt, tol, obj_scale, mu_min_factor, getenv("NPOL") ? atoi(getenv("NPOL")) : 4,
                                  getenv("WDC") ? atof(getenv("WDC")) : 0.0);
   const int model = model_from_env();
   const Params P = derive_params(raw14, 1, 0, model);      // as the thread kernel: no circular move formulation
@@ -206,7 +214,7 @@ extern "C" int hostsim_solve_coop(const double* raw14, int nt, const double* tim
   std::vector<double> h(N + 1), tau(N + 1);
   for (int k = 0; k <= N; ++k) { tau[k] = time ? time[k] : (double)k / N; h[k] = k ? tau[k] - tau[k - 1] : 0.0; }
   Mesh M{N, h.data(), tau.data()};
-  const Options O = make_options(tol, obj_scale, mu_min_factor, getenv("NPOL") ? atoi(getenv("NPOL")) : 4,
+  const Options O = make_options(nt, tol, obj_scale, mu_min_factor, getenv("NPOL") ? atoi(getenv("NPOL")) : 4,
                                  getenv("WDC") ? atof(getenv("WDC")) : 0.0);
   const int model = model_from_env();
   const bool DC = O.w_dcost > 0;
@@ -235,7 +243,7 @@ extern "C" int hostsim_solve_colloc(const double* raw14, int nt, const double* t
   std::vector<double> h(N + 1), tau(N + 1);
   for (int k = 0; k <= N; ++k) { tau[k] = time ? time[k] : (double)k / N; h[k] = k ? tau[k] - tau[k - 1] : 0.0; }
   Mesh M{N, h.data(), tau.data()};
-  Options O = make_options(tol, obj_scale, mu_min_factor, getenv("NPOL") ? atoi(getenv("NPOL")) : 4, 0.0);
+  Options O = make_options(nt, tol, obj_scale, mu_min_factor, getenv("NPOL") ? atoi(getenv("NPOL")) : 4, 0.0);
   if (getenv("TF0")) O.tf_guess = atof(getenv("TF0"));
   const Params P = derive_params(raw14, 1, 0, LMATO_MODEL_ELLIPTICAL);   // NODES >= 3: the elliptical model only
   colloc::Coll C;
@@ -260,7 +268,7 @@ extern "C" int hostsim_reference(const double* raw14, int nt, double mu_ref, dou
   std::vector<double> h(N + 1), tau(N + 1);
   for (int k = 0; k <= N; ++k) { tau[k] = (double)k / N; h[k] = k ? tau[k] - tau[k - 1] : 0.0; }
   Mesh M{N, h.data(), tau.data()};
-  Options O = make_options(10.0 * mu_ref, 10.0, 0.1, 0, 0.0);
+  Options O = reference_options(make_options(nt, 1e-10, 10.0, 1e-3, 4, 0.0), mu_ref);
   if (getenv("KEPS")) O.kappa_eps = atof(getenv("KEPS"));
   if (getenv("KMU")) O.kappa_mu = atof(getenv("KMU"));
   const Params P = derive_params(raw14, 1, 0, model_from_env());
@@ -286,7 +294,7 @@ extern "C" double hostsim_warm_batch(int nprob, int nt, double wdc, double mu_re
   std::vector<double> h(N + 1), tau(N + 1);
   for (int k = 0; k <= N; ++k) { tau[k] = (double)k / N; h[k] = k ? tau[k] - tau[k - 1] : 0.0; }
   Mesh M{N, h.data(), tau.data()};
-  Options O = make_options(1e-10, 10.0, 1e-3, 2, wdc);
+  Options O = make_options(nt, 1e-10, 10.0, 1e-3, 2, wdc);
   if (getenv("THMUW")) O.theta_mu_warm = atof(getenv("THMUW"));
   if (getenv("KEPS")) O.kappa_eps = atof(getenv("KEPS"));
   if (getenv("KMU")) O.kappa_mu = atof(getenv("KMU"));
@@ -324,4 +332,16 @@ extern "C" double hostsim_warm_batch(int nprob, int nt, double wdc, double mu_re
   }
   hostsim_set_start(nullptr, nullptr, nullptr);
   return itsum / nprob;
+}
+
+// plan_solve (csrc/ascent_plan.h) for a handle with the default options but for kernel, coop_lanes, dcost and
+// warm_start: out = {kind, lanes, ctas_per_sm, move, grid, slots, ws_bytes, alloc_bytes, warm, use_dc}.
+extern "C" void hostsim_plan(int sm_count, int nt, int nodes, int model, int kernel, int coop_lanes, double dcost,
+                             int warm_start, int64_t B, int has_guess, int64_t warm_batch, int64_t* out) {
+  lmato_options o = default_options();
+  o.kernel = kernel; o.coop_lanes = coop_lanes; o.dcost = dcost; o.warm_start = warm_start;
+  const LaunchPlan p = plan_solve(sm_count, nt, nodes, model, o, B, has_guess != 0, warm_batch);
+  const int64_t v[10] = {p.kernel.kind, p.kernel.lanes, p.kernel.ctas_per_sm, p.kernel.move, p.grid, p.slots,
+                         (int64_t)p.ws_bytes, (int64_t)p.alloc_bytes, p.warm, p.use_dc};
+  for (int i = 0; i < 10; ++i) out[i] = v[i];
 }
