@@ -10,6 +10,10 @@
  * this boundary; every function returns an lmato_status_t and lmato_last_error() gives
  * the text of the last failure on the calling thread.
  *
+ * Beyond the reference's solve there are post-solve checks: lmato_coast_orbit (the PDF's orbit coast) and
+ * lmato_fly_control, which flies each solved control through the continuous dynamics and reports how far the vehicle
+ * really ends up from the target orbit (the transcription error of the solve).
+ *
  * Threading: a handle is bound to one CUDA device and must be used from one host thread
  * at a time.  Solves on one handle share its workspace: they are serialised on the device even when
  * issued on different streams (a solve on a new stream waits for the handle's previous solve).
@@ -236,6 +240,29 @@ lmato_status_t lmato_measure_fp64_peak(lmato_handle* h, double* gflops);
  * Asynchronous on `stream`. */
 lmato_status_t lmato_coast_orbit(lmato_handle* h, const double* state, int64_t B, double gm, double dt,
                                  int64_t nsteps, double* out, void* stream);
+
+/* Post-solve flight check (no counterpart in the reference): fly each solved control through the continuous ascent
+ * dynamics (LO:114-136) and report where the vehicle really ends up.  A solve returns the optimum of the transcribed
+ * problem (backward Euler for NODES = 2); flown, the NODES = 2 plan of the reference script (nt = 200) misses the
+ * target radius by about 2 km and the target speed by about 10 m/s (DESIGN.md section 7).  Classical RK4 in
+ * normalised time with `substeps` equal sub-steps per mesh step, the MV of node k held on (t_{k-1}, t_k] (MV_TYPE = 0,
+ * LO:29, as both transcriptions hold it), from the pinned zeros of node 0 (LO:145-151).  The flight does not depend on
+ * the handle's NODES; it uses the handle's mesh and model.  One thread per problem.
+ *   params     [LMATO_NPARAM][B]
+ *   traj       [LMATO_NVAR][nt][B]   a solve's out_traj; only the MV row is read (angledoubledot, or angle for
+ *                                    LMATO_MODEL_CIRCULAR, PDF p.27)
+ *   tf         [B]   the solved scaled final time
+ *   out_final  [LMATO_NFLY][B]
+ *   out_traj   [LMATO_NVAR][nt][B] or NULL: the flown states in the layout of a solve (node 0 zero, the acceleration
+ *              rows evaluated at the flown nodes, the MV row copied from traj, rows the model lacks zero)
+ * DEVICE pointers, asynchronous on `stream`.  The call neither uses nor waits for the handle's solve workspace: stream
+ * order is the only ordering it needs with respect to solves.  Problems that did not converge are flown as given.
+ * LMATO_ERR_INVALID for a NULL handle or buffer, B < 0 or substeps < 1; B = 0 does nothing. */
+#define LMATO_NFLY 10   /* rows: y, ydot, x, xdot, angle, angledot, mass at tf (scaled, like out_traj),
+                           radius miss [m], speed miss [m/s], flight-path angle [rad] */
+lmato_status_t lmato_fly_control(lmato_handle* h, const double* params, int64_t B, const double* traj,
+                                 const double* tf, int32_t substeps, double* out_final /* [LMATO_NFLY][B] */,
+                                 double* out_traj /* [LMATO_NVAR][nt][B] or NULL */, void* stream);
 
 /* Device self-test of the solver's branch-free FP64 math (rcp, rsqrt, log, sin, cos) against the
  * CUDA math library: max_err5 = {rel rcp, rel rsqrt, rel log, abs sin, abs cos}. */

@@ -21,6 +21,9 @@ INCLUDE = os.path.join(os.path.dirname(_HERE), "include")
 NPARAM = 14
 NVAR = 10
 NSENS = 4
+NFLY = 10
+FLY_ROWS = ["y", "ydot", "x", "xdot", "angle", "angledot", "mass", "radius_miss_m", "speed_miss_mps",
+            "flight_path_angle_rad"]                             # rows of lmato_fly_control's out_final
 SENS_ROWS = ["Ft", "M0", "M_dot", "angle_doubledot_max"]      # lmato_sens_t
 PARAM_ROWS = ["G", "M", "R0", "Ft", "M0", "M_dot", "fuel_mass", "angle_doubledot_max",
               "r_periapsis", "r_apoapsis", "final_time", "mass_scalar", "angle_ub", "u_bound"]
@@ -68,7 +71,7 @@ def build_library(force: bool = False, verbose: bool = False) -> str:
     every source; ``LAST_BUILD`` says which)."""
     import time as _time
     srcs = [os.path.join(CSRC, f) for f in ("ascent_cabi.cu", "ascent_ipm.cuh", "ascent_ipm_dc.cuh", "ascent_coop.cuh", "ascent_colloc.cuh",
-                                            "ascent_model.cuh", "ascent_result.cuh", "ascent_plan.h")]
+                                            "ascent_fly.cuh", "ascent_model.cuh", "ascent_result.cuh", "ascent_plan.h")]
     srcs.append(os.path.join(INCLUDE, "lmato_b200.h"))
     if not force and os.path.exists(LIB_PATH):
         if all(os.path.getmtime(LIB_PATH) >= os.path.getmtime(s) for s in srcs):
@@ -115,6 +118,7 @@ def lib() -> C.CDLL:
     L.lmato_measure_fp64_peak.argtypes = [vp, C.POINTER(C.c_double)]
     L.lmato_selftest_math.argtypes = [vp, C.POINTER(C.c_double)]
     L.lmato_coast_orbit.argtypes = [vp, vp, i64, C.c_double, C.c_double, i64, vp, vp]
+    L.lmato_fly_control.argtypes = [vp, vp, i64, vp, vp, i32, vp, vp, vp]
     L.lmato_set_sensitivity_output.argtypes = [vp, vp]
     L.lmato_set_initial_guess.argtypes = [vp, vp, vp]
     L.lmato_collocation_rule.argtypes = [i32, vp, vp]
@@ -126,7 +130,7 @@ def lib() -> C.CDLL:
     for name in ("lmato_create", "lmato_destroy", "lmato_set_options", "lmato_solve_batch",
                  "lmato_solve_batch_host", "lmato_workspace_bytes", "lmato_kernel_launches",
                  "lmato_last_kernel_ms", "lmato_measure_fp64_peak", "lmato_selftest_math", "lmato_coast_orbit",
-                 "lmato_set_sensitivity_output", "lmato_set_initial_guess", "lmato_multi_create", "lmato_multi_destroy",
+                 "lmato_fly_control", "lmato_set_sensitivity_output", "lmato_set_initial_guess", "lmato_multi_create", "lmato_multi_destroy",
                  "lmato_multi_set_options", "lmato_multi_device_count", "lmato_multi_solve_host", "lmato_collocation_rule"):
         getattr(L, name).restype = C.c_int
     _lib = L
@@ -136,7 +140,8 @@ def lib() -> C.CDLL:
 EXPORTED_SYMBOLS = ["lmato_default_options", "lmato_create", "lmato_destroy", "lmato_set_options",
                     "lmato_solve_batch", "lmato_solve_batch_host", "lmato_workspace_bytes",
                     "lmato_kernel_launches", "lmato_last_kernel_ms", "lmato_measure_fp64_peak",
-                    "lmato_selftest_math", "lmato_coast_orbit", "lmato_set_sensitivity_output", "lmato_set_initial_guess", "lmato_last_error",
+                    "lmato_selftest_math", "lmato_coast_orbit", "lmato_fly_control", "lmato_set_sensitivity_output",
+                    "lmato_set_initial_guess", "lmato_last_error",
                     "lmato_version", "lmato_multi_create", "lmato_multi_destroy", "lmato_multi_set_options",
                     "lmato_multi_device_count", "lmato_multi_solve_host", "lmato_collocation_rule"]
 

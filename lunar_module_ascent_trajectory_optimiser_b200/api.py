@@ -18,6 +18,7 @@ scaled units the reference's ``.value`` lists use.
     tf.value[0]                  (LO:178)       solution.tf
     y.value, x.value, ...        (LO:188-202)   solution.states["y"], ...  ([B, nt])
     failure -> Exception         (LO:177)       optimise(): raises; optimise_batch(): status[b]
+    (no counterpart)                            fly(): the solved control flown through LO:114-136
 
 Host code is Python; all numerical work happens in hand-written sm_100a CUDA kernels
 behind the C ABI of ``include/lmato_b200.h`` (ctypes).  PyTorch provides device memory,
@@ -344,6 +345,28 @@ class AscentSolver:
                         "lmato_coast_orbit")
         return {"r_min": out[0], "r_max": out[1], "final_state": out[2:6]}
 
+    def fly_control(self, rows: torch.Tensor, traj: torch.Tensor, tf: torch.Tensor,
+                    substeps: int, trajectories: bool = True) -> Dict[str, torch.Tensor]:
+        """``lmato_fly_control``: fly the MV row of ``traj`` ``[NVAR, nt, B]`` (a solve's output on this handle's mesh)
+        with final times ``tf`` ``[B]`` and parameters ``rows`` ``[NPARAM, B]`` through the continuous dynamics.  CUDA
+        float64 tensors on this solver's device; asynchronous on the current stream.  Returns ``"final"``
+        ``[NFLY, B]`` (rows ``_cabi.FLY_ROWS``) and ``"traj"`` ``[NVAR, nt, B]`` (None without ``trajectories``)."""
+        B = int(tf.shape[0]) if tf.dim() == 1 else -1
+        for name, t, shape in (("rows", rows, (_cabi.NPARAM, B)), ("traj", traj, (_cabi.NVAR, self.nt, B)),
+                               ("tf", tf, (B,))):
+            if t.device != self.device or t.dtype != torch.float64 or tuple(t.shape) != shape:
+                raise ValueError(f"{name} must be a float64 tensor of shape {shape} on {self.device}")
+        rows, traj, tf = rows.contiguous(), traj.contiguous(), tf.contiguous()
+        out = {"final": torch.empty((_cabi.NFLY, B), dtype=torch.float64, device=self.device),
+               "traj": torch.empty_like(traj) if trajectories else None}
+        ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p()
+        with torch.cuda.device(self.device):
+            stream = torch.cuda.current_stream(self.device).cuda_stream
+            _cabi.check(_cabi.lib().lmato_fly_control(self._h, ptr(rows), B, ptr(traj), ptr(tf), int(substeps),
+                                                      ptr(out["final"]), ptr(out["traj"]), C.c_void_p(stream)),
+                        "lmato_fly_control")
+        return out
+
     def selftest_math(self):
         e = (C.c_double * 5)()
         _cabi.check(_cabi.lib().lmato_selftest_math(self._h, e), "lmato_selftest_math")
@@ -583,6 +606,97 @@ def final_state_si(sol: AscentBatchSolution, params: AscentParams) -> torch.Tens
     S, R0 = rows[_cabi.PARAM_ROWS.index("r_periapsis")], rows[_cabi.PARAM_ROWS.index("R0")]
     st = sol.states
     return torch.stack([-st["x"][:, -1] * S, st["y"][:, -1] * S + R0, -st["xdot"][:, -1] * S, st["ydot"][:, -1] * S])
+
+
+# ---------------------------------------------------------------------------------------
+# post-solve flight: the solved control flown through the continuous dynamics
+# ---------------------------------------------------------------------------------------
+# Length of one RK4 sub-step in normalised time: 16 sub-steps per step of the reference's nt = 200 mesh.
+FLY_SUBSTEP = 1.0 / (16 * 199)
+
+
+def default_fly_substeps(time: torch.Tensor) -> int:
+    """RK4 sub-steps per mesh step that :func:`fly` takes by default: the smallest power of two that keeps every
+    sub-step of the mesh ``time`` no longer than ``FLY_SUBSTEP``.
+
+    On the reference mesh (nt = 200) that is 16: the smallest power of two for which multiplying the count by 4
+    changes the flown end state by less than 1e-10 relative (measured on the host build against the oracle fixtures:
+    16 -> 64 changes it by 1.4e-11, 8 -> 32 by 2.5e-10).  RK4's error is set by the sub-step length, so a coarser mesh
+    gets more sub-steps per step; on every fixture mesh (nt 20 ... 200, uniform and non-uniform, both models) the
+    count this gives changes the end state by at most 1.0e-11 when it is multiplied by 4
+    (``tests/test_fly_on_host.py``)."""
+    hmax = float(torch.diff(time.to(torch.float64).cpu()).max())
+    n = 1
+    while hmax > n * FLY_SUBSTEP * (1 + 1e-9):       # (a uniform mesh's steps differ from 1/(nt-1) by rounding)
+        n *= 2
+    return n
+
+
+@dataclasses.dataclass
+class FlownAscent:
+    """A solved control flown through the continuous dynamics (:func:`fly`).  ``B`` = 1 for an :class:`AscentSolution`."""
+    states: Dict[str, torch.Tensor]   # name -> [B, nt], the names of the solution's states, scaled units
+    final_state: Dict[str, torch.Tensor]   # y, ydot, x, xdot, angle, angledot, mass at tf -> [B], scaled
+    radius_miss_m: torch.Tensor       # [B] flown radius at tf minus the target radius R0 + r_periapsis (LO:161)
+    speed_miss_mps: torch.Tensor      # [B] flown speed at tf minus the target speed (LO:75, 169)
+    flight_path_angle_rad: torch.Tensor   # [B] asin(r.v / (|r| |v|)) at tf; the target is 0 (LO:173)
+    substeps: int                     # RK4 sub-steps per mesh step
+    S: torch.Tensor                   # [B] distance scale r_periapsis (LO:73)
+    R0: torch.Tensor                  # [B] lunar radius
+
+    def final_state_si(self) -> torch.Tensor:
+        """Flown insertion state in the frame of :func:`final_state_si`: ``[4, B]`` = (-x*S, y*S+R0, -xdot*S, ydot*S),
+        the start state :meth:`AscentSolver.coast_orbit` takes."""
+        f, S = self.final_state, self.S
+        return torch.stack([-f["x"] * S, f["y"] * S + self.R0, -f["xdot"] * S, f["ydot"] * S])
+
+
+def fly(solution: Union[AscentBatchSolution, AscentSolution], params: AscentParams,
+        substeps: Optional[int] = None) -> FlownAscent:
+    """Fly the solved control of ``solution`` through the continuous ascent dynamics (LO:114-136) on the GPU and
+    report each problem's insertion miss.
+
+    A solve returns the optimum of the transcribed problem; this shows how far the vehicle ends up from the target
+    orbit when it flies that control.  Classical RK4 with ``substeps`` sub-steps per mesh step (default:
+    :func:`default_fly_substeps`), the MV of node k held on (t_{k-1}, t_k] as both transcriptions hold it, so the
+    flight does not depend on NODES.  ``params`` are the solve's parameters.  ``solution`` needs its trajectories
+    and may live on the CPU or a GPU; the results follow its placement, as :func:`optimise_batch` does.  Problems that
+    did not converge are flown as given (check ``solution.status``)."""
+    if solution.control is None or not solution.states:
+        raise ValueError("fly() needs a solution with trajectories")
+    model = "circular" if solution.control_name == "angle" else "elliptical"
+    if params.model != model:
+        raise ValueError(f"params are of the {params.model} model, the solution of the {model} model")
+    single = isinstance(solution, AscentSolution)
+    expand = (lambda t: t.unsqueeze(0)) if single else (lambda t: t)
+    src = solution.control.device
+    dev = src if src.type == "cuda" else torch.device("cuda", torch.cuda.current_device())
+    solver = _get_solver(Mesh(time=solution.time.tolist()), SolverOptions(), dev, model)
+    control = expand(solution.control)
+    B, nt = int(control.shape[0]), int(control.shape[1])
+    if nt != solver.nt:
+        raise ValueError(f"the solution has {nt} nodes, its time grid {solver.nt}")
+    cols = []
+    for name in _cabi.VAR_ROWS:
+        if name == solution.control_name:
+            cols.append(control)
+        elif name in solution.states:
+            cols.append(expand(solution.states[name]))
+        else:
+            cols.append(torch.zeros_like(control))
+    traj = torch.stack([c.to(dev, torch.float64).transpose(0, 1) for c in cols])      # [NVAR, nt, B]
+    tf = torch.as_tensor(solution.tf, dtype=torch.float64).reshape(-1).to(dev)
+    rows = params.rows(B, device=dev)
+    n = default_fly_substeps(solution.time) if substeps is None else int(substeps)
+    out = solver.fly_control(rows, traj, tf, n)
+    if src.type != "cuda":
+        out = {k: v.cpu() for k, v in out.items()}
+        rows = rows.cpu()
+    fin = out["final"]
+    states = {name: out["traj"][i].transpose(0, 1) for i, name in enumerate(_cabi.VAR_ROWS) if name in solution.states}
+    return FlownAscent(states=states, final_state={n_: fin[i] for i, n_ in enumerate(_cabi.FLY_ROWS[:7])},
+                       radius_miss_m=fin[7], speed_miss_mps=fin[8], flight_path_angle_rad=fin[9], substeps=n,
+                       S=rows[_cabi.PARAM_ROWS.index("r_periapsis")], R0=rows[_cabi.PARAM_ROWS.index("R0")])
 
 
 # ---------------------------------------------------------------------------------------

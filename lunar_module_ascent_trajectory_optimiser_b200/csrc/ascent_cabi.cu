@@ -15,6 +15,8 @@
 // problems from a device-side queue and never returns to the host during a solve (barrier updates,
 // fraction-to-boundary, filter line search and convergence masks live in the owning lanes).  Tensor cores are
 // not used: the stage blocks are 8x8 FP64 and the recursion over stages is sequential (DESIGN.md).
+// Post-solve checks run one problem per thread: coast_orbit_kernel (the PDF's orbit coast) and fly_control_kernel (the
+// solved control flown through the continuous dynamics, ascent_fly.cuh).
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -25,6 +27,7 @@
 
 #include "../../include/lmato_b200.h"
 #include "ascent_colloc.cuh"
+#include "ascent_fly.cuh"
 #include "ascent_plan.h"
 #include "ascent_result.cuh"
 
@@ -352,6 +355,18 @@ __global__ void __launch_bounds__(128) coast_orbit_kernel(const double* __restri
   }
   out[0 * B + b] = sqrt(r2min); out[1 * B + b] = sqrt(r2max);
   out[2 * B + b] = x; out[3 * B + b] = y; out[4 * B + b] = vx; out[5 * B + b] = vy;
+}
+
+// Post-solve flight (ascent_fly.cuh): one problem per thread; every read and write of a [..][B] row is coalesced
+// across the warp's 32 problems.
+__global__ void __launch_bounds__(128) fly_control_kernel(const double* __restrict__ params, long B, int model,
+                                                          const double* __restrict__ tau, int nt,
+                                                          const double* __restrict__ traj, const double* __restrict__ tf,
+                                                          int substeps, double* __restrict__ fin, double* __restrict__ out) {
+  const long b = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const Params P = derive_params(params, B, b, model);
+  fly_one(P, model, tau, nt, traj, tf[b], substeps, B, b, fin, out);
 }
 
 // Self-test of the branch-free math against the CUDA library: max relative errors of
@@ -765,6 +780,19 @@ lmato_status_t lmato_coast_orbit(lmato_handle* h, const double* state, int64_t B
   CUDA_TRY(cudaSetDevice(h->device));
   cudaStream_t st = (cudaStream_t)stream;
   coast_orbit_kernel<<<(unsigned)((B + 127) / 128), 128, 0, st>>>(state, (long)B, gm, dt, (long)nsteps, out);
+  CUDA_TRY(cudaGetLastError());
+  h->launches += 1;
+  return LMATO_OK;
+}
+
+lmato_status_t lmato_fly_control(lmato_handle* h, const double* params, int64_t B, const double* traj,
+                                 const double* tf, int32_t substeps, double* out_final, double* out_traj, void* stream) {
+  if (!h || B < 0 || substeps < 1) { set_err("lmato_fly_control: bad argument"); return LMATO_ERR_INVALID; }
+  if (B == 0) return LMATO_OK;
+  if (!params || !traj || !tf || !out_final) { set_err("lmato_fly_control: NULL buffer"); return LMATO_ERR_INVALID; }
+  CUDA_TRY(cudaSetDevice(h->device));
+  fly_control_kernel<<<(unsigned)((B + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
+      params, (long)B, h->model, h->d_tau, h->nt, traj, tf, substeps, out_final, out_traj);
   CUDA_TRY(cudaGetLastError());
   h->launches += 1;
   return LMATO_OK;

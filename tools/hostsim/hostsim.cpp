@@ -16,6 +16,7 @@
 #include <random>
 #include <array>
 #include "ascent_colloc.cuh"
+#include "ascent_fly.cuh"
 #include "ascent_plan.h"
 #include "ascent_result.cuh"
 
@@ -344,4 +345,15 @@ extern "C" void hostsim_plan(int sm_count, int nt, int nodes, int model, int ker
   const int64_t v[10] = {p.kernel.kind, p.kernel.lanes, p.kernel.ctas_per_sm, p.kernel.move, p.grid, p.slots,
                          (int64_t)p.ws_bytes, (int64_t)p.alloc_bytes, p.warm, p.use_dc};
   for (int i = 0; i < 10; ++i) out[i] = v[i];
+}
+
+// The post-solve flight (csrc/ascent_fly.cuh) of one problem, as fly_control_kernel runs it: raw14 the parameter
+// column, model lmato_model_t, time the mesh (NULL = uniform), traj [10][nt] a solve's output, fin [LMATO_NFLY], out
+// [10][nt] or NULL.
+extern "C" void hostsim_fly(const double* raw14, int model, int nt, const double* time, const double* traj, double tf,
+                            int substeps, double* fin, double* out) {
+  std::vector<double> tau(nt);
+  for (int k = 0; k < nt; ++k) tau[k] = time ? time[k] : (double)k / (nt - 1);
+  const Params P = derive_params(raw14, 1, 0, model);
+  fly_one(P, model, tau.data(), nt, traj, tf, substeps, 1, 0, fin, out);
 }
