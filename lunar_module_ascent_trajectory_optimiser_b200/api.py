@@ -185,6 +185,26 @@ class AscentSolution:
     control_name: str = "angledoubledot"
 
 
+def _empty(shape, dtype: torch.dtype, device: Optional[torch.device]) -> torch.Tensor:
+    """A result array of a solve: on ``device``, or in pinned host memory when ``device`` is None."""
+    kw = dict(device=device) if device is not None else dict(pin_memory=True)
+    return torch.empty(shape, dtype=dtype, **kw)
+
+
+def alloc_outputs(nt: int, B: int, trajectories: bool = True,
+                  device: Optional[torch.device] = None) -> Dict[str, torch.Tensor]:
+    """The result arrays of a solve of ``B`` problems on an ``nt``-node mesh (the output layout of
+    ``include/lmato_b200.h``): on ``device``, or in pinned host memory when ``device`` is None."""
+    return {
+        "traj": _empty((_cabi.NVAR, nt, B), torch.float64, device) if trajectories else None,
+        "tf": _empty(B, torch.float64, device),
+        "final_mass": _empty(B, torch.float64, device),
+        "status": _empty(B, torch.int32, device),
+        "iterations": _empty(B, torch.int32, device),
+        "kkt": _empty(B, torch.float64, device),
+    }
+
+
 class AscentSolver:
     """Owns one C-ABI handle: one device, one mesh, one model."""
 
@@ -230,15 +250,7 @@ class AscentSolver:
     # -- raw entry points ---------------------------------------------------------------
     def alloc_outputs(self, B: int, trajectories: bool = True, on_device: bool = True) -> Dict[str, torch.Tensor]:
         """Result buffers for ``solve_rows(..., out=...)`` (device memory or pinned host memory)."""
-        kw = dict(device=self.device) if on_device else dict(pin_memory=True)
-        return {
-            "traj": torch.empty((_cabi.NVAR, self.nt, B), dtype=torch.float64, **kw) if trajectories else None,
-            "tf": torch.empty(B, dtype=torch.float64, **kw),
-            "final_mass": torch.empty(B, dtype=torch.float64, **kw),
-            "status": torch.empty(B, dtype=torch.int32, **kw),
-            "iterations": torch.empty(B, dtype=torch.int32, **kw),
-            "kkt": torch.empty(B, dtype=torch.float64, **kw),
-        }
+        return alloc_outputs(self.nt, B, trajectories, self.device if on_device else None)
 
     def solve_rows(self, rows: torch.Tensor, trajectories: bool = True,
                    out: Optional[Dict[str, torch.Tensor]] = None,
@@ -260,16 +272,16 @@ class AscentSolver:
         on_dev = rows.is_cuda
         if on_dev and rows.device != self.device:
             raise ValueError(f"rows live on {rows.device}, solver on {self.device}")
+        dev = self.device if on_dev else None
         if out is None:
-            out = self.alloc_outputs(B, trajectories, on_dev)
+            out = alloc_outputs(self.nt, B, trajectories, dev)
         else:
             if out["tf"].shape[0] != B or out["tf"].is_cuda != on_dev or (trajectories and out["traj"] is None):
                 raise ValueError("out buffers do not match this call (batch size / placement / trajectories)")
             if not trajectories:
                 out = dict(out, traj=None)
         if sensitivities:
-            kw = dict(device=self.device) if on_dev else dict(pin_memory=True)
-            out = dict(out, dtf=torch.empty((_cabi.NSENS, B), dtype=torch.float64, **kw))
+            out = dict(out, dtf=_empty((_cabi.NSENS, B), torch.float64, dev))
         if B == 0:
             return out
         ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p()
@@ -429,11 +441,7 @@ class AscentMultiSolver:
             raise ValueError("rows must be a CPU float64 tensor [NPARAM, B]")
         rows = rows.contiguous()
         B = int(rows.shape[1])
-        kw = dict(pin_memory=True)
-        out = {"traj": torch.empty((_cabi.NVAR, self.nt, B), dtype=torch.float64, **kw) if trajectories else None,
-               "tf": torch.empty(B, dtype=torch.float64, **kw), "final_mass": torch.empty(B, dtype=torch.float64, **kw),
-               "status": torch.empty(B, dtype=torch.int32, **kw), "iterations": torch.empty(B, dtype=torch.int32, **kw),
-               "kkt": torch.empty(B, dtype=torch.float64, **kw)}
+        out = alloc_outputs(self.nt, B, trajectories)
         if B == 0:
             return out
         ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p()

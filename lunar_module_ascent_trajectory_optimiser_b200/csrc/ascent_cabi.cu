@@ -400,16 +400,14 @@ struct lmato_handle {
   double* d_ws = nullptr;
   size_t ws_bytes = 0;
   int* d_counter = nullptr;
-  // staging for the host-buffer entry point
-  double* d_params = nullptr; size_t params_bytes = 0;
-  double* d_out = nullptr; size_t out_bytes = 0;
+  // the device copy of a host solve's arrays (stage_and_solve), for lmato_solve_batch_host and the device list
+  double* d_stage = nullptr; size_t stage_bytes = 0;
   double* d_ref = nullptr;        // reference column of the warm start: [REF_ROWS][nt]
   double* d_refparams = nullptr;  // [NPARAM] batch-mean parameters + scratch outputs of the reference solve
   lmato_options opt;
   double* sens_out = nullptr;     // optional extra output of the next solves (lmato_set_sensitivity_output)
   const double* guess_traj = nullptr;   // optional start point of the next solves (lmato_set_initial_guess)
   const double* guess_tf = nullptr;
-  double* d_guess = nullptr; size_t guess_bytes = 0;   // staging of a host guess
   int64_t launches = 0;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   cudaStream_t last_stream = nullptr;
@@ -537,7 +535,7 @@ lmato_status_t lmato_destroy(lmato_handle* h) {
   if (!h) return LMATO_OK;
   cudaSetDevice(h->device);
   cudaFree(h->d_h); cudaFree(h->d_tau); cudaFree(h->d_ws); cudaFree(h->d_counter);
-  cudaFree(h->d_params); cudaFree(h->d_out); cudaFree(h->d_ref); cudaFree(h->d_refparams); cudaFree(h->d_guess); cudaFree(h->d_coll);
+  cudaFree(h->d_stage); cudaFree(h->d_ref); cudaFree(h->d_refparams); cudaFree(h->d_coll);
   if (h->ev0) cudaEventDestroy(h->ev0);
   if (h->ev1) cudaEventDestroy(h->ev1);
   delete h;
@@ -589,38 +587,40 @@ static bool host_can_address(const void* p) {
   return attr.type != cudaMemoryTypeDevice;
 }
 
-// lmato_solve_batch for B problems that belong to a batch of warm_batch problems (ascent_plan.h, plan_solve).
-static lmato_status_t solve_batch(lmato_handle* h, const double* params, int64_t B, double* out_traj, double* out_tf,
-                                  double* out_final_mass, int32_t* out_status, int32_t* out_iters, double* out_kkt,
-                                  cudaStream_t st, int64_t warm_batch) {
-  if (!h) { set_err("lmato_solve_batch: NULL handle"); return LMATO_ERR_INVALID; }
-  if (B < 0) { set_err("lmato_solve_batch: negative batch"); return LMATO_ERR_INVALID; }
-  if (B == 0) return LMATO_OK;
-  if (!params || !out_tf || !out_final_mass || !out_status || !out_iters) {
-    set_err("lmato_solve_batch: NULL buffer");
+// The argument checks of every solve entry point (`fn` names it in the message).  An empty batch is valid.
+static lmato_status_t check_batch(const char* fn, const void* handle, const double* params, int64_t B,
+                                  const double* out_tf, const double* out_final_mass, const int32_t* out_status,
+                                  const int32_t* out_iters) {
+  if (!handle) { set_err("%s: NULL handle", fn); return LMATO_ERR_INVALID; }
+  if (B < 0) { set_err("%s: negative batch", fn); return LMATO_ERR_INVALID; }
+  if (B > 0 && (!params || !out_tf || !out_final_mass || !out_status || !out_iters)) {
+    set_err("%s: NULL buffer", fn);
     return LMATO_ERR_INVALID;
   }
-  CUDA_TRY(cudaSetDevice(h->device));
-  if (!kernel_can_address(h->sens_out) || !kernel_can_address(h->guess_traj) || !kernel_can_address(h->guess_tf)) {
-    set_err("lmato_solve_batch: the registered sensitivity output / start point is not device-addressable memory "
-            "(lmato_solve_batch takes DEVICE pointers; use lmato_solve_batch_host for host buffers)");
-    return LMATO_ERR_INVALID;
-  }
-  if (h->nodes > 2 && (h->sens_out || h->guess_traj)) {
+  return LMATO_OK;
+}
+
+// Solves the out.B > 0 problems of `params` into `out`, starting from guess_traj / guess_tf when they are given, on
+// h's device (the current one).  The problems belong to a batch of warm_batch problems (ascent_plan.h, plan_solve).
+// Every pointer is a device pointer.
+static lmato_status_t solve_batch(lmato_handle* h, const double* params, const double* guess_traj, const double* guess_tf,
+                                  const ResultOut& out, cudaStream_t st, int64_t warm_batch) {
+  if (h->nodes > 2 && (out.sens || guess_traj)) {
     set_err("lmato_solve_batch: sensitivities and caller-supplied start points are implemented for NODES = 2 only");
     return LMATO_ERR_UNSUPPORTED;
   }
   // Every solve on a handle shares its workspace, work-queue counter and warm-start reference.  A solve issued on
   // a different stream than the previous one first waits (on the device) for that one to finish.
   if (h->timed && st != h->last_stream) CUDA_TRY(cudaStreamWaitEvent(st, h->ev1, 0));
-  const LaunchPlan plan = plan_solve(h->sm_count, h->nt, h->nodes, h->model, h->opt, B, h->guess_traj != nullptr, warm_batch);
+  const int64_t B = out.B;
+  const LaunchPlan plan = plan_solve(h->sm_count, h->nt, h->nodes, h->model, h->opt, B, guess_traj != nullptr, warm_batch);
   if (plan.alloc_bytes > h->ws_bytes && h->timed) CUDA_TRY(cudaEventSynchronize(h->ev1));   // the previous solve may still be using it
   CUDA_TRY(grow(&h->d_ws, &h->ws_bytes, plan.alloc_bytes));
   CUDA_TRY(cudaMemsetAsync(h->d_counter, 0, sizeof(int), st));
   KArgs a;
   a.params = params;
-  a.res = ResultOut{out_traj, out_tf, out_final_mass, out_status, out_iters, out_kkt, h->sens_out, (long)B};
-  a.guess_traj = h->guess_traj; a.guess_tf = h->guess_tf;
+  a.res = out;
+  a.guess_traj = guess_traj; a.guess_tf = guess_tf;
   a.ws = h->d_ws; a.slots = plan.slots; a.N = h->nt - 1; a.h = h->d_h; a.tau = h->d_tau;
   a.counter = h->d_counter;
   a.model = h->model;
@@ -657,7 +657,16 @@ lmato_status_t lmato_solve_batch(lmato_handle* h, const double* params, int64_t 
                                  double* out_traj, double* out_tf, double* out_final_mass,
                                  int32_t* out_status, int32_t* out_iters, double* out_kkt,
                                  void* stream) {
-  return solve_batch(h, params, B, out_traj, out_tf, out_final_mass, out_status, out_iters, out_kkt,
+  const lmato_status_t rc = check_batch("lmato_solve_batch", h, params, B, out_tf, out_final_mass, out_status, out_iters);
+  if (rc != LMATO_OK || B == 0) return rc;
+  CUDA_TRY(cudaSetDevice(h->device));
+  if (!kernel_can_address(h->sens_out) || !kernel_can_address(h->guess_traj) || !kernel_can_address(h->guess_tf)) {
+    set_err("lmato_solve_batch: the registered sensitivity output / start point is not device-addressable memory "
+            "(lmato_solve_batch takes DEVICE pointers; use lmato_solve_batch_host for host buffers)");
+    return LMATO_ERR_INVALID;
+  }
+  return solve_batch(h, params, h->guess_traj, h->guess_tf,
+                     ResultOut{out_traj, out_tf, out_final_mass, out_status, out_iters, out_kkt, h->sens_out, (long)B},
                      (cudaStream_t)stream, B);
 }
 
@@ -683,68 +692,96 @@ static double* pinned_alias(double* host) {
   return static_cast<double*>(attr.devicePointer);
 }
 
+// The host arrays of one solve (include/lmato_b200.h), each a [rows][B] block: the inputs first, then the outputs.  A
+// shard of the batch is the columns [lo, lo + n) of every array.  An array the caller passes as NULL is absent.
+enum HostArrayId { kParams, kGuessTraj, kGuessTf, kTraj, kSens, kTf, kFinalMass, kKkt, kStatus, kIters, kHostArrays };
+constexpr int kHostInputs = kTraj;
+
+struct HostArray {
+  void* host;          // the caller's array, or NULL
+  size_t rows, elem;   // elem: bytes per element
+  void* dev;           // the shard's [rows][n] block that the solve reads or writes (set by stage_and_solve)
+};
+
+struct HostSolve {
+  HostArray a[kHostArrays];
+  int64_t B, lo, n;
+};
+
+static HostSolve host_solve(int nt, int64_t B, const double* params, const double* guess_traj, const double* guess_tf,
+                            double* traj, double* sens, double* tf, double* final_mass, double* kkt, int32_t* status,
+                            int32_t* iters) {
+  const size_t d = sizeof(double), i = sizeof(int32_t), nv = (size_t)LMATO_NVAR * nt;
+  return HostSolve{{{const_cast<double*>(params), LMATO_NPARAM, d}, {const_cast<double*>(guess_traj), nv, d},
+                    {const_cast<double*>(guess_tf), 1, d}, {traj, nv, d}, {sens, LMATO_NSENS, d}, {tf, 1, d},
+                    {final_mass, 1, d}, {kkt, 1, d}, {status, 1, i}, {iters, 1, i}},
+                   B, 0, 0};
+}
+
+// Copies the shard's columns of one array between the caller's block and the device.  The whole batch, or a single
+// row, is one contiguous run and takes one flat copy (the 1 GB of trajectories of a 65 536-problem solve among them);
+// the columns of a block of several rows take one 2D copy.
+static cudaError_t copy_columns(const HostSolve& s, const HostArray& a, cudaMemcpyKind kind, cudaStream_t st) {
+  char* host = static_cast<char*>(a.host) + a.elem * s.lo;
+  const size_t w = a.elem * s.n, pitch = a.elem * s.B;
+  const bool up = kind == cudaMemcpyHostToDevice;
+  if (s.n == s.B || a.rows == 1)
+    return up ? cudaMemcpyAsync(a.dev, host, w * a.rows, kind, st) : cudaMemcpyAsync(host, a.dev, w * a.rows, kind, st);
+  return up ? cudaMemcpy2DAsync(a.dev, w, host, pitch, w, a.rows, kind, st)
+            : cudaMemcpy2DAsync(host, pitch, a.dev, w, w, a.rows, kind, st);
+}
+
+// Carves h's staging buffer for the columns [lo, lo + n) of s, uploads their inputs and launches their solve on st
+// (h's device is the current one).  Nothing here waits for the device unless the staging buffer has to grow.
+// in_place: the shard is the whole batch, and a pinned trajectory array is written by the kernel directly.
+static lmato_status_t stage_and_solve(lmato_handle* h, HostSolve& s, int64_t lo, int64_t n, cudaStream_t st,
+                                      bool in_place) {
+  s.lo = lo; s.n = n;
+  // The trajectories are 16 KB per problem (1 GB for 65 536 problems).  If the caller's array is pinned the kernel
+  // can write them there directly, chunk by chunk as problems finish, so that the transfer over PCIe overlaps the
+  // solve.  The kernel writes rows of stride n, so only a whole batch can be written in place.
+  double* alias = in_place ? pinned_alias(static_cast<double*>(s.a[kTraj].host)) : nullptr;
+  if (alias) s.a[kTraj].host = nullptr;         // written in place: neither staged nor downloaded
+  // every array starts on a 256-byte boundary, as an allocation of its own would
+  auto room = [&](const HostArray& a) { return a.host ? (a.elem * a.rows * (size_t)n + 255) & ~(size_t)255 : 0; };
+  size_t bytes = 0;
+  for (const HostArray& a : s.a) bytes += room(a);
+  if (bytes > h->stage_bytes) CUDA_TRY(cudaStreamSynchronize(st));   // the previous call's copies may still use it
+  CUDA_TRY(grow(&h->d_stage, &h->stage_bytes, bytes));
+  char* p = reinterpret_cast<char*>(h->d_stage);
+  for (HostArray& a : s.a) { a.dev = a.host ? p : nullptr; p += room(a); }
+  if (alias) s.a[kTraj].dev = alias;
+  for (int i = 0; i < kHostInputs; ++i)
+    if (s.a[i].host) CUDA_TRY(copy_columns(s, s.a[i], cudaMemcpyHostToDevice, st));
+  auto dev = [&](int i) { return static_cast<double*>(s.a[i].dev); };
+  const ResultOut out{dev(kTraj), dev(kTf), dev(kFinalMass), static_cast<int*>(s.a[kStatus].dev),
+                      static_cast<int*>(s.a[kIters].dev), dev(kKkt), dev(kSens), (long)n};
+  return solve_batch(h, dev(kParams), dev(kGuessTraj), dev(kGuessTf), out, st, s.B);
+}
+
+// Queues the copies of the shard's outputs into the caller's arrays on st.  A copy into pageable memory returns only
+// when it is done, so a caller with several devices issues every launch before the first download.
+static lmato_status_t download(const HostSolve& s, cudaStream_t st) {
+  for (int i = kHostInputs; i < kHostArrays; ++i)
+    if (s.a[i].host) CUDA_TRY(copy_columns(s, s.a[i], cudaMemcpyDeviceToHost, st));
+  return LMATO_OK;
+}
+
 lmato_status_t lmato_solve_batch_host(lmato_handle* h, const double* params, int64_t B,
                                       double* out_traj, double* out_tf, double* out_final_mass,
                                       int32_t* out_status, int32_t* out_iters, double* out_kkt) {
-  if (!h) { set_err("lmato_solve_batch_host: NULL handle"); return LMATO_ERR_INVALID; }
-  if (B < 0) { set_err("lmato_solve_batch_host: negative batch"); return LMATO_ERR_INVALID; }
-  if (B == 0) return LMATO_OK;
-  if (!params || !out_tf || !out_final_mass || !out_status || !out_iters) {
-    set_err("lmato_solve_batch_host: NULL buffer");
-    return LMATO_ERR_INVALID;
-  }
+  lmato_status_t rc = check_batch("lmato_solve_batch_host", h, params, B, out_tf, out_final_mass, out_status, out_iters);
+  if (rc != LMATO_OK || B == 0) return rc;
   CUDA_TRY(cudaSetDevice(h->device));
-  const size_t pbytes = sizeof(double) * LMATO_NPARAM * (size_t)B;
-  CUDA_TRY(grow(&h->d_params, &h->params_bytes, pbytes));
-  // The per-node trajectories are 16 KB per problem (1 GB for 65 536 problems).  If the caller's
-  // buffer is pinned the kernel writes them there directly, chunk by chunk as problems finish, so the
-  // transfer over PCIe overlaps the solve; a pageable buffer is filled by a copy after the kernel.
-  double* traj_alias = pinned_alias(out_traj);
-  const size_t traj_n = out_traj ? (size_t)LMATO_NVAR * h->nt * (size_t)B : 0;
-  const size_t traj_stage = traj_alias ? 0 : traj_n;
   if (!host_can_address(h->sens_out) || !host_can_address(h->guess_traj) || !host_can_address(h->guess_tf)) {
     set_err("lmato_solve_batch_host: the registered sensitivity output / start point is device memory "
             "(lmato_solve_batch_host takes HOST pointers)");
     return LMATO_ERR_INVALID;
   }
-  double* sens_host = h->sens_out;       // for this entry point the registered pointer is a HOST buffer
-  const size_t sens_n = sens_host ? (size_t)LMATO_NSENS * (size_t)B : 0;
-  // layout of d_out: traj (only when staged) | sens | tf | fmass | kkt | status | iters
-  const size_t obytes = sizeof(double) * (traj_stage + sens_n + 3 * (size_t)B) + sizeof(int32_t) * 2 * (size_t)B;
-  CUDA_TRY(grow(&h->d_out, &h->out_bytes, obytes));
-  double* d_traj = out_traj ? (traj_alias ? traj_alias : h->d_out) : nullptr;
-  double* d_sens = sens_host ? h->d_out + traj_stage : nullptr;
-  double* d_tf = h->d_out + traj_stage + sens_n;
-  double* d_fm = d_tf + B;
-  double* d_kkt = d_fm + B;
-  int32_t* d_st = (int32_t*)(d_kkt + B);
-  int32_t* d_it = d_st + B;
+  HostSolve s = host_solve(h->nt, B, params, h->guess_traj, h->guess_tf, out_traj, h->sens_out, out_tf, out_final_mass,
+                           out_kkt, out_status, out_iters);
   cudaStream_t st = nullptr;
-  CUDA_TRY(cudaMemcpyAsync(h->d_params, params, pbytes, cudaMemcpyHostToDevice, st));
-  // a registered start point is a HOST buffer for this entry point: stage it
-  const double* guess_traj_host = h->guess_traj;
-  const double* guess_tf_host = h->guess_tf;
-  if (guess_traj_host) {
-    const size_t gn = (size_t)LMATO_NVAR * h->nt * (size_t)B;
-    const size_t gbytes = sizeof(double) * (gn + (size_t)B);
-    CUDA_TRY(grow(&h->d_guess, &h->guess_bytes, gbytes));
-    CUDA_TRY(cudaMemcpyAsync(h->d_guess, guess_traj_host, sizeof(double) * gn, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(h->d_guess + gn, guess_tf_host, sizeof(double) * (size_t)B, cudaMemcpyHostToDevice, st));
-    h->guess_traj = h->d_guess; h->guess_tf = h->d_guess + gn;
-  }
-  h->sens_out = d_sens;
-  lmato_status_t rc = lmato_solve_batch(h, h->d_params, B, d_traj, d_tf, d_fm, d_st, d_it, d_kkt, st);
-  h->sens_out = sens_host;
-  h->guess_traj = guess_traj_host; h->guess_tf = guess_tf_host;
-  if (rc != LMATO_OK) return rc;
-  if (sens_host) CUDA_TRY(cudaMemcpyAsync(sens_host, d_sens, sizeof(double) * sens_n, cudaMemcpyDeviceToHost, st));
-  if (out_traj && !traj_alias)
-    CUDA_TRY(cudaMemcpyAsync(out_traj, d_traj, sizeof(double) * traj_n, cudaMemcpyDeviceToHost, st));
-  CUDA_TRY(cudaMemcpyAsync(out_tf, d_tf, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
-  CUDA_TRY(cudaMemcpyAsync(out_final_mass, d_fm, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
-  if (out_kkt) CUDA_TRY(cudaMemcpyAsync(out_kkt, d_kkt, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
-  CUDA_TRY(cudaMemcpyAsync(out_status, d_st, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, st));
-  CUDA_TRY(cudaMemcpyAsync(out_iters, d_it, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, st));
+  if ((rc = stage_and_solve(h, s, 0, B, st, true)) != LMATO_OK || (rc = download(s, st)) != LMATO_OK) return rc;
   CUDA_TRY(cudaStreamSynchronize(st));
   return LMATO_OK;
 }
@@ -848,17 +885,14 @@ lmato_status_t lmato_measure_fp64_peak(lmato_handle* h, double* gflops) {
 
 // ---------------------------------------------------------------------------------------
 // device list: one host process, several GPUs (SURVEY 8b/8e).  Problem i goes to device floor(i*G/B)
-// (contiguous index ranges); every device solves its shard with its own handle, concurrently (all launches
-// are asynchronous), and writes its slice of the caller's HOST result arrays.  The problems are independent
-// and the results land on the host, so there is no collective to own here; the one-process-per-GPU path with
-// its single NCCL allgather is `sharded_solve` in the Python host layer.
+// (contiguous index ranges); every device solves its shard with its own handle, through that handle's staging
+// buffer, concurrently (all launches are asynchronous), and writes its slice of the caller's HOST result arrays.  The
+// problems are independent and the results land on the host, so there is no collective to own here; the
+// one-process-per-GPU path with its single NCCL allgather is `sharded_solve` in the Python host layer.
 // ---------------------------------------------------------------------------------------
 struct lmato_multi {
   std::vector<lmato_handle*> h;
   std::vector<cudaStream_t> st;
-  std::vector<double*> d_params;   // per device [NPARAM][Bshard]
-  std::vector<double*> d_out;      // per device: traj | tf | fmass | kkt | status | iters
-  std::vector<size_t> params_bytes, out_bytes;
 };
 
 lmato_status_t lmato_multi_destroy(lmato_multi* m) {
@@ -866,8 +900,6 @@ lmato_status_t lmato_multi_destroy(lmato_multi* m) {
   for (size_t g = 0; g < m->h.size(); ++g) {
     if (m->h[g]) cudaSetDevice(m->h[g]->device);
     if (g < m->st.size() && m->st[g]) cudaStreamDestroy(m->st[g]);
-    if (g < m->d_params.size()) cudaFree(m->d_params[g]);
-    if (g < m->d_out.size()) cudaFree(m->d_out[g]);
     lmato_destroy(m->h[g]);
   }
   delete m;
@@ -882,8 +914,6 @@ lmato_status_t lmato_multi_create(lmato_multi** out, const int32_t* devices, int
   lmato_multi* m = new (std::nothrow) lmato_multi();
   if (!m) { set_err("lmato_multi_create: out of host memory"); return LMATO_ERR_INVALID; }
   m->h.assign(ndev, nullptr); m->st.assign(ndev, nullptr);
-  m->d_params.assign(ndev, nullptr); m->d_out.assign(ndev, nullptr);
-  m->params_bytes.assign(ndev, 0); m->out_bytes.assign(ndev, 0);
   for (int g = 0; g < ndev; ++g) {
     lmato_status_t rc = lmato_create(&m->h[g], devices[g], nt, time, nodes, model);
     if (rc == LMATO_OK && (cudaSetDevice(devices[g]) != cudaSuccess ||
@@ -915,56 +945,25 @@ lmato_status_t lmato_multi_device_count(lmato_multi* m, int32_t* n) {
 lmato_status_t lmato_multi_solve_host(lmato_multi* m, const double* params, int64_t B,
                                       double* out_traj, double* out_tf, double* out_final_mass,
                                       int32_t* out_status, int32_t* out_iters, double* out_kkt) {
-  if (!m) { set_err("lmato_multi_solve_host: NULL handle"); return LMATO_ERR_INVALID; }
-  if (B < 0) { set_err("lmato_multi_solve_host: negative batch"); return LMATO_ERR_INVALID; }
-  if (B == 0) return LMATO_OK;
-  if (!params || !out_tf || !out_final_mass || !out_status || !out_iters) {
-    set_err("lmato_multi_solve_host: NULL buffer");
-    return LMATO_ERR_INVALID;
-  }
+  lmato_status_t rc = check_batch("lmato_multi_solve_host", m, params, B, out_tf, out_final_mass, out_status, out_iters);
+  if (rc != LMATO_OK || B == 0) return rc;
   const int G = (int)m->h.size();
-  const int nt = m->h[0]->nt;
-  struct Shard { int64_t lo, n; double *traj, *tf, *fm, *kkt; int32_t *st, *it; };
-  std::vector<Shard> sh(G);
-  // phase 1: every device gets its parameter columns and its launch (nothing here waits for a device)
+  std::vector<HostSolve> sh(G, host_solve(m->h[0]->nt, B, params, nullptr, nullptr, out_traj, nullptr, out_tf,
+                                          out_final_mass, out_kkt, out_status, out_iters));
+  // every device gets its columns and its launch before anything waits; the shards of one batch keep the batch warm
+  // start even when a shard alone is small (stage_and_solve passes the whole batch's size).  Every shard is staged,
+  // that of a one-device list too: on a B200 the kernel's stores into pinned memory made a one-device list 8 % faster
+  // on 65 536 problems at nt = 200 but 20 % slower on 4 096 problems at nt = 2001 than the copy after the solve.
   for (int g = 0; g < G; ++g) {
-    lmato_handle* h = m->h[g];
-    Shard& s = sh[g];
-    s.lo = (B * g) / G;
-    s.n = (B * (g + 1)) / G - s.lo;
-    if (s.n == 0) continue;
-    CUDA_TRY(cudaSetDevice(h->device));
-    const size_t pbytes = sizeof(double) * LMATO_NPARAM * (size_t)s.n;
-    const size_t traj_n = out_traj ? (size_t)LMATO_NVAR * nt * (size_t)s.n : 0;
-    const size_t obytes = sizeof(double) * (traj_n + 3 * (size_t)s.n) + sizeof(int32_t) * 2 * (size_t)s.n;
-    // the previous solve on this stream may still be using the buffers
-    if (pbytes > m->params_bytes[g] || obytes > m->out_bytes[g]) CUDA_TRY(cudaStreamSynchronize(m->st[g]));
-    CUDA_TRY(grow(&m->d_params[g], &m->params_bytes[g], pbytes));
-    CUDA_TRY(grow(&m->d_out[g], &m->out_bytes[g], obytes));
-    s.traj = out_traj ? m->d_out[g] : nullptr;
-    s.tf = m->d_out[g] + traj_n; s.fm = s.tf + s.n; s.kkt = s.fm + s.n;
-    s.st = (int32_t*)(s.kkt + s.n); s.it = s.st + s.n;
-    // columns [lo, lo+n) of the row-major [NPARAM][B] block
-    CUDA_TRY(cudaMemcpy2DAsync(m->d_params[g], sizeof(double) * s.n, params + s.lo, sizeof(double) * B,
-                               sizeof(double) * s.n, LMATO_NPARAM, cudaMemcpyHostToDevice, m->st[g]));
-    // the shards of one batch keep the batch warm start even when a shard alone is small
-    const lmato_status_t rc = solve_batch(h, m->d_params[g], s.n, s.traj, s.tf, s.fm, s.st, s.it, s.kkt, m->st[g], B);
-    if (rc != LMATO_OK) return rc;
-  }
-  // phase 2: every device writes its slice of the host arrays
-  for (int g = 0; g < G; ++g) {
-    const Shard& s = sh[g];
-    if (s.n == 0) continue;
+    const int64_t lo = (B * g) / G, n = (B * (g + 1)) / G - lo;
+    if (n == 0) continue;                      // (sh[g].n stays 0: the later loops skip it)
     CUDA_TRY(cudaSetDevice(m->h[g]->device));
-    cudaStream_t st = m->st[g];
-    if (out_traj)
-      CUDA_TRY(cudaMemcpy2DAsync(out_traj + s.lo, sizeof(double) * B, s.traj, sizeof(double) * s.n, sizeof(double) * s.n,
-                                 (size_t)LMATO_NVAR * nt, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaMemcpyAsync(out_tf + s.lo, s.tf, sizeof(double) * s.n, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaMemcpyAsync(out_final_mass + s.lo, s.fm, sizeof(double) * s.n, cudaMemcpyDeviceToHost, st));
-    if (out_kkt) CUDA_TRY(cudaMemcpyAsync(out_kkt + s.lo, s.kkt, sizeof(double) * s.n, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaMemcpyAsync(out_status + s.lo, s.st, sizeof(int32_t) * s.n, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaMemcpyAsync(out_iters + s.lo, s.it, sizeof(int32_t) * s.n, cudaMemcpyDeviceToHost, st));
+    if ((rc = stage_and_solve(m->h[g], sh[g], lo, n, m->st[g], false)) != LMATO_OK) return rc;
+  }
+  for (int g = 0; g < G; ++g) {
+    if (sh[g].n == 0) continue;
+    CUDA_TRY(cudaSetDevice(m->h[g]->device));
+    if ((rc = download(sh[g], m->st[g])) != LMATO_OK) return rc;
   }
   for (int g = 0; g < G; ++g) {
     if (sh[g].n == 0) continue;

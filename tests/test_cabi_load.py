@@ -76,7 +76,13 @@ def test_argument_validation_without_gpu(built_lib):
     assert L.lmato_create(C.byref(h), 0, 200, None, 3, 1) == 4        # NODES >= 3 with the circular model: unsupported
     assert L.lmato_create(C.byref(h), 0, 200, None, 2, 7) == 1        # unknown model
     assert L.lmato_solve_batch(None, None, 1, None, None, None, None, None, None, None) == 1
+    assert L.lmato_solve_batch_host(None, None, 1, None, None, None, None, None, None) == 1
+    assert L.lmato_multi_solve_host(None, None, 1, None, None, None, None, None, None) == 1
+    assert b"lmato_multi_solve_host: NULL handle" in L.lmato_last_error()
     assert L.lmato_destroy(None) == 0
+    if not torch.cuda.is_available():
+        m = C.c_void_p()
+        assert L.lmato_multi_create(C.byref(m), (C.c_int32 * 1)(0), 1, 200, None, 2, 0) == 3 and not m.value   # LMATO_ERR_NO_DEVICE
 
 
 def test_product_does_not_import_oracle():
