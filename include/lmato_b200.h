@@ -218,6 +218,19 @@ typedef enum lmato_sens {
 } lmato_sens_t;
 lmato_status_t lmato_set_sensitivity_output(lmato_handle* h, double* out_dtf);
 
+/* d tf / d params[p] for every row p of the params block:  out_dtf_dp [LMATO_NPARAM][B], row p = LMATO_P_*.
+ * Registered, switched off (NULL), addressed and checked like lmato_set_sensitivity_output (a DEVICE
+ * pointer for lmato_solve_batch, a HOST pointer for lmato_solve_batch_host; entries of problems that did not
+ * converge are meaningless), and independent of it: either output, both or neither may be registered, and
+ * registering this one changes no bit of any other output.  Its rows Ft, M0, M_dot and angle_doubledot_max are the
+ * values of lmato_set_sensitivity_output, bit for bit.  Each entry is the partial derivative with respect to that
+ * one row, the other rows held: tf in the reference's scaled units (0..1) per unit of the raw row, from the same
+ * envelope-theorem pass over the converged iterate, i.e. the derivative of the whole objective (with the move term
+ * when DCOST > 0) divided by obj_scale.  r_periapsis is both the target perilune and the distance scale of the
+ * scaled dynamics; its row covers both roles.  For LMATO_MODEL_CIRCULAR the rows angle_doubledot_max and u_bound
+ * are NaN: that model reads neither.  NODES >= 3: the solve answers LMATO_ERR_UNSUPPORTED while it is registered. */
+lmato_status_t lmato_set_param_sensitivity_output(lmato_handle* h, double* out_dtf_dp);
+
 /* The collocation rule used for NODES = 2..6 (host only, no GPU needed): tau[NODES-1] = the non-initial Lobatto
  * points on (0,1], N[(NODES-1)^2] row-major with  h N f_{1..} = z_{1..} - z_0  (SURVEY Appendix B.2). */
 lmato_status_t lmato_collocation_rule(int32_t nodes, double* tau, double* N);

@@ -120,6 +120,7 @@ def lib() -> C.CDLL:
     L.lmato_coast_orbit.argtypes = [vp, vp, i64, C.c_double, C.c_double, i64, vp, vp]
     L.lmato_fly_control.argtypes = [vp, vp, i64, vp, vp, i32, vp, vp, vp]
     L.lmato_set_sensitivity_output.argtypes = [vp, vp]
+    L.lmato_set_param_sensitivity_output.argtypes = [vp, vp]
     L.lmato_set_initial_guess.argtypes = [vp, vp, vp]
     L.lmato_collocation_rule.argtypes = [i32, vp, vp]
     L.lmato_multi_create.argtypes = [C.POINTER(vp), C.POINTER(i32), i32, i32, vp, i32, i32]
@@ -130,7 +131,8 @@ def lib() -> C.CDLL:
     for name in ("lmato_create", "lmato_destroy", "lmato_set_options", "lmato_solve_batch",
                  "lmato_solve_batch_host", "lmato_workspace_bytes", "lmato_kernel_launches",
                  "lmato_last_kernel_ms", "lmato_measure_fp64_peak", "lmato_selftest_math", "lmato_coast_orbit",
-                 "lmato_fly_control", "lmato_set_sensitivity_output", "lmato_set_initial_guess", "lmato_multi_create", "lmato_multi_destroy",
+                 "lmato_fly_control", "lmato_set_sensitivity_output", "lmato_set_param_sensitivity_output",
+                 "lmato_set_initial_guess", "lmato_multi_create", "lmato_multi_destroy",
                  "lmato_multi_set_options", "lmato_multi_device_count", "lmato_multi_solve_host", "lmato_collocation_rule"):
         getattr(L, name).restype = C.c_int
     _lib = L
@@ -141,6 +143,7 @@ EXPORTED_SYMBOLS = ["lmato_default_options", "lmato_create", "lmato_destroy", "l
                     "lmato_solve_batch", "lmato_solve_batch_host", "lmato_workspace_bytes",
                     "lmato_kernel_launches", "lmato_last_kernel_ms", "lmato_measure_fp64_peak",
                     "lmato_selftest_math", "lmato_coast_orbit", "lmato_fly_control", "lmato_set_sensitivity_output",
+                    "lmato_set_param_sensitivity_output",
                     "lmato_set_initial_guess", "lmato_last_error",
                     "lmato_version", "lmato_multi_create", "lmato_multi_destroy", "lmato_multi_set_options",
                     "lmato_multi_device_count", "lmato_multi_solve_host", "lmato_collocation_rule"]

@@ -156,9 +156,14 @@ class AscentBatchSolution:
     kkt_error: torch.Tensor          # [B]
     time: torch.Tensor               # [nt] normalised mesh (m.time)
     # optional: d tf / d parameter, name -> [B] (scaled tf per unit of the raw parameter), for
-    # Ft, M0, M_dot, angle_doubledot_max (NaN for the circular model, which has no such limit); only with
-    # ``sensitivities=True``
+    # Ft, M0, M_dot, angle_doubledot_max (NaN for the circular model, which has no such limit) with
+    # ``sensitivities=True``, for every name of PARAM_ROWS with ``sensitivities="all"`` (the circular model: NaN for
+    # angle_doubledot_max and u_bound, which it does not read).  Partial derivatives: one row of the parameter block
+    # moves, the others stay (see optimise_batch).
     dtf_dparam: Optional[Dict[str, torch.Tensor]] = None
+    # optional, ``sensitivities="all"`` only: d final_mass / d parameter, name -> [B] (kg per unit of the raw
+    # parameter), the partial derivatives of final_mass = M0 - M_dot * final_time * tf
+    dfinal_mass_dparam: Optional[Dict[str, torch.Tensor]] = None
     # which reference variable `control` is: the MV `angledoubledot` (LO:96) or, for the circular model, the MV
     # `angle` (PDF p.27 src 69-73)
     control_name: str = "angledoubledot"
@@ -254,17 +259,20 @@ class AscentSolver:
 
     def solve_rows(self, rows: torch.Tensor, trajectories: bool = True,
                    out: Optional[Dict[str, torch.Tensor]] = None,
-                   sensitivities: bool = False,
+                   sensitivities: Union[bool, str] = False,
                    guess: Optional[Dict[str, torch.Tensor]] = None) -> Dict[str, torch.Tensor]:
         """``rows``: ``[NPARAM, B]`` float64.  CUDA tensor -> device entry point, results stay on
         the device (asynchronous on the current stream).  CPU tensor -> host entry point
         (H2D + solve + D2H, synchronous), results in pinned host memory.  ``out``: buffers from
         :meth:`alloc_outputs` to write into (avoids re-allocating ~1 GB of trajectories per call).
         ``sensitivities``: also return ``"dtf"`` ``[NSENS, B]`` = d tf / d (Ft, M0, M_dot,
-        angle_doubledot_max) from the multipliers at the solution (``lmato_set_sensitivity_output``).
+        angle_doubledot_max) from the multipliers at the solution (``lmato_set_sensitivity_output``);
+        ``sensitivities="all"``: instead ``"dtf_all"`` ``[NPARAM, B]`` = d tf / d every row of ``rows``
+        (``lmato_set_param_sensitivity_output``).
         ``guess``: ``{"traj": [NVAR, nt, B], "tf": [B]}`` (e.g. a previous result of this method, same
         placement as ``rows``) to start from instead of the built-in start (``lmato_set_initial_guess``)."""
         L = _cabi.lib()
+        sens_key = _sens_key(sensitivities)
         if rows.dtype != torch.float64 or rows.dim() != 2 or rows.shape[0] != _cabi.NPARAM:
             raise ValueError("rows must be float64 [NPARAM, B]")
         rows = rows.contiguous()
@@ -280,8 +288,8 @@ class AscentSolver:
                 raise ValueError("out buffers do not match this call (batch size / placement / trajectories)")
             if not trajectories:
                 out = dict(out, traj=None)
-        if sensitivities:
-            out = dict(out, dtf=_empty((_cabi.NSENS, B), torch.float64, dev))
+        if sens_key is not None:
+            out = dict(out, **{sens_key: _empty((_SENS_OUT[sens_key][0], B), torch.float64, dev)})
         if B == 0:
             return out
         ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p()
@@ -292,15 +300,16 @@ class AscentSolver:
                 raise ValueError("guess must be {'traj': float64 [NVAR, nt, B], 'tf': float64 [B]} placed like rows")
             gt, gf = gt.contiguous(), gf.contiguous()
             _cabi.check(L.lmato_set_initial_guess(self._h, ptr(gt), ptr(gf)), "lmato_set_initial_guess")
-        if sensitivities:
-            _cabi.check(L.lmato_set_sensitivity_output(self._h, ptr(out["dtf"])), "lmato_set_sensitivity_output")
+        if sens_key is not None:
+            fn = _SENS_OUT[sens_key][1]
+            _cabi.check(getattr(L, fn)(self._h, ptr(out[sens_key])), fn)
         try:
             self._solve_call(L, rows, B, out, on_dev, ptr)
             if guess is not None and on_dev:
                 torch.cuda.current_stream(self.device).synchronize()    # the guess buffers may be temporaries
         finally:
-            if sensitivities:
-                L.lmato_set_sensitivity_output(self._h, C.c_void_p())
+            if sens_key is not None:
+                getattr(L, _SENS_OUT[sens_key][1])(self._h, C.c_void_p())
             if guess is not None:
                 L.lmato_set_initial_guess(self._h, C.c_void_p(), C.c_void_p())
         return out
@@ -462,6 +471,31 @@ def _c_options(o: SolverOptions) -> "_cabi.LmatoOptions":
                               rtol=float(o.rtol))
 
 
+# the key of a solve_rows result and the C entry that registers it, per `sensitivities` setting
+_SENS_OUT = {"dtf": (_cabi.NSENS, "lmato_set_sensitivity_output"),
+             "dtf_all": (_cabi.NPARAM, "lmato_set_param_sensitivity_output")}
+
+
+def _sens_key(sensitivities: Union[bool, str]) -> Optional[str]:
+    if isinstance(sensitivities, str) and sensitivities != "all":
+        raise ValueError(f"sensitivities must be False, True or 'all', not {sensitivities!r}")
+    return "dtf_all" if sensitivities == "all" else "dtf" if sensitivities else None
+
+
+def dfinal_mass_dparam(dtf: torch.Tensor, rows: torch.Tensor, tf: torch.Tensor) -> torch.Tensor:
+    """``[NPARAM, B]`` partial derivatives of final_mass = M0 - M_dot * final_time * tf (the library's output,
+    LO:123) with respect to every row of the parameter block, from ``dtf`` = d tf / d row (``[NPARAM, B]``)."""
+    rows = rows.to(dtf.device)
+    tf = tf.to(dtf.device)
+    i = _cabi.PARAM_ROWS.index
+    mdot, T = rows[i("M_dot")], rows[i("final_time")]
+    out = -(mdot * T) * dtf
+    out[i("M0")] += 1.0
+    out[i("M_dot")] -= T * tf
+    out[i("final_time")] -= mdot * tf
+    return out
+
+
 def package_solution(raw: Dict[str, torch.Tensor], rows: torch.Tensor, time: torch.Tensor,
                      model: str = "elliptical") -> AscentBatchSolution:
     traj = raw["traj"]
@@ -478,11 +512,18 @@ def package_solution(raw: Dict[str, torch.Tensor], rows: torch.Tensor, time: tor
         else:
             control = states.pop("angledoubledot")
     T = rows[_cabi.PARAM_ROWS.index("final_time")]
-    dtf = raw.get("dtf")
+    dtf, dtf_all = raw.get("dtf"), raw.get("dtf_all")
+    dtf_dparam = dfm_dparam = None
+    if dtf is not None:
+        dtf_dparam = {n: dtf[i] for i, n in enumerate(_cabi.SENS_ROWS)}
+    elif dtf_all is not None:
+        dtf_dparam = {n: dtf_all[i] for i, n in enumerate(_cabi.PARAM_ROWS)}
+        dfm = dfinal_mass_dparam(dtf_all, rows, raw["tf"])
+        dfm_dparam = {n: dfm[i] for i, n in enumerate(_cabi.PARAM_ROWS)}
     return AscentBatchSolution(tf=raw["tf"], tf_seconds=raw["tf"] * T.to(raw["tf"].device), states=states,
                                control=control, final_mass=raw["final_mass"], status=raw["status"],
                                iterations=raw["iterations"], kkt_error=raw["kkt"], time=time,
-                               dtf_dparam=None if dtf is None else {n: dtf[i] for i, n in enumerate(_cabi.SENS_ROWS)},
+                               dtf_dparam=dtf_dparam, dfinal_mass_dparam=dfm_dparam,
                                control_name="angle" if model == "circular" else "angledoubledot")
 
 
@@ -553,7 +594,7 @@ def sharded_solve(rows: torch.Tensor, solve_fn: Callable[[torch.Tensor], Dict[st
 
 def multi_device_solve(rows: torch.Tensor, solvers: List["AscentSolver"], trajectories: bool = True,
                        out_device: Union[str, torch.device, None] = None,
-                       sensitivities: bool = False) -> Dict[str, torch.Tensor]:
+                       sensitivities: Union[bool, str] = False) -> Dict[str, torch.Tensor]:
     """One host process, several GPUs (no torchrun): problem i goes to GPU ``floor(i*G/B)`` (the same
     contiguous index partition as :func:`sharded_solve`).  The device entry point is asynchronous, so
     all launches are issued first and every GPU solves its shard concurrently; the shards are then
@@ -730,7 +771,7 @@ def _get_solver(mesh: Mesh, options: SolverOptions, device, model: str) -> Ascen
 def optimise_batch(params: AscentParams, mesh: Optional[Mesh] = None,
                    options: Optional[SolverOptions] = None, device=None, batch: Optional[int] = None,
                    trajectories: bool = True, group=None,
-                   devices: Optional[Sequence[int]] = None, sensitivities: bool = False,
+                   devices: Optional[Sequence[int]] = None, sensitivities: Union[bool, str] = False,
                    guess: Optional[AscentBatchSolution] = None) -> AscentBatchSolution:
     """Solve a batch of ascent problems (one per entry of the ``[B]`` parameter tensors).
 
@@ -746,7 +787,13 @@ def optimise_batch(params: AscentParams, mesh: Optional[Mesh] = None,
     collective: the shards are copied into one result block, see :func:`multi_device_solve`).
 
     ``sensitivities``: also return ``dtf_dparam`` (d tf / d Ft, M0, M_dot, angle_doubledot_max per
-    problem; SURVEY 8f.4).  Not available together with ``group``.
+    problem; SURVEY 8f.4).  ``sensitivities="all"``: ``dtf_dparam`` for every name of ``PARAM_ROWS`` and
+    ``dfinal_mass_dparam`` (d final_mass / d the same rows).  Not available together with ``group``.
+    These are partial derivatives with respect to rows of the parameter block (``params.rows()``), each row moved
+    with the others held.  Where a field of ``params`` sets more than one row, the total derivative is the sum over
+    those rows: ``mass_scalar=None`` follows ``fuel_mass``, so the derivative with respect to the reference's tied
+    fuel mass is ``dtf_dparam["fuel_mass"] + dtf_dparam["mass_scalar"]``; with ``Isp`` given, ``M_dot`` is derived
+    from ``Ft`` and ``Isp`` and the ``Ft`` row holds thrust at fixed ``M_dot``.
 
     ``guess``: a previous :class:`AscentBatchSolution` of the same batch size and mesh (elliptical
     model) to start from -- the counterpart of the ``value=`` arguments at LO:39, 83-96.  Single
@@ -754,6 +801,7 @@ def optimise_batch(params: AscentParams, mesh: Optional[Mesh] = None,
     """
     mesh = mesh or Mesh()
     options = options or SolverOptions()
+    _sens_key(sensitivities)
     if options.dcost is None:          # the move-suppression weight travels with the model parameters
         options = dataclasses.replace(options, dcost=float(params.dcost))
     on_dev = any(isinstance(getattr(params, f.name), torch.Tensor) and getattr(params, f.name).is_cuda

@@ -406,6 +406,7 @@ struct lmato_handle {
   double* d_refparams = nullptr;  // [NPARAM] batch-mean parameters + scratch outputs of the reference solve
   lmato_options opt;
   double* sens_out = nullptr;     // optional extra output of the next solves (lmato_set_sensitivity_output)
+  double* psens_out = nullptr;    // another one (lmato_set_param_sensitivity_output)
   const double* guess_traj = nullptr;   // optional start point of the next solves (lmato_set_initial_guess)
   const double* guess_tf = nullptr;
   int64_t launches = 0;
@@ -605,7 +606,7 @@ static lmato_status_t check_batch(const char* fn, const void* handle, const doub
 // Every pointer is a device pointer.
 static lmato_status_t solve_batch(lmato_handle* h, const double* params, const double* guess_traj, const double* guess_tf,
                                   const ResultOut& out, cudaStream_t st, int64_t warm_batch) {
-  if (h->nodes > 2 && (out.sens || guess_traj)) {
+  if (h->nodes > 2 && (out.sens || out.psens || guess_traj)) {
     set_err("lmato_solve_batch: sensitivities and caller-supplied start points are implemented for NODES = 2 only");
     return LMATO_ERR_UNSUPPORTED;
   }
@@ -620,6 +621,7 @@ static lmato_status_t solve_batch(lmato_handle* h, const double* params, const d
   KArgs a;
   a.params = params;
   a.res = out;
+  a.res.params = params;
   a.guess_traj = guess_traj; a.guess_tf = guess_tf;
   a.ws = h->d_ws; a.slots = plan.slots; a.N = h->nt - 1; a.h = h->d_h; a.tau = h->d_tau;
   a.counter = h->d_counter;
@@ -660,13 +662,15 @@ lmato_status_t lmato_solve_batch(lmato_handle* h, const double* params, int64_t 
   const lmato_status_t rc = check_batch("lmato_solve_batch", h, params, B, out_tf, out_final_mass, out_status, out_iters);
   if (rc != LMATO_OK || B == 0) return rc;
   CUDA_TRY(cudaSetDevice(h->device));
-  if (!kernel_can_address(h->sens_out) || !kernel_can_address(h->guess_traj) || !kernel_can_address(h->guess_tf)) {
+  if (!kernel_can_address(h->sens_out) || !kernel_can_address(h->psens_out) || !kernel_can_address(h->guess_traj) ||
+      !kernel_can_address(h->guess_tf)) {
     set_err("lmato_solve_batch: the registered sensitivity output / start point is not device-addressable memory "
             "(lmato_solve_batch takes DEVICE pointers; use lmato_solve_batch_host for host buffers)");
     return LMATO_ERR_INVALID;
   }
   return solve_batch(h, params, h->guess_traj, h->guess_tf,
-                     ResultOut{out_traj, out_tf, out_final_mass, out_status, out_iters, out_kkt, h->sens_out, (long)B},
+                     ResultOut{out_traj, out_tf, out_final_mass, out_status, out_iters, out_kkt, h->sens_out, (long)B,
+                               h->psens_out},
                      (cudaStream_t)stream, B);
 }
 
@@ -694,7 +698,7 @@ static double* pinned_alias(double* host) {
 
 // The host arrays of one solve (include/lmato_b200.h), each a [rows][B] block: the inputs first, then the outputs.  A
 // shard of the batch is the columns [lo, lo + n) of every array.  An array the caller passes as NULL is absent.
-enum HostArrayId { kParams, kGuessTraj, kGuessTf, kTraj, kSens, kTf, kFinalMass, kKkt, kStatus, kIters, kHostArrays };
+enum HostArrayId { kParams, kGuessTraj, kGuessTf, kTraj, kSens, kPsens, kTf, kFinalMass, kKkt, kStatus, kIters, kHostArrays };
 constexpr int kHostInputs = kTraj;
 
 struct HostArray {
@@ -709,11 +713,12 @@ struct HostSolve {
 };
 
 static HostSolve host_solve(int nt, int64_t B, const double* params, const double* guess_traj, const double* guess_tf,
-                            double* traj, double* sens, double* tf, double* final_mass, double* kkt, int32_t* status,
-                            int32_t* iters) {
+                            double* traj, double* sens, double* psens, double* tf, double* final_mass, double* kkt,
+                            int32_t* status, int32_t* iters) {
   const size_t d = sizeof(double), i = sizeof(int32_t), nv = (size_t)LMATO_NVAR * nt;
   return HostSolve{{{const_cast<double*>(params), LMATO_NPARAM, d}, {const_cast<double*>(guess_traj), nv, d},
-                    {const_cast<double*>(guess_tf), 1, d}, {traj, nv, d}, {sens, LMATO_NSENS, d}, {tf, 1, d},
+                    {const_cast<double*>(guess_tf), 1, d}, {traj, nv, d}, {sens, LMATO_NSENS, d},
+                    {psens, LMATO_NPARAM, d}, {tf, 1, d},
                     {final_mass, 1, d}, {kkt, 1, d}, {status, 1, i}, {iters, 1, i}},
                    B, 0, 0};
 }
@@ -755,7 +760,7 @@ static lmato_status_t stage_and_solve(lmato_handle* h, HostSolve& s, int64_t lo,
     if (s.a[i].host) CUDA_TRY(copy_columns(s, s.a[i], cudaMemcpyHostToDevice, st));
   auto dev = [&](int i) { return static_cast<double*>(s.a[i].dev); };
   const ResultOut out{dev(kTraj), dev(kTf), dev(kFinalMass), static_cast<int*>(s.a[kStatus].dev),
-                      static_cast<int*>(s.a[kIters].dev), dev(kKkt), dev(kSens), (long)n};
+                      static_cast<int*>(s.a[kIters].dev), dev(kKkt), dev(kSens), (long)n, dev(kPsens)};
   return solve_batch(h, dev(kParams), dev(kGuessTraj), dev(kGuessTf), out, st, s.B);
 }
 
@@ -773,13 +778,14 @@ lmato_status_t lmato_solve_batch_host(lmato_handle* h, const double* params, int
   lmato_status_t rc = check_batch("lmato_solve_batch_host", h, params, B, out_tf, out_final_mass, out_status, out_iters);
   if (rc != LMATO_OK || B == 0) return rc;
   CUDA_TRY(cudaSetDevice(h->device));
-  if (!host_can_address(h->sens_out) || !host_can_address(h->guess_traj) || !host_can_address(h->guess_tf)) {
+  if (!host_can_address(h->sens_out) || !host_can_address(h->psens_out) || !host_can_address(h->guess_traj) ||
+      !host_can_address(h->guess_tf)) {
     set_err("lmato_solve_batch_host: the registered sensitivity output / start point is device memory "
             "(lmato_solve_batch_host takes HOST pointers)");
     return LMATO_ERR_INVALID;
   }
-  HostSolve s = host_solve(h->nt, B, params, h->guess_traj, h->guess_tf, out_traj, h->sens_out, out_tf, out_final_mass,
-                           out_kkt, out_status, out_iters);
+  HostSolve s = host_solve(h->nt, B, params, h->guess_traj, h->guess_tf, out_traj, h->sens_out, h->psens_out, out_tf,
+                           out_final_mass, out_kkt, out_status, out_iters);
   cudaStream_t st = nullptr;
   if ((rc = stage_and_solve(h, s, 0, B, st, true)) != LMATO_OK || (rc = download(s, st)) != LMATO_OK) return rc;
   CUDA_TRY(cudaStreamSynchronize(st));
@@ -806,6 +812,12 @@ lmato_status_t lmato_set_initial_guess(lmato_handle* h, const double* guess_traj
 lmato_status_t lmato_set_sensitivity_output(lmato_handle* h, double* out_dtf) {
   if (!h) { set_err("lmato_set_sensitivity_output: NULL handle"); return LMATO_ERR_INVALID; }
   h->sens_out = out_dtf;
+  return LMATO_OK;
+}
+
+lmato_status_t lmato_set_param_sensitivity_output(lmato_handle* h, double* out_dtf_dp) {
+  if (!h) { set_err("lmato_set_param_sensitivity_output: NULL handle"); return LMATO_ERR_INVALID; }
+  h->psens_out = out_dtf_dp;
   return LMATO_OK;
 }
 
@@ -948,7 +960,7 @@ lmato_status_t lmato_multi_solve_host(lmato_multi* m, const double* params, int6
   lmato_status_t rc = check_batch("lmato_multi_solve_host", m, params, B, out_tf, out_final_mass, out_status, out_iters);
   if (rc != LMATO_OK || B == 0) return rc;
   const int G = (int)m->h.size();
-  std::vector<HostSolve> sh(G, host_solve(m->h[0]->nt, B, params, nullptr, nullptr, out_traj, nullptr, out_tf,
+  std::vector<HostSolve> sh(G, host_solve(m->h[0]->nt, B, params, nullptr, nullptr, out_traj, nullptr, nullptr, out_tf,
                                           out_final_mass, out_kkt, out_status, out_iters));
   // every device gets its columns and its launch before anything waits; the shards of one batch keep the batch warm
   // start even when a shard alone is small (stage_and_solve passes the whole batch's size).  Every shard is staged,

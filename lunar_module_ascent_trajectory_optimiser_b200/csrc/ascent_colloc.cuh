@@ -731,6 +731,9 @@ struct SweepsColloc {
     }
     if (lam) lam[0] = lam[1] = lam[2] = NAN;
   }
+  LM_HD static void node_duals(const colloc::Nws&, int, int, double* d) {
+    for (int i = 0; i < 9; ++i) d[i] = NAN;
+  }
   LM_HD static void remerit(const Mesh&, const Options&, const colloc::Nws&, int, double, Scal&) {}
 };
 

@@ -1191,6 +1191,14 @@ struct SweepsCoop {
     if (!lam) return;
     lam[0] = r[coop::X_LAM + 1]; lam[1] = r[coop::X_LAM + 3]; lam[2] = r[coop::X_LAM + 5];
   }
+  // the multipliers of node k (as ws_node_duals): the six defect rows, the angle's upper bound, the control's bounds
+  template <class CW>
+  LM_HD static void node_duals(const CW& W, int cur, int k, double* d) {
+    double r[coop::XR];
+    coop::ldv<coop::XR>(W.X(cur, k), r);
+    for (int i = 0; i < 6; ++i) d[i] = r[coop::X_LAM + i];
+    d[6] = r[coop::X_ZUA]; d[7] = r[coop::X_ZLU]; d[8] = r[coop::X_ZUU];
+  }
   template <class CW>
   LM_HD static void remerit(const Mesh&, const Options&, const CW&, int, double, Scal&) {}
 };

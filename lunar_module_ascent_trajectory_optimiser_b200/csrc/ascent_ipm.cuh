@@ -1399,10 +1399,19 @@ LM_HD void ws_node(const Ws& W, int cur, int k, double* x, double* lam) {
   lam[2] = WS_AT(sp, cur * SW::NITER + SW::FLAM + 5);
 }
 
+// The multipliers of node k of iterate `cur` (same layouts as ws_node): d[0..5] those of the six defect rows, d[6] that
+// of the angle's upper bound, d[7], d[8] those of the control's lower and upper bound.
+template <class SW>
+LM_HD void ws_node_duals(const Ws& W, int cur, int k, double* d) {
+  const double* sp = W.stage(k);
+  for (int i = 0; i < 6; ++i) d[i] = WS_AT(sp, cur * SW::NITER + SW::FLAM + i);
+  for (int i = 0; i < 3; ++i) d[6 + i] = WS_AT(sp, cur * SW::NITER + SW::FZLA + 1 + i);
+}
+
 // Sweeps policy of the 7-state formulation (dcost = 0); ascent_ipm_dc.cuh provides the 8-state one.
 struct Sweeps7 {
-  enum : int { NFIELDS = N_FIELDS, NITER = N_ITER, FZ = F_Z, FU = F_U, FLAM = F_LAM, REFROWS = REF_ROWS, MOVE_TERM = 0,
-               LANES_PER_PROBLEM = 1, STORES_REF = 0 };
+  enum : int { NFIELDS = N_FIELDS, NITER = N_ITER, FZ = F_Z, FU = F_U, FLAM = F_LAM, FZLA = F_ZLA, REFROWS = REF_ROWS,
+               MOVE_TERM = 0, LANES_PER_PROBLEM = 1, STORES_REF = 0 };
   LM_HD static int n_eq(const Ws&, int N) { return 6 * N + 3; }
   LM_HD static int n_bd(const Ws&, int N) { return 4 * N + 4; }
   LM_HD static bool backward(const Params& P, const Mesh& M, const Options& O, const Ws& W, int src, const Scal& c0,
@@ -1435,6 +1444,7 @@ struct Sweeps7 {
     for (int i = 0; i < 6; ++i) { WS_AT(s0, F_Z + i) = 0.0; WS_AT(s0, N_ITER + F_Z + i) = 0.0; WS_AT(s0, F_DS + i) = 0.0; }
   }
   LM_HD static void node(const Ws& W, int cur, int k, double* x, double* lam) { ws_node<Sweeps7>(W, cur, k, x, lam); }
+  LM_HD static void node_duals(const Ws& W, int cur, int k, double* d) { ws_node_duals<Sweeps7>(W, cur, k, d); }
   LM_HD static void remerit(const Mesh&, const Options&, const Ws&, int, double, Scal&) {}
 };
 

@@ -738,8 +738,8 @@ LM_SWEEP void riccati_forward(const Params& P, const Mesh& M, const Options& O, 
 
 // Sweeps policy of the 8-state (DCOST) formulation.
 struct Sweeps8 {
-  enum : int { NFIELDS = dc::N_FIELDS, NITER = dc::N_ITER, FZ = dc::F_Z, FU = dc::F_U, FLAM = dc::F_LAM, REFROWS = dc::REF_ROWS,
-               MOVE_TERM = 1, LANES_PER_PROBLEM = 1, STORES_REF = 0 };
+  enum : int { NFIELDS = dc::N_FIELDS, NITER = dc::N_ITER, FZ = dc::F_Z, FU = dc::F_U, FLAM = dc::F_LAM, FZLA = dc::F_ZLA,
+               REFROWS = dc::REF_ROWS, MOVE_TERM = 1, LANES_PER_PROBLEM = 1, STORES_REF = 0 };
   LM_HD static int n_eq(const Ws&, int N) { return 7 * N + 3; }
   LM_HD static int n_bd(const Ws&, int N) { return 6 * N + 4; }
   LM_HD static bool backward(const Params& P, const Mesh& M, const Options& O, const Ws& W, int src, const Scal& c0,
@@ -769,6 +769,7 @@ struct Sweeps8 {
     for (int i = 0; i < 7; ++i) { WS_AT(s0, dc::F_Z + i) = 0.0; WS_AT(s0, dc::N_ITER + dc::F_Z + i) = 0.0; WS_AT(s0, dc::F_DS + i) = 0.0; }
   }
   LM_HD static void node(const Ws& W, int cur, int k, double* x, double* lam) { ws_node<Sweeps8>(W, cur, k, x, lam); }
+  LM_HD static void node_duals(const Ws& W, int cur, int k, double* d) { ws_node_duals<Sweeps8>(W, cur, k, d); }
   LM_HD static void remerit(const Mesh&, const Options&, const Ws&, int, double, Scal&) {}
 };
 

@@ -110,6 +110,47 @@ LM_HD Params derive_params(const double* __restrict__ p, long B, long b, int mod
   return P;
 }
 
+// Partial derivatives of a function of Params (the Lagrangian of the NLP, ascent_result.cuh) with respect to the
+// fields it reads.  S is the distance scale where the dynamics read it (X = x*S, Y = y*S + R0, Sinv = 1/S); the
+// terminal rows read R0S, rt and vt2 instead.  mT = mflow*T and tf_ub = min(1, 1/(mflow*T)) depend on mflow and T
+// alone, so their partials are carried in mflow and T (mflow: through the mass mT*tau*tf and tf_ub; T: through the
+// step h*T*tf, the mass and tf_ub).
+struct ParamsGrad {
+  double GM, R0, Ft, M0, S, ms, mflow, asc, T, a_ub, u_ub, vt2, rt, R0S;
+};
+
+// The chain rule through derive_params: out[r * ostride] = d / d p[r] for every row r of problem b's raw parameter
+// column, given g = the partials with respect to the derived fields.  The circular model does not read
+// angle_doubledot_max and u_bound (derive_params overrides asc and u_ub): those two rows are NaN.
+LM_HD void derive_params_grad(const double* __restrict__ p, long B, long b, int model, const ParamsGrad& g,
+                              double* __restrict__ out, long ostride) {
+  const double G = p[LMATO_P_G * B + b], Mm = p[LMATO_P_M * B + b];
+  const double R0 = p[LMATO_P_R0 * B + b];
+  const double fuel = p[LMATO_P_FUEL_MASS * B + b];
+  const double rp = p[LMATO_P_R_PERIAPSIS * B + b], ra = p[LMATO_P_R_APOAPSIS * B + b];
+  const double GM = G * Mm;
+  const double D = R0 + 0.5 * (rp + ra);
+  const double vt2 = GM / D / (rp * rp);                  // vt2 = GM / (D S^2), D = R0 + (rp + ra)/2, S = rp
+  const double gGM = g.GM + g.vt2 * vt2 / GM;             // GM = G*M
+  const double gD = -g.vt2 * vt2 / D;                     // d vt2 / d D = -vt2 / D
+  const double gR0S = g.rt + g.R0S;                       // rt = R0S + 1, R0S = R0 / S
+  const bool circ = model == LMATO_MODEL_CIRCULAR;
+  out[LMATO_P_G * ostride] = gGM * Mm;
+  out[LMATO_P_M * ostride] = gGM * G;
+  out[LMATO_P_R0 * ostride] = g.R0 + gR0S / rp + gD;
+  out[LMATO_P_FT * ostride] = g.Ft;
+  out[LMATO_P_M0 * ostride] = g.M0;
+  out[LMATO_P_M_DOT * ostride] = g.mflow / fuel;                                     // mflow = M_dot / fuel_mass
+  out[LMATO_P_FUEL_MASS * ostride] = -g.mflow * (p[LMATO_P_M_DOT * B + b] / fuel) / fuel;
+  out[LMATO_P_ANGLE_DOUBLEDOT_MAX * ostride] = circ ? NAN : g.asc / 3.0;           // asc = angle_doubledot_max / 3
+  out[LMATO_P_R_PERIAPSIS * ostride] = g.S - gR0S * R0 / (rp * rp) + gD * 0.5 - 2.0 * g.vt2 * vt2 / rp;
+  out[LMATO_P_R_APOAPSIS * ostride] = gD * 0.5;
+  out[LMATO_P_FINAL_TIME * ostride] = g.T;
+  out[LMATO_P_MASS_SCALAR * ostride] = g.ms;
+  out[LMATO_P_ANGLE_UB * ostride] = g.a_ub;
+  out[LMATO_P_U_BOUND * ostride] = circ ? NAN : g.u_ub;
+}
+
 // 1 in the circular model with the move term (the MV slot holds the pitch angle), else 0
 LM_HD double mv_is_angle(const Params& P) { return (P.coup5 == 0.0 && P.asc == 0.0) ? 1.0 : 0.0; }
 

@@ -141,6 +141,11 @@ int main(int argc, char** argv) {
 static double* g_dtf = nullptr;
 extern "C" void hostsim_set_sensitivity_output(double* dtf) { g_dtf = dtf; }
 
+// d tf / d params[p] for every row p (LMATO_NPARAM values) of the next hostsim_solve / hostsim_solve_coop calls, or
+// NULL: the counterpart of lmato_set_param_sensitivity_output.
+static double* g_dtf_all = nullptr;
+extern "C" void hostsim_set_param_sensitivity_output(double* dtf_all) { g_dtf_all = dtf_all; }
+
 // ctypes entry for developer-side comparisons against tests/golden (NOT the product path).
 extern "C" int hostsim_solve(const double* raw14, int nt, const double* time, double tol, double obj_scale,
                              double mu_min_factor, double* traj /* [10][nt] */, double* tf_out, int* iters, double* kkt) {
@@ -159,7 +164,7 @@ extern "C" int hostsim_solve(const double* raw14, int nt, const double* time, do
   Ws W{ws.data(), (long)nfields * LANES, tile.data()};
   int status;
   double fmass;
-  const ResultOut R{traj, tf_out, &fmass, &status, iters, kkt, g_dtf, 1};
+  const ResultOut R{traj, tf_out, &fmass, &status, iters, kkt, g_dtf, 1, g_dtf_all, raw14};
   if (DC) solve_one<Sweeps8>(R, P, M, O, model, W);
   else solve_one<Sweeps7>(R, P, M, O, model, W);
   return status;
@@ -225,7 +230,7 @@ extern "C" int hostsim_solve_coop(const double* raw14, int nt, const double* tim
   coop::Cws W{ws.data(), nt, scr.data(), 0, 1u, 1u, 0.0, 0.0, 0, 0u};
   int status;
   double fmass;
-  const ResultOut R{traj, tf_out, &fmass, &status, iters, kkt, g_dtf, 1};
+  const ResultOut R{traj, tf_out, &fmass, &status, iters, kkt, g_dtf, 1, g_dtf_all, raw14};
   const bool vrec = getenv("VREC") != nullptr;     // the variant that keeps W_k, g_k instead of running the adjoint recursion
   if (DC && model == LMATO_MODEL_CIRCULAR) solve_one<SweepsCoop<1, 1, 2, false>>(R, P, M, O, model, W);
   else if (DC && vrec) solve_one<SweepsCoop<1, 1, true, true>>(R, P, M, O, model, W);
